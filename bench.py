@@ -244,6 +244,38 @@ def layer_diff(got, ref):
     return out
 
 
+# whole blocks per layer whose voxels --dump-outputs writes: with every block index of the two C2
+# layers (at most 4096 + 32768 blocks) that stays under 53 MB in all
+DUMP_BLOCKS = 256
+
+
+def dump_outputs(out_dir, layers, stats):
+    """--dump-outputs: what the timed path hands its caller after its last step, as
+    out_dir/<name>.npy.  Per layer: every block index (the (z,y,x) order of download()) and its
+    flags, and distance, weight and rgba of DUMP_BLOCKS blocks (all of them when there are fewer),
+    a seeded choice of rows of that list stored as <layer>_sample_rows; the voxel fields are float32,
+    indices, flags and counters float64.  Per call statistics struct: one scalar per field."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {}
+    for name, layer in layers.items():
+        idx, vox, flags = layer.download()
+        rows = np.arange(len(idx))
+        if len(idx) > DUMP_BLOCKS:
+            rows = np.sort(np.random.default_rng(0).choice(len(idx), DUMP_BLOCKS, replace=False))
+        arrays[f"{name}_block_idx"] = idx.astype(np.float64)
+        arrays[f"{name}_flags"] = flags.astype(np.float64)
+        arrays[f"{name}_sample_rows"] = rows.astype(np.float64)
+        arrays[f"{name}_distance"] = vox["distance"][rows].astype(np.float32)
+        arrays[f"{name}_weight"] = vox["weight"][rows].astype(np.float32)
+        arrays[f"{name}_rgba"] = vox["rgba"][rows].astype(np.float32)
+    for name, st in stats.items():
+        for field, _ in st._fields_:
+            arrays[f"{name}_{field}"] = np.array(getattr(st, field), np.float64)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+    return arrays
+
+
 def time_sharded(subs, poses, partial, owned, ctx, barrier, max_over_ranks, sum_over_ranks, vox,
                  stream):
     """The server's global merge over all ranks, timed on the device (max over ranks): every rank
@@ -456,9 +488,10 @@ def run_ours(args, rank, world, local_rank):
         integ.integrateBatch(e["poses"], e["d_pts"], e["d_cols"], e["offs"])
         if ev:
             ev[1].record(stream)
-        mergeLayerAintoLayerB(submap, e["T_M_S"], glob)
+        mst = mergeLayerAintoLayerB(submap, e["T_M_S"], glob)
         if ev:
             ev[2].record(stream)
+        return mst
 
     def run_e2e(entries, pipelined=True):
         """Every step: H2D of its inputs from pinned host memory (cg_stage_batch_async, double
@@ -488,7 +521,9 @@ def run_ours(args, rank, world, local_rank):
 
     def run_pipelined(entries):
         """Inputs resident in HBM; the first half of step k+1 (cg_prepare_batch_device) is queued
-        before step k is completed (cg_integrate_prepared) and merged."""
+        before step k is completed (cg_integrate_prepared) and merged.  Returns the MergeStats
+        of the last step."""
+        mst = None
         if entries:
             e = entries[0]
             integ.prepareBatch(0, e["poses"], e["d_pts"], e["d_cols"], e["offs"])
@@ -498,13 +533,15 @@ def run_ours(args, rank, world, local_rank):
                 integ.prepareBatch((k + 1) % 2, n["poses"], n["d_pts"], n["d_cols"], n["offs"])
             submap.clear()
             integ.integratePrepared(k % 2)
-            mergeLayerAintoLayerB(submap, e["T_M_S"], glob)
+            mst = mergeLayerAintoLayerB(submap, e["T_M_S"], glob)
+        return mst
 
     results = {}
     # "device": inputs resident in HBM, no instrumentation (-> value); "profiled": the same steps
     # with the library's stage timers on (-> stages_ms_per_step, roofline); "e2e": host buffers
     legs = ("device", "profiled", "e2e") if args.profile_mode else \
         ("device", "profiled", "pipelined", "e2e", "e2e_plain")
+    headline_leg = "pipelined" if "pipelined" in legs else "device"   # the leg `value` reports
     for leg in legs:
         glob.clear()
         if leg in ("device", "profiled"):
@@ -525,6 +562,7 @@ def run_ours(args, rank, world, local_rank):
         barrier()
         ev_a.record(stream)
         d2h = 0
+        last_merge = None
         if leg in ("device", "profiled"):
             for k in range(args.steps):
                 # profile mode: the last un-instrumented step sits in an NVTX range, so that ncu
@@ -532,11 +570,11 @@ def run_ours(args, rank, world, local_rank):
                 mark = args.profile_mode and leg == "device" and k == args.steps - 1
                 if mark:
                     torch.cuda.nvtx.range_push("cg_step")
-                step_device(pool[(args.warmup + k) % pool_n], evs[k])
+                last_merge = step_device(pool[(args.warmup + k) % pool_n], evs[k])
                 if mark:
                     torch.cuda.nvtx.range_pop()
         elif leg == "pipelined":
-            run_pipelined([pool[(args.warmup + k) % pool_n] for k in range(args.steps)])
+            last_merge = run_pipelined([pool[(args.warmup + k) % pool_n] for k in range(args.steps)])
         else:
             d2h = run_e2e([pool[(args.warmup + k) % pool_n] for k in range(args.steps)],
                           pipelined=(leg == "e2e"))
@@ -559,6 +597,10 @@ def run_ours(args, rank, world, local_rank):
             if leg == "profiled":
                 res["profile"] = ctx.profile()
         results[leg] = res
+        if args.dump_outputs and rank == 0 and leg == headline_leg:
+            # before the next leg clears the layers; integ.last_stats is the last step's
+            dump_outputs(args.dump_outputs, {"submap": submap, "global": glob},
+                         {"integrate": integ.last_stats, "merge": last_merge})
 
     # ---- server-side global merge at the C2 shape: 2 robots x 20 submaps projected into one
     # global TSDF with cblox getProjectedMap() semantics (one call, batched on the device)
@@ -873,7 +915,7 @@ def run_ours(args, rank, world, local_rank):
                         / n_used / 2)
         # headline: the pipelined loop (the first half of step k+1 is queued before step k is
         # completed: cg_prepare_batch_device / cg_integrate_prepared); the plain-call loop beside it
-        hv = results.get("pipelined", dv)
+        hv = results[headline_leg]
         roof = roofline_record(prof, args.steps, hv["total_ms"] / args.steps,
                                (dv["bytes_int"] + dv["bytes_merge"]) / args.steps, per_step)
         line = {
@@ -991,7 +1033,15 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--profile-mode", action="store_true",
                     help="skip the accounting pass and the CPU baseline (for runs under ncu)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps of the leg `value` reports, write what its last "
+                         "step left (the fused submap, the global layer, the call statistics) as "
+                         "DIR/<name>.npy; rank 0, config C2")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.config != "C2"):
+        ap.error("--dump-outputs covers the CUDA arm of config C2")
     args.warmup = max(args.warmup, 0)
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

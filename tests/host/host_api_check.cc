@@ -3,7 +3,8 @@
 // writes the input frames, runs this program on the GPU box and compares the layers it writes
 // with the CPU oracle.
 //   host_api_check nogpu                       -> exit 0 iff creating a context fails loudly
-//   host_api_check run <in.bin> <out.bin>      -> integrate frames, merge, dump both layers
+//   host_api_check run <in.bin> <out.bin>      -> integrate frames, merge, dump both layers (and
+//                                                 the connected mesh as <out.bin>.ply)
 //   host_api_check time <in.bin> <passes>      -> the live path as a C++ host drives it: one
 //                                                 integratePointCloud call per frame with pageable
 //                                                 std::vector inputs; prints the mean ms per call
@@ -139,7 +140,7 @@ int main(int argc, char** argv) {
       const cg::Point& b = mesh.vertices[i];
       if (a.x != b.x || a.y != b.y || a.z != b.z) return 78;
     }
-    if (!cg::outputMeshAsPly("/tmp/cg_host_api_check.ply", connected)) return 79;
+    if (!cg::outputMeshAsPly(std::string(argv[3]) + ".ply", connected)) return 79;
   }
   // ... and what the client's MapServer does with its combined map (map_server.h:141-145,
   // map_server.cpp:112-113): batch ESDF, then the traversable cloud

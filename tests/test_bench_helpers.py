@@ -52,3 +52,49 @@ def test_layer_diff_reports_margins():
     b["weight"][0, 9] = 2.1
     assert not bench.layer_diff((idx, b, None), (idx, a, None))["within_tolerance"]
     assert not bench.layer_diff((np.array([[1, 0, 0]], np.int32), a, None), (idx, a, None))["block_sets_equal"]
+
+
+class _FakeLayer:
+    def __init__(self, blocks, seed):
+        import numpy as np
+        from coxgraph_b200 import VOXEL_DTYPE
+        rng = np.random.default_rng(seed)
+        self.idx = np.stack([np.arange(blocks), np.zeros(blocks), np.zeros(blocks)], 1).astype(np.int32)
+        self.vox = np.zeros((blocks, 4096), VOXEL_DTYPE)
+        self.vox["distance"] = rng.standard_normal((blocks, 4096))
+        self.vox["weight"] = rng.random((blocks, 4096))
+        self.vox["rgba"] = rng.integers(0, 256, (blocks, 4096, 4))
+        self.flags = rng.integers(0, 4, blocks).astype(np.uint8)
+
+    def download(self):
+        return self.idx, self.vox, self.flags
+
+
+def test_dump_outputs_writes_a_fixed_sample_as_float_arrays(tmp_path):
+    import numpy as np
+    from coxgraph_b200 import capi
+    big, small = _FakeLayer(bench.DUMP_BLOCKS + 40, 1), _FakeLayer(7, 2)
+    st = capi.MergeStats(blocks_in=5, blocks_candidate=9, blocks_out=8)
+    out = bench.dump_outputs(str(tmp_path / "a"), {"global": big, "submap": small}, {"merge": st})
+    again = bench.dump_outputs(str(tmp_path / "b"), {"global": big, "submap": small}, {"merge": st})
+    for name, arr in out.items():
+        on_disk = np.load(tmp_path / "a" / f"{name}.npy")
+        assert on_disk.dtype in (np.float32, np.float64), name
+        assert np.array_equal(on_disk, arr) and np.array_equal(on_disk, again[name]), name
+    rows = out["global_sample_rows"].astype(int)
+    assert len(rows) == bench.DUMP_BLOCKS and len(np.unique(rows)) == len(rows)
+    assert np.array_equal(out["global_distance"], big.vox["distance"][rows])
+    assert np.array_equal(out["global_rgba"], big.vox["rgba"][rows].astype(np.float32))
+    assert np.array_equal(out["global_block_idx"], big.idx) and np.array_equal(out["global_flags"], big.flags)
+    assert np.array_equal(out["submap_sample_rows"], np.arange(7))
+    assert out["merge_blocks_out"] == 8.0 and out["merge_blocks_candidate"] == 9.0
+    # the largest dump of the bench's layers (4096- and 32768-block capacities) fits in 64 MB
+    worst = sum(b * 4 * 8 + min(b, bench.DUMP_BLOCKS) * (8 + 4096 * 6 * 4) for b in (4096, 32768))
+    assert worst <= 64e6
+
+
+def test_bench_refuses_zero_steps():
+    import subprocess
+    import sys
+    r = subprocess.run([sys.executable, bench.__file__, "--steps", "0"], capture_output=True, text=True)
+    assert r.returncode == 2 and "--steps" in r.stderr
