@@ -257,8 +257,7 @@ struct cg_context : cg::FrontBufs {
   bool own_stream = false;
   cudaEvent_t wait_event = nullptr;         // cg_context_wait_stream
   cg::HostStager* stager = nullptr;         // pageable inputs (lazy, host_stage.cu)
-  cudaStream_t copy_stream = nullptr;       // pipelined host->device transfers (lazy)
-  std::vector<cudaEvent_t> copy_events;
+  cudaStream_t copy_stream = nullptr;       // cg_stage_batch_async transfers (lazy)
   cg::DevBuf stage_pts[2], stage_cols[2];   // cg_stage_batch_async double buffer
   cudaEvent_t stage_ready[2] = {nullptr, nullptr};
   size_t stage_points[2] = {0, 0};

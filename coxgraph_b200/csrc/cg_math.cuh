@@ -70,6 +70,18 @@ __device__ __forceinline__ Xform inverse(const Xform& T) {
   const V3 r = rotate(T.w, cv, T.t);
   return Xform{T.w, cv, V3{-r.x, -r.y, -r.z}};
 }
+// inverse() on the host: rotate(w, conj(v), t) spelled out in the same operation order (host code
+// is compiled without FMA contraction, see Makefile), so it gives the device's bits
+inline Xform inverse_xform_host(const Xform& T) {
+  const float w = T.w;
+  const V3 cv = V3{-T.v.x, -T.v.y, -T.v.z};
+  const V3 t = T.t;
+  V3 uv = V3{cv.y * t.z - cv.z * t.y, cv.z * t.x - cv.x * t.z, cv.x * t.y - cv.y * t.x};
+  uv = V3{uv.x + uv.x, uv.y + uv.y, uv.z + uv.z};
+  const V3 cr = V3{cv.y * uv.z - cv.z * uv.y, cv.z * uv.x - cv.x * uv.z, cv.x * uv.y - cv.y * uv.x};
+  const V3 r = V3{(t.x + w * uv.x) + cr.x, (t.y + w * uv.y) + cr.y, (t.z + w * uv.z) + cr.z};
+  return Xform{w, cv, V3{-r.x, -r.y, -r.z}};
+}
 
 // getGridIndexFromPoint: floor(x * inv + 1e-6)
 __device__ __forceinline__ int grid_index(float x, float inv) {

@@ -2514,17 +2514,9 @@ static int32_t upload_frame_tables(FrontBufs& fb, size_t F, const float* h_poses
   return CG_OK;
 }
 
-// Frames grouped for a pipelined host->device transfer: group g covers frames
-// [bounds[g], bounds[g+1]) and may start once ready[g] has fired on the copy stream.
-struct TransferPlan {
-  std::vector<size_t> bounds;
-  std::vector<cudaEvent_t> ready;
-};
-
 static int32_t integrate_job(cg_layer* L, const cg_integrator_config* cfg, size_t F,
                              const float* h_poses, const float* d_points, const uint8_t* d_colors,
-                             const uint64_t* offs, int freespace, cg_integrate_stats* stats,
-                             const TransferPlan* plan = nullptr) {
+                             const uint64_t* offs, int freespace, cg_integrate_stats* stats) {
   if (cfg->method == CG_METHOD_FAST) {
     set_error("method FAST is order- and wall-clock-dependent in the reference and has no "
               "deterministic device form; use MERGED or SIMPLE");
@@ -2543,28 +2535,15 @@ static int32_t integrate_job(cg_layer* L, const cg_integrator_config* cfg, size_
     stats->points_in = offs[F] - offs[0];
   }
   const size_t max_group_points = env_size("CG_MAX_GROUP_POINTS", size_t(48) << 20);
-  // poses and frame offsets (relative to the job's first point) go up once per job; with a
-  // transfer plan the caller already queued them on the copy stream ahead of the point data
-  if (!plan) {
-    int32_t urc = upload_frame_tables(*L->ctx, F, h_poses, offs, L->ctx->stream);
-    if (urc) return urc;
-  }
-  int32_t rc = CG_OK;
-  if (plan) {
-    // the copies of group g+1.. proceed on the copy stream while group g is fused
-    for (size_t g = 0; g + 1 < plan->bounds.size() && rc == CG_OK; ++g) {
-      CG_CUDA(cudaStreamWaitEvent(L->ctx->stream, plan->ready[g], 0));
-      rc = integrate_group(L, cfg, P, h_poses, d_points, d_colors, offs, plan->bounds[g],
-                           plan->bounds[g + 1], stats);
-    }
-  } else {
-    size_t f0 = 0;
-    while (f0 < F && rc == CG_OK) {
-      size_t f1 = f0 + 1;
-      while (f1 < F && offs[f1 + 1] - offs[f0] <= max_group_points) ++f1;
-      rc = integrate_group(L, cfg, P, h_poses, d_points, d_colors, offs, f0, f1, stats);
-      f0 = f1;
-    }
+  // poses and frame offsets (relative to the job's first point) go up once per job
+  int32_t rc = upload_frame_tables(*L->ctx, F, h_poses, offs, L->ctx->stream);
+  if (rc) return rc;
+  size_t f0 = 0;
+  while (f0 < F && rc == CG_OK) {
+    size_t f1 = f0 + 1;
+    while (f1 < F && offs[f1 + 1] - offs[f0] <= max_group_points) ++f1;
+    rc = integrate_group(L, cfg, P, h_poses, d_points, d_colors, offs, f0, f1, stats);
+    f0 = f1;
   }
   const int32_t rc2 = finish_call(L, nullptr);
   if (stats) stats->blocks_allocated = L->num_blocks - blocks_before;
@@ -2774,51 +2753,6 @@ int32_t cg_integrate_batch(cg_layer* L, const cg_integrator_config* cfg, size_t 
   std::vector<uint64_t> rel(F + 1);
   for (size_t f = 0; f <= F; ++f) rel[f] = offs[f] - first;
   cg_context* ctx = L->ctx;
-  // Optional (CG_H2D_CHUNK_POINTS > 0): the host->device copy is cut into groups of frames on a
-  // second stream so that fusing group g overlaps the copy of group g+1.  Off by default: at the
-  // C2 size every group costs ~0.5 ms of latency-bound kernel tails, more than the overlap wins
-  // (measured); overlapping across jobs (cg_stage_batch_async) is what pays.
-  const size_t chunk_points = env_size("CG_H2D_CHUNK_POINTS", 0);
-  if (F > 1 && total > 2 * chunk_points && chunk_points > 0) {
-    for (size_t f = 0; f < F; ++f)
-      if (offs[f + 1] < offs[f]) {
-        set_error("frame_offsets must be non-decreasing");
-        return CG_ERR_INVALID_ARG;
-      }
-    CG_CUDA(cudaSetDevice(ctx->device));
-    CG_CUDA(ctx->points.reserve(total * 3 * sizeof(float)));
-    CG_CUDA(ctx->colors.reserve(total * 4));
-    if (!ctx->copy_stream)
-      CG_CUDA(cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
-    TransferPlan plan;
-    plan.bounds.push_back(0);
-    for (size_t f = 1; f <= F; ++f)
-      if (f == F || rel[f] - rel[plan.bounds.back()] >= chunk_points) plan.bounds.push_back(f);
-    const size_t G = plan.bounds.size() - 1;
-    int32_t urc = upload_frame_tables(*ctx, F, poses, rel.data(), ctx->stream);
-    if (urc) return urc;
-    while (ctx->copy_events.size() < G) {
-      cudaEvent_t e;
-      CG_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-      ctx->copy_events.push_back(e);
-    }
-    for (size_t g = 0; g < G; ++g) {
-      const size_t a = rel[plan.bounds[g]], b = rel[plan.bounds[g + 1]];
-      CG_CUDA(cudaMemcpyAsync(ctx->points.as<float>() + 3 * a, pts + 3 * (first + a),
-                              (b - a) * 3 * sizeof(float), cudaMemcpyHostToDevice,
-                              ctx->copy_stream));
-      CG_CUDA(cudaMemcpyAsync(ctx->colors.as<uint8_t>() + 4 * a, cols + 4 * (first + a),
-                              (b - a) * 4, cudaMemcpyHostToDevice, ctx->copy_stream));
-      CG_CUDA(cudaEventRecord(ctx->copy_events[g], ctx->copy_stream));
-      plan.ready.push_back(ctx->copy_events[g]);
-    }
-    const int32_t rc = integrate_job(L, cfg, F, poses, ctx->points.as<float>(),
-                                     ctx->colors.as<uint8_t>(), rel.data(), freespace, stats, &plan);
-    // the staging buffers are reused by the next call: the copies must have drained even if the
-    // job failed early
-    cudaStreamSynchronize(ctx->copy_stream);
-    return rc;
-  }
   int32_t rc = stage_inputs(ctx, pts + 3 * first, cols + 4 * first, total);
   if (rc) return rc;
   return cg_integrate_batch_device(L, cfg, F, poses, ctx->points.as<float>(),

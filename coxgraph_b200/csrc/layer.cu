@@ -1,7 +1,6 @@
 // layer.cu — context and Layer<TsdfVoxel> replacement: creation, clear, upload, download.
 // Boundary: include/coxgraph_b200.h.  Reference data contract: voxblox Layer / Block /
 // TsdfVoxel as consumed at coxgraph/include/coxgraph/utils/msg_converter.h:49-50,107-109.
-#include <cstdlib>
 #include <cub/cub.cuh>
 #include <stdarg.h>
 #include <string.h>
@@ -412,11 +411,6 @@ cudaError_t init_front_words(FrontBufs& fb) {
   return cudaMemset(fb.d_front_err, 0, sizeof(int32_t));
 }
 bool side_stream(FrontBufs& fb, cudaStream_t like) {
-  static const bool enabled = [] {
-    const char* v = std::getenv("CG_SIDE_STREAM");
-    return !(v && v[0] == '0');
-  }();
-  if (!enabled) return false;
   if (fb.side) return true;
   int prio = 0;
   if (cudaStreamGetPriority(like, &prio) != cudaSuccess) prio = 0;
@@ -577,7 +571,6 @@ int32_t cg_context_destroy(cg_context* ctx) {
   if (ctx->d_walk_counters) cudaFree(ctx->d_walk_counters);
   if (ctx->d_work_counter) cudaFree(ctx->d_work_counter);
   if (ctx->d_long_counter) cudaFree(ctx->d_long_counter);
-  for (cudaEvent_t e : ctx->copy_events) cudaEventDestroy(e);
   for (int i = 0; i < 2; ++i) {
     ctx->stage_pts[i].release();
     ctx->stage_cols[i].release();

@@ -375,21 +375,7 @@ static int32_t enqueue_merge(const cg_layer* A, const float T_B_A[7], cg_layer* 
         A->v, static_cast<int>(nA), T, B->v.block_size, ctx->cand_keys.as<uint64_t>(),
         static_cast<uint32_t>(cap - 1), ctx->cand_list.as<uint64_t>(), ctx->d_counters, B->v.err);
   }
-  // inverse on the host with the same operation order as the device / reference
-  Xform Ti;
-  {
-    const float w = T.w;
-    const V3 cv = V3{-T.v.x, -T.v.y, -T.v.z};
-    // rotate(w, cv, t) spelled out (host code: no FMA contraction, see Makefile flags)
-    const V3 t = T.t;
-    V3 uv = V3{cv.y * t.z - cv.z * t.y, cv.z * t.x - cv.x * t.z, cv.x * t.y - cv.y * t.x};
-    uv = V3{uv.x + uv.x, uv.y + uv.y, uv.z + uv.z};
-    const V3 cr = V3{cv.y * uv.z - cv.z * uv.y, cv.z * uv.x - cv.x * uv.z, cv.x * uv.y - cv.y * uv.x};
-    const V3 r = V3{(t.x + w * uv.x) + cr.x, (t.y + w * uv.y) + cr.y, (t.z + w * uv.z) + cr.z};
-    Ti.w = w;
-    Ti.v = cv;
-    Ti.t = V3{-r.x, -r.y, -r.z};
-  }
+  const Xform Ti = inverse_xform_host(T);
   const unsigned grid = static_cast<unsigned>(
       std::min<size_t>(cand_bound, static_cast<size_t>(ctx->num_sms) * 4));
   const size_t smem = 3 * kVoxelsPerBlock * sizeof(float) + sizeof(SlotTable);
@@ -554,7 +540,7 @@ __global__ void __launch_bounds__(kMergeThreads)
 k_project_batch(const BatchSubmap* __restrict__ desc, LayerView B,
                 const uint64_t* __restrict__ map_keys, const BatchCand* __restrict__ list,
                 const RankTable* __restrict__ table, unsigned long long* done,
-                uint32_t* work_counter, CallCounters* counters, int bulk_prefetch) {
+                uint32_t* work_counter, CallCounters* counters) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   float* s_d = reinterpret_cast<float*>(smem_raw);  // resampled block, planar
   float* s_w = s_d + kVoxelsPerBlock;
@@ -588,27 +574,11 @@ k_project_batch(const BatchSubmap* __restrict__ desc, LayerView B,
       const int az = __float2int_rd((pc.z - reach) * A.block_size_inv);
       const int t = threadIdx.x;
       const int dx = t % kTab, dy = (t / kTab) % kTab, dz = t / (kTab * kTab);
-      const int slot = A.find_slot(pack_block_key(ax + dx, ay + dy, az + dz));
-      tab.slot[t] = slot;
+      tab.slot[t] = A.find_slot(pack_block_key(ax + dx, ay + dy, az + dz));
       if (t == 0) {
         tab.ax = ax;
         tab.ay = ay;
         tab.az = az;
-      }
-      // Optional (CG_MERGE_BULK_PREFETCH=1; measured, off by default — DESIGN.md §4.3): the TMA
-      // unit pulls the three planes of every source block the rotated destination block can
-      // reach into L2 (one cp.async.bulk.prefetch per block, 48 KB) while the taps are set up.
-      if (bulk_prefetch && slot >= 0) {
-        const V3 cb = V3{center_coord(ax + dx, A.block_size), center_coord(ay + dy, A.block_size),
-                         center_coord(az + dz, A.block_size)};
-        const V3 dv = cb - pc;
-        const float lim = reach + 0.8660254f * A.block_size;
-        if (dot3(dv, dv) <= lim * lim) {
-          const float* src = A.dist_plane(slot);
-          asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(src),
-                       "r"(static_cast<uint32_t>(3 * kVoxelsPerBlock * sizeof(float)))
-                       : "memory");
-        }
       }
     }
     __syncthreads();
@@ -679,23 +649,6 @@ __global__ void k_copy_desc(uint32_t* __restrict__ dst, const uint32_t* __restri
   if (i < n) dst[i] = src[i];
 }
 
-static Xform inverse_host(const Xform& T) {
-  // rotate(w, conj(v), t) spelled out (host code: no FMA contraction, see Makefile flags), the
-  // same operation order as the device / reference
-  const float w = T.w;
-  const V3 cv = V3{-T.v.x, -T.v.y, -T.v.z};
-  const V3 t = T.t;
-  V3 uv = V3{cv.y * t.z - cv.z * t.y, cv.z * t.x - cv.x * t.z, cv.x * t.y - cv.y * t.x};
-  uv = V3{uv.x + uv.x, uv.y + uv.y, uv.z + uv.z};
-  const V3 cr = V3{cv.y * uv.z - cv.z * uv.y, cv.z * uv.x - cv.x * uv.z, cv.x * uv.y - cv.y * uv.x};
-  const V3 r = V3{(t.x + w * uv.x) + cr.x, (t.y + w * uv.y) + cr.y, (t.z + w * uv.z) + cr.z};
-  Xform Ti;
-  Ti.w = w;
-  Ti.v = cv;
-  Ti.t = V3{-r.x, -r.y, -r.z};
-  return Ti;
-}
-
 // submaps [i0, i1) as one batch (descriptors already on the device); everything is enqueued on the
 // context's stream, nothing is read back
 static int32_t project_batch(const cg_layer* const* submaps, const BatchSubmap* h_desc,
@@ -745,15 +698,11 @@ static int32_t project_batch(const cg_layer* const* submaps, const BatchSubmap* 
   }
   {
     StageScope sc(ctx, kStageMergeResample, 1);
-    static const int bulk_prefetch = [] {
-      const char* e = getenv("CG_MERGE_BULK_PREFETCH");
-      return (e && *e == '1') ? 1 : 0;
-    }();
     const unsigned grid = static_cast<unsigned>(
         std::min<size_t>(cand_bound, static_cast<size_t>(ctx->num_sms) * 2));
     k_project_batch<<<grid, kMergeThreads, smem, s>>>(
         d_desc + i0, G->v, ctx->cand_keys.as<uint64_t>(), ctx->merge_cands.as<BatchCand>(), table,
-        done, ctx->d_work_counter, ctx->d_counters, bulk_prefetch);
+        done, ctx->d_work_counter, ctx->d_counters);
   }
   CG_CUDA(cudaGetLastError());
   return CG_OK;
@@ -799,9 +748,35 @@ __global__ void k_flag_dead(LayerView G, const uint32_t* __restrict__ slots,
 static void fill_desc(BatchSubmap& d, const cg_layer* A, const float* pose, uint32_t first) {
   d.A = A->v;
   d.T_B_A = make_xform(pose);
-  d.T_A_B = inverse_host(d.T_B_A);
+  d.T_A_B = inverse_xform_host(d.T_B_A);
   d.first_block = first;
   d.num_blocks = static_cast<uint32_t>(A->num_blocks);
+}
+
+// Puts `count` descriptors into ctx->batch_desc (pinned, device-mapped staging + a copy kernel)
+// and resets the merge counters of the call behind them.  The host writes ctx->h_tables only while
+// no queued kernel reads it: every call that stages through it (the projections here and
+// integrate.cu's upload_frame_tables) ends, on success, in finish_call's stream synchronise.  An
+// error return may leave the copy queued; the CUDA errors that end a call early are sticky, so no
+// later call gets as far as writing the table.
+static int32_t upload_descs(cg_context* ctx, const BatchSubmap* descs, size_t count) {
+  const size_t desc_bytes = count * sizeof(BatchSubmap);
+  if (desc_bytes > ctx->h_tables_cap) {
+    if (ctx->h_tables) cudaFreeHost(ctx->h_tables);
+    ctx->h_tables = nullptr;
+    ctx->h_tables_cap = 0;
+    CG_CUDA(cudaHostAlloc(&ctx->h_tables, desc_bytes * 2, cudaHostAllocMapped));
+    ctx->h_tables_cap = desc_bytes * 2;
+  }
+  memcpy(ctx->h_tables, descs, desc_bytes);
+  void* d_alias = nullptr;
+  CG_CUDA(cudaHostGetDevicePointer(&d_alias, ctx->h_tables, 0));
+  CG_CUDA(ctx->batch_desc.reserve(desc_bytes));
+  ctx->own_launches += 2;
+  k_copy_desc<<<grid_for(desc_bytes / 4, 256), 256, 0, ctx->stream>>>(
+      ctx->batch_desc.as<uint32_t>(), static_cast<const uint32_t*>(d_alias), desc_bytes / 4);
+  k_reset_merge_counters<<<1, 1, 0, ctx->stream>>>(ctx->d_counters);
+  return CG_OK;
 }
 
 static bool pose_changed(const float* a, const float* b, float eps_t, float eps_rot) {
@@ -857,40 +832,23 @@ int32_t cg_project_submaps(const cg_layer* const* submaps, const float* poses, s
     }
   }
   if (n == 0) return finish_call(G, nullptr);
-  // descriptors of all submaps go up once (pinned, device-mapped staging + a copy kernel)
-  const size_t desc_bytes = n * sizeof(BatchSubmap);
-  if (desc_bytes > ctx->h_tables_cap) {
-    if (ctx->h_tables) cudaFreeHost(ctx->h_tables);
-    ctx->h_tables = nullptr;
-    ctx->h_tables_cap = 0;
-    CG_CUDA(cudaHostAlloc(&ctx->h_tables, desc_bytes * 2, cudaHostAllocMapped));
-    ctx->h_tables_cap = desc_bytes * 2;
-  }
-  BatchSubmap* h = static_cast<BatchSubmap*>(ctx->h_tables);
+  // descriptors of all submaps go up once
+  std::vector<BatchSubmap> h(n);
   uint64_t blocks_in = 0;
   for (size_t i0 = 0; i0 < n; i0 += kBatchMax) {
     uint32_t total = 0;
     for (size_t i = i0; i < std::min(n, i0 + static_cast<size_t>(kBatchMax)); ++i) {
-      h[i].A = submaps[i]->v;
-      h[i].T_B_A = make_xform(poses + 7 * i);
-      h[i].T_A_B = inverse_host(h[i].T_B_A);
-      h[i].first_block = total;  // prefix sum inside the submap's batch
-      h[i].num_blocks = static_cast<uint32_t>(submaps[i]->num_blocks);
+      fill_desc(h[i], submaps[i], poses + 7 * i, total);  // prefix sum inside the submap's batch
       total += h[i].num_blocks;
     }
     blocks_in += total;
   }
-  void* d_alias = nullptr;
-  CG_CUDA(cudaHostGetDevicePointer(&d_alias, ctx->h_tables, 0));
-  CG_CUDA(ctx->batch_desc.reserve(desc_bytes));
-  ctx->own_launches += 2;
-  k_copy_desc<<<grid_for(desc_bytes / 4, 256), 256, 0, ctx->stream>>>(
-      ctx->batch_desc.as<uint32_t>(), static_cast<const uint32_t*>(d_alias), desc_bytes / 4);
-  k_reset_merge_counters<<<1, 1, 0, ctx->stream>>>(ctx->d_counters);
+  int32_t urc = upload_descs(ctx, h.data(), n);
+  if (urc) return urc;
   // batches of up to 64 submaps, in submap order (the mask of a destination block has one bit per
   // submap of the batch)
   for (size_t i0 = 0; i0 < n; i0 += kBatchMax) {
-    int32_t rc = project_batch(submaps, h, ctx->batch_desc.as<BatchSubmap>(), i0,
+    int32_t rc = project_batch(submaps, h.data(), ctx->batch_desc.as<BatchSubmap>(), i0,
                                std::min(n, i0 + static_cast<size_t>(kBatchMax)), G);
     if (rc) return rc;
   }
@@ -935,16 +893,7 @@ int32_t cg_reproject_submaps(const cg_layer* const* submaps, const float* poses_
   if (moved.empty()) return CG_OK;
   // descriptor table: [0, n) all submaps under their effective pose (batch-relative block prefix),
   // then every moved submap under its old and under its new pose (one prefix over the list)
-  const size_t nd = n + 2 * moved.size();
-  const size_t desc_bytes = nd * sizeof(BatchSubmap);
-  if (desc_bytes > ctx->h_tables_cap) {
-    if (ctx->h_tables) cudaFreeHost(ctx->h_tables);
-    ctx->h_tables = nullptr;
-    ctx->h_tables_cap = 0;
-    CG_CUDA(cudaHostAlloc(&ctx->h_tables, desc_bytes * 2, cudaHostAllocMapped));
-    ctx->h_tables_cap = desc_bytes * 2;
-  }
-  BatchSubmap* h = static_cast<BatchSubmap*>(ctx->h_tables);
+  std::vector<BatchSubmap> h(n + 2 * moved.size());
   {
     size_t mi = 0;
     for (size_t i0 = 0; i0 < n; i0 += kBatchMax) {
@@ -967,13 +916,8 @@ int32_t cg_reproject_submaps(const cg_layer* const* submaps, const float* poses_
     dirty_src += h[n + 2 * k + 1].num_blocks;
     dirty_bound += 2 * mark_bound(submaps[i], G, h[n + 2 * k].num_blocks);
   }
-  void* d_alias = nullptr;
-  CG_CUDA(cudaHostGetDevicePointer(&d_alias, ctx->h_tables, 0));
-  CG_CUDA(ctx->batch_desc.reserve(desc_bytes));
-  ctx->own_launches += 2;
-  k_copy_desc<<<grid_for(desc_bytes / 4, 256), 256, 0, s>>>(
-      ctx->batch_desc.as<uint32_t>(), static_cast<const uint32_t*>(d_alias), desc_bytes / 4);
-  k_reset_merge_counters<<<1, 1, 0, s>>>(ctx->d_counters);
+  int32_t urc = upload_descs(ctx, h.data(), h.size());
+  if (urc) return urc;
   const BatchSubmap* d_desc = ctx->batch_desc.as<BatchSubmap>();
   uint32_t dirty_total = 0, dirty_existing = 0;
   uint64_t removed = 0;
@@ -1031,7 +975,7 @@ int32_t cg_reproject_submaps(const cg_layer* const* submaps, const float* poses_
     }
     // every submap that reaches a dirty block is folded into it again, in submap order
     for (size_t i0 = 0; i0 < n; i0 += kBatchMax) {
-      int32_t rc = project_batch(submaps, h, d_desc, i0, std::min(n, i0 + static_cast<size_t>(kBatchMax)),
+      int32_t rc = project_batch(submaps, h.data(), d_desc, i0, std::min(n, i0 + static_cast<size_t>(kBatchMax)),
                                  G, ctx->stage_a.as<uint64_t>(), static_cast<uint32_t>(cap - 1));
       if (rc) return rc;
     }

@@ -172,23 +172,6 @@ __global__ void k_frame_cloud(const FrameMap* __restrict__ frames, const float* 
   }
 }
 
-static Xform inverse_pose_host(const float* T7) {
-  // (q*, -(q* (x) t)) with rotate() spelled out in the device's operation order (host code is
-  // compiled without FMA contraction, see Makefile)
-  const float w = T7[0];
-  const V3 cv = V3{-T7[1], -T7[2], -T7[3]};
-  const V3 t = V3{T7[4], T7[5], T7[6]};
-  V3 uv = V3{cv.y * t.z - cv.z * t.y, cv.z * t.x - cv.x * t.z, cv.x * t.y - cv.y * t.x};
-  uv = V3{uv.x + uv.x, uv.y + uv.y, uv.z + uv.z};
-  const V3 cr = V3{cv.y * uv.z - cv.z * uv.y, cv.z * uv.x - cv.x * uv.z, cv.x * uv.y - cv.y * uv.x};
-  const V3 r = V3{(t.x + w * uv.x) + cr.x, (t.y + w * uv.y) + cr.y, (t.z + w * uv.z) + cr.z};
-  Xform Ti;
-  Ti.w = w;
-  Ti.v = cv;
-  Ti.t = V3{-r.x, -r.y, -r.z};
-  return Ti;
-}
-
 // Builds the per-pose clouds on the device: ctx->mesh_pts_c / mesh_cols_c, offsets in *offs.
 static int32_t mesh_frames_device(cg_context* ctx, const cg_mesh* m, float vs, size_t F,
                                   const float* poses, const double* stamps,
@@ -318,7 +301,7 @@ static int32_t mesh_frames_device(cg_context* ctx, const cg_mesh* m, float vs, s
     const double id = stamps[i] == stamps[0] ? 0 : round((stamps[i] - stamps[0]) / 0.05);
     const uint32_t bucket = static_cast<uint8_t>(static_cast<long long>(id));
     const uint64_t p0 = h_first[bucket], p1 = h_first[bucket + 1];
-    fm[i].T_C_G = inverse_pose_host(poses + 7 * i);
+    fm[i].T_C_G = inverse_xform_host(make_xform(poses + 7 * i));
     fm[i].src = p0;
     fm[i].dst = run;
     fm[i].n = static_cast<uint32_t>(p1 - p0);

@@ -80,16 +80,6 @@ def test_batch_split_path(gpu_ctx, monkeypatch):
     gl.close()
 
 
-def test_batch_pipelined_transfer(gpu_ctx, monkeypatch):
-    """Host-pointer batches are copied group by group on a second stream while earlier groups
-    are fused; the result is the one of the plain sequence."""
-    monkeypatch.setenv("CG_H2D_CHUNK_POINTS", "3000")
-    frames = util.small_frames(6, stride=8)
-    got, ref, gl = _run_both(gpu_ctx, frames, batch=True)
-    util.compare_layers(got, ref, "pipelined batch")
-    gl.close()
-
-
 def test_far_points_regroup_then_out_of_range(gpu_ctx):
     """The bundle keys cover the box of voxels (relative to the sensor) that earlier jobs measured;
     a point outside it makes the library redo the group with the measured extent instead of
