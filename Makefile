@@ -11,8 +11,9 @@ NVFLAGS = $(ARCH) -DCG_DEFAULT_ALPHA=$(DEFAULT_ALPHA) -O3 -std=c++17 -lineinfo -
 SRC  = coxgraph_b200/csrc
 OBJ  = build/obj
 LIB  = coxgraph_b200/lib/libcoxgraph_b200.so
-HDRS = $(SRC)/cg_math.cuh $(SRC)/cg_internal.cuh $(SRC)/host_stage.cuh $(SRC)/cg_raycast_direct.cuh include/coxgraph_b200.h
-OBJS = $(OBJ)/layer.o $(OBJ)/integrate.o $(OBJ)/merge.o $(OBJ)/exchange.o $(OBJ)/comm.o $(OBJ)/mesh_recover.o $(OBJ)/mesh.o $(OBJ)/mesh_connect.o $(OBJ)/esdf.o $(OBJ)/host_stage.o $(OBJ)/selftest.o
+HDRS = $(SRC)/cg_math.cuh $(SRC)/cg_internal.cuh $(SRC)/host_stage.cuh $(SRC)/cg_raycast_direct.cuh \
+       $(SRC)/integrate.cuh include/coxgraph_b200.h
+OBJS = $(OBJ)/layer.o $(OBJ)/integrate.o $(OBJ)/integrate_front.o $(OBJ)/integrate_back.o $(OBJ)/merge.o $(OBJ)/exchange.o $(OBJ)/comm.o $(OBJ)/mesh_recover.o $(OBJ)/mesh.o $(OBJ)/mesh_connect.o $(OBJ)/esdf.o $(OBJ)/host_stage.o $(OBJ)/selftest.o
 
 HOSTCHK = build/host_api_check
 

@@ -211,8 +211,8 @@ struct PendingEvent {
   cudaEvent_t start, stop;
 };
 
-// Everything a job's layer-independent front half (points -> one ray per bundle, integrate.cu)
-// writes and its back half reads.  The context is set 0 (plain calls); cg_prepare_batch_* uses
+// Everything a job's layer-independent front half (points -> one ray per bundle,
+// integrate_front.cu) writes and its back half reads.  The context is set 0 (plain calls); cg_prepare_batch_* uses
 // further sets on a second stream so that the front half of a later job overlaps the back half of
 // the current one.
 struct FrontBufs {
@@ -269,7 +269,7 @@ struct cg_context : cg::FrontBufs {
   cg::DevBuf seg_keys_a, seg_keys_b, seg_idx_a, seg_idx_b, seg_recs;  // (ray, block) segments
   cg::DevBuf seg_order;  // update lists in size-class order
   cg::DevBuf seg_bins;
-  // per-call touch set (integrate.cu "back half"): kept all-clear between calls
+  // per-call touch set (integrate_back.cu): kept all-clear between calls
   cg::DevBuf touch_ord, touch_entry, touch_acc, touch_bits;
   uint32_t* d_touch_count = nullptr;  // [0] blocks touched, [1] general (voxel, ray) keys emitted
   uint32_t* d_walk_counters = nullptr;  // [0],[1] dynamic work counters, [2] bundle key reach

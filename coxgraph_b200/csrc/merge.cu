@@ -756,9 +756,9 @@ static void fill_desc(BatchSubmap& d, const cg_layer* A, const float* pose, uint
 // Puts `count` descriptors into ctx->batch_desc (pinned, device-mapped staging + a copy kernel)
 // and resets the merge counters of the call behind them.  The host writes ctx->h_tables only while
 // no queued kernel reads it: every call that stages through it (the projections here and
-// integrate.cu's upload_frame_tables) ends, on success, in finish_call's stream synchronise.  An
-// error return may leave the copy queued; the CUDA errors that end a call early are sticky, so no
-// later call gets as far as writing the table.
+// integrate_front.cu's upload_frame_tables) ends, on success, in finish_call's stream
+// synchronise.  An error return may leave the copy queued; the CUDA errors that end a call early
+// are sticky, so no later call gets as far as writing the table.
 static int32_t upload_descs(cg_context* ctx, const BatchSubmap* descs, size_t count) {
   const size_t desc_bytes = count * sizeof(BatchSubmap);
   if (desc_bytes > ctx->h_tables_cap) {

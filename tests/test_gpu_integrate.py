@@ -285,9 +285,21 @@ def test_prepared_jobs_equal_plain_calls(gpu_ctx):
     stream, own scratch set) before job k is completed.  Same layer, bit for bit, as the plain
     cg_integrate_batch_device calls; a job the fast path cannot take (a point outside the
     bundle-key box) silently goes the plain way."""
+    _prepared_vs_plain(gpu_ctx)
+
+
+@pytest.mark.parametrize("over", [{"method": 0}, {"enable_anti_grazing": 1}],
+                         ids=["simple", "merged_anti_grazing"])
+def test_prepared_jobs_equal_plain_calls_other_configs(gpu_ctx, over):
+    """The same for the SIMPLE integrator and for the merged one with anti-grazing: the prepared
+    path then queues a front half without bundles, or one that also builds the grazing set."""
+    _prepared_vs_plain(gpu_ctx, **over)
+
+
+def _prepared_vs_plain(gpu_ctx, **over):
     import torch
     from coxgraph_b200 import Layer, TsdfIntegrator
-    _, gcfg = util.make_cfgs()
+    _, gcfg = util.make_cfgs(**over)
     dev = torch.device("cuda", 0)
     jobs = []
     for k in range(4):
