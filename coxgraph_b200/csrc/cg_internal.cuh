@@ -315,6 +315,9 @@ struct cg_context : cg::FrontBufs {
     int freespace = 0;
     float voxel_size = 0.0f;
     bool front_queued = false;   // false: the job did not fit the one-group fast path
+    // completes the staged copy of d_points / d_colors (cg_prepare_batch_staged); the job waits
+    // on it only when it runs the plain way, on the context's stream
+    cudaEvent_t inputs_ready = nullptr;
   } prepared[2];
   double stage_ms[cg::kNumStages] = {};
   uint64_t stage_launches[cg::kNumStages] = {};

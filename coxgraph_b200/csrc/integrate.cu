@@ -149,11 +149,13 @@ static int32_t integrate_group(cg_layer* L, const cg_integrator_config* cfg,
 // its own and completed by `queued_done` (h_poses / offs are then that job's copies).  It is used
 // when it came out right; otherwise — a point outside the key box, too many voxel visits for one
 // group, a ray out of range — it is dropped and the job runs the plain way, which regroups,
-// retries and reports.
+// retries and reports.  `inputs_ready`: the staged copy of d_points / d_colors, which the plain way
+// must wait for (a queued front half already did).
 static int32_t integrate_job(cg_layer* L, const cg_integrator_config* cfg, size_t F,
                              const float* h_poses, const float* d_points, const uint8_t* d_colors,
                              const uint64_t* offs, int freespace, cg_integrate_stats* stats,
-                             const FrontBufs* queued = nullptr, cudaEvent_t queued_done = nullptr) {
+                             const FrontBufs* queued = nullptr, cudaEvent_t queued_done = nullptr,
+                             cudaEvent_t inputs_ready = nullptr) {
   if (!L || !cfg || !h_poses || !offs || (offs[F] > offs[0] && (!d_points || !d_colors))) {
     set_error("cg_integrate: null argument");
     return CG_ERR_INVALID_ARG;
@@ -180,6 +182,7 @@ static int32_t integrate_job(cg_layer* L, const cg_integrator_config* cfg, size_
     }
   }
   if (!done) {
+    if (inputs_ready) CG_CUDA(cudaStreamWaitEvent(ctx->stream, inputs_ready, 0));
     // poses and frame offsets (relative to the job's first point) go up once per job
     rc = upload_frame_tables(*ctx, F, h_poses, offs, ctx->stream);
     if (rc) return rc;
@@ -267,6 +270,7 @@ static int32_t prepare_job(cg_layer* L, const cg_integrator_config* cfg, size_t 
   pj.d_colors = d_cols ? d_cols + 4 * offs[0] : nullptr;
   pj.freespace = freespace;
   pj.voxel_size = L->v.voxel_size;
+  pj.inputs_ready = inputs_ready;
   const size_t total = pj.offs[F];
   // the fast path: a valid merged / simple job that is one group; everything else is left to the
   // plain path inside cg_integrate_prepared (which also reports the errors)
@@ -329,7 +333,7 @@ int32_t cg_integrate_prepared(cg_layer* L, int32_t slot, cg_integrate_stats* sta
   const bool usable = pj.front_queued && pj.voxel_size == L->v.voxel_size;
   return integrate_job(L, &pj.cfg, pj.offs.size() - 1, pj.poses.data(), pj.d_points, pj.d_colors,
                        pj.offs.data(), pj.freespace, stats, usable ? &ctx->prep[slot] : nullptr,
-                       ctx->prep_done[slot]);
+                       ctx->prep_done[slot], pj.inputs_ready);
 }
 
 void cg_integrator_config_default(cg_integrator_config* c) {

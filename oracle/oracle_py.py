@@ -15,6 +15,10 @@ _LIB_PATH = os.path.join(_HERE, "_build", "libtsdf_oracle.so")
 VOXELS_PER_BLOCK = 4096
 VOXEL_DTYPE = np.dtype([("distance", "<f4"), ("weight", "<f4"), ("rgba", "u1", (4,))])
 assert VOXEL_DTYPE.itemsize == 12
+# orc_visit: one updateTsdfVoxel call (global voxel index, sdf, effective weight, ray colour)
+VISIT_DTYPE = np.dtype([("idx", "<i4", (3,)), ("sdf", "<f4"), ("weight", "<f4"),
+                        ("rgba", "u1", (4,))])
+assert VISIT_DTYPE.itemsize == 24
 
 
 class IntegratorConfig(C.Structure):
@@ -83,6 +87,12 @@ def lib():
         L.orc_integrate_pointcloud.argtypes = [
             C.c_void_p, C.POINTER(IntegratorConfig), C.c_void_p, C.c_void_p, C.c_void_p,
             C.c_size_t, C.c_int32, C.POINTER(C.c_uint64)]
+        L.orc_integrate_pointcloud_traced.restype = C.c_int32
+        L.orc_integrate_pointcloud_traced.argtypes = [
+            C.c_void_p, C.POINTER(IntegratorConfig), C.c_void_p, C.c_void_p, C.c_void_p,
+            C.c_size_t, C.c_int32, C.POINTER(C.c_uint64), C.POINTER(C.c_void_p),
+            C.POINTER(C.c_size_t)]
+        L.orc_trace_free.argtypes = [C.c_void_p]
         L.orc_integrate_pointcloud_mt.restype = C.c_int32
         L.orc_integrate_pointcloud_mt.argtypes = [
             C.c_void_p, C.POINTER(IntegratorConfig), C.c_void_p, C.c_void_p, C.c_void_p,
@@ -181,11 +191,28 @@ class Layer:
     def num_blocks(self):
         return lib().orc_layer_num_blocks(self._h)
 
-    def integrate(self, cfg, T_G_C, points, colors, freespace=False, threads=0):
+    def integrate(self, cfg, T_G_C, points, colors, freespace=False, threads=0, trace=False):
+        """integratePointCloud.  trace=True (single thread only) returns every voxel update of
+        the call in order as a VISIT_DTYPE array."""
         pts = _f32(points, (-1, 3))
         cols = np.ascontiguousarray(colors, dtype=np.uint8).reshape(-1, 4)
         assert len(pts) == len(cols)
         T = _f32(T_G_C, (7,))
+        if trace and threads and threads > 0:
+            raise ValueError("the visit trace needs the single-threaded integrator (threads=0)")
+        if trace:
+            touched, buf, n = C.c_uint64(0), C.c_void_p(), C.c_size_t(0)
+            rc = lib().orc_integrate_pointcloud_traced(self._h, C.byref(cfg), _ptr(T), _ptr(pts),
+                                                       _ptr(cols), len(pts), int(freespace),
+                                                       C.byref(touched), C.byref(buf), C.byref(n))
+            if rc != 0:
+                raise RuntimeError(f"oracle integrate failed rc={rc}")
+            self.last_blocks_touched = touched.value
+            out = np.zeros(n.value, VISIT_DTYPE)
+            if n.value:
+                C.memmove(out.ctypes.data, buf, n.value * VISIT_DTYPE.itemsize)
+                lib().orc_trace_free(buf)
+            return out
         if threads and threads > 0:
             rc = lib().orc_integrate_pointcloud_mt(self._h, C.byref(cfg), _ptr(T), _ptr(pts),
                                                    _ptr(cols), len(pts), int(freespace), threads)

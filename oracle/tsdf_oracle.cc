@@ -16,6 +16,7 @@
 #include <algorithm>
 #include <atomic>
 #include <cmath>
+#include <cstdlib>
 #include <cstring>
 #include <deque>
 #include <memory>
@@ -304,6 +305,7 @@ struct RayCaster {
 struct Cfg {
   orc_integrator_config c;
   float voxel_size, voxel_size_inv, vps_inv;
+  std::vector<orc_visit>* trace = nullptr;  // every update_voxel call, in order (single thread)
 };
 
 // R1 isPointValid (+ non-finite points are dropped, as voxblox_ros TsdfServer does before
@@ -354,6 +356,10 @@ inline void update_voxel(const Cfg& cfg, V3 origin, V3 point_G, L3 gvi, Color co
   if (cfg.c.use_sparsity_compensation_factor) {
     if (std::fabs(sdf) < trunc) updated_weight *= cfg.c.sparsity_compensation_factor;
   }
+  if (cfg.trace)
+    cfg.trace->push_back(orc_visit{static_cast<int32_t>(gvi.x), static_cast<int32_t>(gvi.y),
+                                   static_cast<int32_t>(gvi.z), sdf, updated_weight,
+                                   {color.r, color.g, color.b, color.a}});
   auto guard = lock(gvi);
   (void)guard;
   const float new_weight = voxel->weight + updated_weight;
@@ -983,11 +989,13 @@ void orc_layer_upload(orc_layer* l, const int32_t* idx, const void* voxels, cons
   }
 }
 
-int32_t orc_integrate_pointcloud(orc_layer* layer, const orc_integrator_config* c,
-                                 const float T[7], const float* pts, const uint8_t* cols,
-                                 size_t n, int32_t freespace, uint64_t* touched) {
+static int32_t integrate_single(orc_layer* layer, const orc_integrator_config* c,
+                                const float T[7], const float* pts, const uint8_t* cols,
+                                size_t n, int32_t freespace, uint64_t* touched,
+                                std::vector<orc_visit>* trace) {
   if (!layer || !c || !T || (n && (!pts || !cols))) return -1;
-  const Cfg cfg = make_cfg(layer, c);
+  Cfg cfg = make_cfg(layer, c);
+  cfg.trace = trace;
   const Xform X = load_xform(T);
   switch (c->method) {
     case 0:
@@ -999,6 +1007,31 @@ int32_t orc_integrate_pointcloud(orc_layer* layer, const orc_integrator_config* 
   }
   return -2;
 }
+
+int32_t orc_integrate_pointcloud(orc_layer* layer, const orc_integrator_config* c,
+                                 const float T[7], const float* pts, const uint8_t* cols,
+                                 size_t n, int32_t freespace, uint64_t* touched) {
+  return integrate_single(layer, c, T, pts, cols, n, freespace, touched, nullptr);
+}
+
+int32_t orc_integrate_pointcloud_traced(orc_layer* layer, const orc_integrator_config* c,
+                                        const float T[7], const float* pts, const uint8_t* cols,
+                                        size_t n, int32_t freespace, uint64_t* touched,
+                                        orc_visit** trace, size_t* num_visits) {
+  if (!trace || !num_visits) return -1;
+  *trace = nullptr;
+  *num_visits = 0;
+  std::vector<orc_visit> rec;
+  const int32_t rc = integrate_single(layer, c, T, pts, cols, n, freespace, touched, &rec);
+  if (rc != 0 || rec.empty()) return rc;
+  *trace = static_cast<orc_visit*>(std::malloc(rec.size() * sizeof(orc_visit)));
+  if (!*trace) return -3;
+  std::memcpy(*trace, rec.data(), rec.size() * sizeof(orc_visit));
+  *num_visits = rec.size();
+  return 0;
+}
+
+void orc_trace_free(orc_visit* trace) { std::free(trace); }
 
 int32_t orc_integrate_pointcloud_mt(orc_layer* layer, const orc_integrator_config* c,
                                     const float T[7], const float* pts, const uint8_t* cols,

@@ -75,6 +75,25 @@ int32_t orc_integrate_pointcloud(orc_layer* layer, const orc_integrator_config* 
                                  const uint8_t* colors_rgba, size_t n,
                                  int32_t freespace_points, uint64_t* blocks_touched);
 
+/* One call of updateTsdfVoxel: the global voxel index, the signed distance, the weight after
+ * drop-off and sparsity compensation, and the ray colour. */
+typedef struct orc_visit {
+  int32_t x, y, z;
+  float sdf;
+  float weight;
+  uint8_t rgba[4];
+} orc_visit;
+
+/* orc_integrate_pointcloud that also records every voxel update, in call order (anti-grazing
+ * skips are not updates).  The arithmetic is the same.  On success *trace is a malloc'd array of
+ * *num_visits records (free it with orc_trace_free). */
+int32_t orc_integrate_pointcloud_traced(orc_layer* layer, const orc_integrator_config* cfg,
+                                        const float T_G_C[7], const float* points_xyz,
+                                        const uint8_t* colors_rgba, size_t n,
+                                        int32_t freespace_points, uint64_t* blocks_touched,
+                                        orc_visit** trace, size_t* num_visits);
+void orc_trace_free(orc_visit* trace);
+
 /* Timing variant: voxblox-style threading (striped voxel mutexes, allocation mutex).
  * Result is order-nondeterministic like the real thing; used only as CPU baseline. */
 int32_t orc_integrate_pointcloud_mt(orc_layer* layer, const orc_integrator_config* cfg,

@@ -55,9 +55,10 @@ def test_one_giant_bundle(gpu_ctx):
 
 @pytest.mark.parametrize("carving", [1, 0])
 def test_thousands_of_updates_per_voxel(gpu_ctx, carving):
-    """300 frames of the same small cluster from the same pose: every voxel on the way gets
-    > 2048 updates (free-space ones near the sensor: the closed form; band ones: ordered replay
-    across sub-blocks), all in one job."""
+    """300 frames of the same small cluster from the same pose, all in one job: the free-space
+    voxels near the sensor get > 2048 updates (the fixed-point sum), the band ones up to about
+    1400 (the warp replay).  Band lists of 2048 or more are in test_gpu_update_paths.py; the
+    closed form of k_long_finish is never reached (DESIGN §4.2)."""
     rng = np.random.default_rng(5)
     base = np.array([0.3, -0.2, 1.4])
     frames = []

@@ -296,6 +296,53 @@ def test_prepared_jobs_equal_plain_calls_other_configs(gpu_ctx, over):
     _prepared_vs_plain(gpu_ctx, **over)
 
 
+@pytest.mark.parametrize("way", ["fast", "groups", "other_voxel_size"])
+def test_prepared_staged_jobs_equal_plain_calls(gpu_ctx, monkeypatch, way):
+    """cg_prepare_batch_staged: the inputs come from cg_stage_batch_async's copy stream.  "fast":
+    the queued front half waits for the copy.  "groups" (CG_MAX_GROUP_POINTS below the job) and
+    "other_voxel_size" (integrated through a second integrator whose layer has another voxel size,
+    so the queued front half is dropped) run the job the plain way on the context's stream, which
+    must wait for the copy too.  The slot first holds cloud X, which is integrated; then cloud Y
+    (same point count: nothing is reallocated, so a read that does not wait sees X's points, which
+    are valid points) — 25 full frames, long enough a copy for an unordered read to overtake it —
+    is staged, prepared and integrated at once.  The layer must be a plain integrateBatch of Y."""
+    _staged_vs_plain(gpu_ctx, monkeypatch, way)
+
+
+def _staged_vs_plain(gpu_ctx, monkeypatch, way):
+    import torch
+    from coxgraph_b200 import Layer, TsdfIntegrator
+    _, gcfg = util.make_cfgs()
+    clouds = []
+    for robot, submap in ((0, 0), (1, 2)):  # X, Y
+        frames = util.small_frames(25, stride=1, robot=robot, submap=submap)
+        poses = np.stack([T for (T, _, _) in frames]).astype(np.float32)
+        p = torch.from_numpy(np.concatenate([p for (_, p, _) in frames])).pin_memory().numpy()
+        c = torch.from_numpy(np.concatenate([c for (_, _, c) in frames])).pin_memory().numpy()
+        offs = np.cumsum([0] + [len(p_) for (_, p_, _) in frames]).astype(np.uint64)
+        clouds.append((poses, p, c, offs))
+    (px, xp, xc, xo), (py, yp, yc, yo) = clouds
+    assert len(xp) == len(yp)
+    if way == "groups":
+        monkeypatch.setenv("CG_MAX_GROUP_POINTS", str(int(yo[-1]) // 3))
+    vs = 0.1 if way == "other_voxel_size" else 0.05
+    scratch = Layer(gpu_ctx, 0.05, max_blocks=16384)
+    ix = TsdfIntegrator(gcfg, scratch)
+    ix.stageBatch(0, xp, xc)
+    ix.integrateStaged(0, px, xo)
+    target, ref = Layer(gpu_ctx, vs, max_blocks=16384), Layer(gpu_ctx, vs, max_blocks=16384)
+    it = TsdfIntegrator(gcfg, target)
+    prep = ix if way == "other_voxel_size" else it  # the slots belong to the context
+    prep.stageBatch(0, yp, yc)
+    prep.prepareStaged(1, 0, py, yo)
+    st = it.integratePrepared(1)
+    assert st.points_in == int(yo[-1]) and st.rays > 0
+    TsdfIntegrator(gcfg, ref).integrateBatch(py, yp, yc, yo)
+    util.compare_layers(target.download(), ref.download(), f"staged job ({way}) vs plain", exact=True)
+    for L in (scratch, target, ref):
+        L.close()
+
+
 def _prepared_vs_plain(gpu_ctx, **over):
     import torch
     from coxgraph_b200 import Layer, TsdfIntegrator

@@ -1,4 +1,7 @@
-"""GPU parity: cg_merge_layer_into_layer / cg_project_submaps against the CPU oracle.
+"""GPU parity: cg_merge_layer_into_layer / cg_project_submaps against the CPU oracle.  Both sides
+merge the same input layers, so the results must be bit-identical (distance, weight, colour and
+block flags); only test_integrate_then_merge_end_to_end, whose inputs are fused separately, is
+held to the tolerance.
 Reference call sites: coxgraph/src/client/map_server.cpp:59-73,
 coxgraph/src/server/visualizer/server_visualizer.cpp:123-126."""
 import numpy as np
@@ -51,8 +54,7 @@ def test_merge_matches_oracle(gpu_ctx, pose_id):
         assert st.blocks_out == ob.last_blocks_out
         assert st.blocks_in == oa.num_blocks
         util.compare_layers(gb.download(), ob.download(), f"merge pose {pose_id} rep {rep}",
-                            check_flags=True)
-    assert util.exact_fraction(gb.download(), ob.download()) > 0.999
+                            exact=True, check_flags=True)
     ga.close()
     gb.close()
 
@@ -74,12 +76,12 @@ def test_merge_between_different_voxel_sizes(gpu_ctx, src_voxel, dst_voxel):
     ob.merge_from(subs_o[0], poses[0])
     st = mergeLayerAintoLayerB(subs_g[0], poses[0], gb)
     assert st.blocks_out == ob.last_blocks_out
-    util.compare_layers(gb.download(), ob.download(), "single merge", check_flags=True)
+    util.compare_layers(gb.download(), ob.download(), "single merge", exact=True, check_flags=True)
     og, gg = orc.Layer(dst_voxel), Layer(gpu_ctx, dst_voxel, max_blocks=16384)
     for o, T in zip(subs_o, poses):
         og.merge_from(o, T)
     getProjectedMap(subs_g, np.stack(poses), gg)
-    util.compare_layers(gg.download(), og.download(), "projection", check_flags=True)
+    util.compare_layers(gg.download(), og.download(), "projection", exact=True, check_flags=True)
     for L in subs_g + [gb, gg]:
         L.close()
 
@@ -102,8 +104,8 @@ def test_dense_submaps_project_matches_oracle(gpu_ctx):
     gg = Layer(gpu_ctx, 0.05, max_blocks=8192)
     st = getProjectedMap(subs_g, np.stack(poses), gg, want_stats=True)
     assert st.blocks_in == sum(ol.num_blocks for ol in subs_o)
-    util.compare_layers(gg.download(), og.download(), "dense projection", check_flags=True)
-    assert util.exact_fraction(gg.download(), og.download()) > 0.999
+    util.compare_layers(gg.download(), og.download(), "dense projection", exact=True,
+                        check_flags=True)
     for g in subs_g + [gg]:
         g.close()
 
@@ -124,7 +126,7 @@ def test_project_submaps_matches_sequential_oracle(gpu_ctx):
     gg = Layer(gpu_ctx, 0.05, max_blocks=8192)
     st = getProjectedMap(gsubs, np.stack(poses), gg, want_stats=True)
     assert st.blocks_in == sum(s.num_blocks for s in subs)
-    util.compare_layers(gg.download(), og.download(), "projected map", check_flags=True)
+    util.compare_layers(gg.download(), og.download(), "projected map", exact=True, check_flags=True)
     # re-projection after a pose update (config 5): fresh global layer, perturbed poses
     rng = np.random.default_rng(synth.SEED)
     poses2 = [synth.perturb_pose(T, rng) for T in poses]
@@ -133,7 +135,8 @@ def test_project_submaps_matches_sequential_oracle(gpu_ctx):
     for s, T in zip(subs, poses2):
         og.merge_from(s, T)
     getProjectedMap(gsubs, np.stack(poses2), gg)
-    util.compare_layers(gg.download(), og.download(), "re-projected map")
+    util.compare_layers(gg.download(), og.download(), "re-projected map", exact=True,
+                        check_flags=True)
     for g in gsubs + [gg]:
         g.close()
 
