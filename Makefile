@@ -13,11 +13,12 @@ OBJ  = build/obj
 LIB  = coxgraph_b200/lib/libcoxgraph_b200.so
 HDRS = $(SRC)/cg_math.cuh $(SRC)/cg_internal.cuh $(SRC)/host_stage.cuh $(SRC)/cg_raycast_direct.cuh \
        $(SRC)/integrate.cuh include/coxgraph_b200.h
-OBJS = $(OBJ)/layer.o $(OBJ)/integrate.o $(OBJ)/integrate_front.o $(OBJ)/integrate_back.o $(OBJ)/merge.o $(OBJ)/exchange.o $(OBJ)/comm.o $(OBJ)/mesh_recover.o $(OBJ)/mesh.o $(OBJ)/mesh_connect.o $(OBJ)/esdf.o $(OBJ)/host_stage.o $(OBJ)/selftest.o
+OBJS = $(OBJ)/layer.o $(OBJ)/integrate.o $(OBJ)/integrate_front.o $(OBJ)/integrate_back.o $(OBJ)/integrate_depth.o $(OBJ)/merge.o $(OBJ)/exchange.o $(OBJ)/comm.o $(OBJ)/mesh_recover.o $(OBJ)/mesh.o $(OBJ)/mesh_connect.o $(OBJ)/esdf.o $(OBJ)/host_stage.o $(OBJ)/selftest.o
 
 HOSTCHK = build/host_api_check
+DEPTHCHK = build/depth_api_check
 
-all: $(LIB) oracle $(HOSTCHK)
+all: $(LIB) oracle $(HOSTCHK) $(DEPTHCHK)
 
 $(OBJ)/%.o: $(SRC)/%.cu $(HDRS)
 	@mkdir -p $(OBJ)
@@ -33,6 +34,11 @@ oracle:
 # C++ host API driver (tests/test_host_cpp.py): plain g++, links only the C ABI
 $(HOSTCHK): tests/host/host_api_check.cc coxgraph_b200/host/coxgraph_b200.hpp include/coxgraph_b200.h $(LIB)
 	g++ -std=c++17 -O1 -Wall -Wextra tests/host/host_api_check.cc -o $@ -Lcoxgraph_b200/lib \
+	    -lcoxgraph_b200 -Wl,-rpath,'$$ORIGIN/../coxgraph_b200/lib'
+
+# C++ depth-image driver (tests/test_host_depth.py)
+$(DEPTHCHK): tests/host/depth_api_check.cc coxgraph_b200/host/coxgraph_b200.hpp include/coxgraph_b200.h $(LIB)
+	g++ -std=c++17 -O1 -Wall -Wextra tests/host/depth_api_check.cc -o $@ -Lcoxgraph_b200/lib \
 	    -lcoxgraph_b200 -Wl,-rpath,'$$ORIGIN/../coxgraph_b200/lib'
 
 clean:

@@ -5,6 +5,6 @@ lib/libcoxgraph_b200.so); `api` mirrors the reference-facing interface on top of
 generates the synthetic depth streams of the benchmark.  Nothing here falls back to the CPU.
 """
 from . import capi  # noqa: F401
-from .api import (Context, Layer, esdfConfig, TsdfIntegrator, TsdfIntegratorConfig,  # noqa: F401
+from .api import (Context, Layer, depthCamera, esdfConfig, TsdfIntegrator, TsdfIntegratorConfig,  # noqa: F401
                   getProjectedMap, mergeLayerAintoLayerB, meshToFrames, recoverMesh,
                   reprojectSubmaps, VOXEL_DTYPE)

@@ -423,6 +423,120 @@ def _integrate_prepared(self, slot):
     return self.last_stats
 
 
+def depthCamera(camera):
+    """capi.DepthCamera from a DepthCamera, or from a dict with width, height, fx, fy, cx, cy (e.g.
+    synth.CAM_640x480) and optional depth_encoding ("16UC1" / "32FC1", default "16UC1") and
+    color_encoding ("rgb8", "rgba8", "bgr8", "bgra8", "mono8", default "rgb8")."""
+    if isinstance(camera, capi.DepthCamera):
+        return camera
+
+    def enc(v, table):
+        return table[v] if isinstance(v, str) else int(v)
+    return capi.DepthCamera(int(camera["width"]), int(camera["height"]), float(camera["fx"]),
+                            float(camera["fy"]), float(camera["cx"]), float(camera["cy"]),
+                            enc(camera.get("depth_encoding", "16UC1"), capi.DEPTH_ENCODINGS),
+                            enc(camera.get("color_encoding", "rgb8"), capi.COLOR_ENCODINGS))
+
+
+def _depth_images(cam, F, depth, color, device):
+    """Checks the images of F frames against the camera; numpy arrays (host) are made contiguous.
+    -> (depth, color, pointer of depth, pointer of color)."""
+    n = F * cam.width * cam.height
+    depth_item = 2 if cam.depth_encoding == capi.DEPTH_16UC1 else 4
+    color_bytes = n * capi.COLOR_PIXEL_BYTES.get(cam.color_encoding, 0)
+    if device:
+        assert _is_cuda_tensor(depth) and _is_cuda_tensor(color)
+        assert depth.is_contiguous() and color.is_contiguous()
+        ok = (depth.numel() == n and depth.element_size() == depth_item and
+              color.numel() * color.element_size() == color_bytes)
+        ptrs = (C.c_void_p(depth.data_ptr()), C.c_void_p(color.data_ptr()))
+    else:
+        dtype = np.uint16 if cam.depth_encoding == capi.DEPTH_16UC1 else np.float32
+        depth = np.ascontiguousarray(depth, dtype)
+        color = np.ascontiguousarray(color, np.uint8)
+        ok = depth.size == n and color.size == color_bytes
+        ptrs = (_ptr(depth), _ptr(color))
+    if not ok:
+        raise ValueError(f"images do not match {F} frames of {cam.width} x {cam.height} with the "
+                         "camera's encodings")
+    return depth, color, ptrs[0], ptrs[1]
+
+
+def _integrate_depth_batch(self, poses, depth, color, camera):
+    """F TsdfServer insertions of registered depth + colour images (depth_image_proc
+    point_cloud_xyzrgb, the finite filter of convertPointcloud, integratePointCloud) as one job:
+    depth [F,H,W] uint16 (16UC1) or float32 (32FC1), color [F,H,W,C].  numpy arrays (host) or
+    contiguous CUDA tensors (device)."""
+    cam = depthCamera(camera)
+    P = np.ascontiguousarray(poses, np.float32).reshape(-1, 7)
+    device = _is_cuda_tensor(depth)
+    depth, color, dp, cp = _depth_images(cam, len(P), depth, color, device)
+    lib = capi.load()
+    if device:
+        self.layer.ctx.wait_torch()
+        capi.check(lib.cg_integrate_depth_batch_device(self.layer._h, C.byref(self.config), len(P),
+                                                       _ptr(P), C.byref(cam), dp, cp,
+                                                       C.byref(self.last_stats)))
+    else:
+        capi.check(lib.cg_integrate_depth_batch(self.layer._h, C.byref(self.config), len(P), _ptr(P),
+                                                C.byref(cam), dp, cp, C.byref(self.last_stats)))
+    return self.last_stats
+
+
+def _integrate_depth_image(self, T_G_C, depth, color, camera):
+    """One frame of integrateDepthBatch: depth [H,W], color [H,W,C]."""
+    return self.integrateDepthBatch(np.asarray(T_G_C, np.float32).reshape(1, 7), depth, color,
+                                    camera)
+
+
+def _stage_depth(self, slot, depth, color, camera):
+    """Queue the host->device copy of the images of a later integrateDepthStaged /
+    prepareDepthStaged job (pinned numpy arrays; returns at once).  Keep them alive until then."""
+    cam = depthCamera(camera)
+    F = int(np.asarray(depth).size // max(1, cam.width * cam.height))
+    depth, color, dp, cp = _depth_images(cam, F, depth, color, False)
+    capi.check(capi.load().cg_stage_depth_async(self.layer.ctx._h, int(slot), C.byref(cam), F, dp, cp))
+    self._staged = getattr(self, "_staged", {})
+    self._staged[int(slot)] = (depth, color)
+
+
+def _integrate_depth_staged(self, slot, poses, camera):
+    """integrateDepthBatch on the images staged in `slot`."""
+    cam = depthCamera(camera)
+    P = np.ascontiguousarray(poses, np.float32).reshape(-1, 7)
+    capi.check(capi.load().cg_integrate_depth_staged(self.layer._h, C.byref(self.config), len(P),
+                                                     _ptr(P), C.byref(cam), int(slot),
+                                                     C.byref(self.last_stats)))
+    getattr(self, "_staged", {}).pop(int(slot), None)
+    return self.last_stats
+
+
+def _prepare_depth(self, slot, poses, depth, color, camera):
+    """prepareBatch for a depth job (CUDA tensors); integratePrepared(slot) completes it."""
+    cam = depthCamera(camera)
+    P = np.ascontiguousarray(poses, np.float32).reshape(-1, 7)
+    depth, color, dp, cp = _depth_images(cam, len(P), depth, color, True)
+    self.layer.ctx.wait_torch()
+    capi.check(capi.load().cg_prepare_depth_device(self.layer._h, C.byref(self.config), len(P),
+                                                   _ptr(P), C.byref(cam), dp, cp, int(slot)))
+    self._prepared = getattr(self, "_prepared", {})
+    self._prepared[int(slot)] = (depth, color)
+
+
+def _prepare_depth_staged(self, slot, stage_slot, poses, camera):
+    """The same for images staged with stageDepth(stage_slot, ...)."""
+    cam = depthCamera(camera)
+    P = np.ascontiguousarray(poses, np.float32).reshape(-1, 7)
+    capi.check(capi.load().cg_prepare_depth_staged(self.layer._h, C.byref(self.config), len(P),
+                                                   _ptr(P), C.byref(cam), int(stage_slot), int(slot)))
+
+
+TsdfIntegrator.integrateDepthBatch = _integrate_depth_batch
+TsdfIntegrator.integrateDepthImage = _integrate_depth_image
+TsdfIntegrator.stageDepth = _stage_depth
+TsdfIntegrator.integrateDepthStaged = _integrate_depth_staged
+TsdfIntegrator.prepareDepth = _prepare_depth
+TsdfIntegrator.prepareDepthStaged = _prepare_depth_staged
 TsdfIntegrator.stageBatch = _stage_batch
 TsdfIntegrator.integrateStaged = _integrate_staged
 TsdfIntegrator.prepareBatch = _prepare_batch

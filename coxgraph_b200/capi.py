@@ -53,6 +53,24 @@ class IntegrateStats(C.Structure):
                 ("points_beyond_reach", C.c_uint64)]
 
 
+DEPTH_16UC1, DEPTH_32FC1 = 0, 1
+COLOR_RGB8, COLOR_RGBA8, COLOR_BGR8, COLOR_BGRA8, COLOR_MONO8 = 0, 1, 2, 3, 4
+# sensor_msgs/Image encodings -> cg_depth_encoding / cg_color_encoding
+DEPTH_ENCODINGS = {"16UC1": DEPTH_16UC1, "mono16": DEPTH_16UC1, "32FC1": DEPTH_32FC1}
+COLOR_ENCODINGS = {"rgb8": COLOR_RGB8, "rgba8": COLOR_RGBA8, "bgr8": COLOR_BGR8, "bgra8": COLOR_BGRA8,
+                   "mono8": COLOR_MONO8}
+COLOR_PIXEL_BYTES = {COLOR_RGB8: 3, COLOR_RGBA8: 4, COLOR_BGR8: 3, COLOR_BGRA8: 4, COLOR_MONO8: 1}
+
+
+class DepthCamera(C.Structure):
+    """cg_depth_camera: CameraInfo intrinsics as image_geometry::PinholeCameraModel reports them
+    (fx = P[0], fy = P[5], cx = P[2], cy = P[6]) and the encodings of the two images."""
+
+    _fields_ = [("width", C.c_int32), ("height", C.c_int32), ("fx", C.c_double),
+                ("fy", C.c_double), ("cx", C.c_double), ("cy", C.c_double),
+                ("depth_encoding", C.c_int32), ("color_encoding", C.c_int32)]
+
+
 class Mesh(C.Structure):
     """cg_mesh: voxblox_msgs/Mesh (with observation history) flattened into plain arrays."""
 
@@ -163,6 +181,20 @@ SYMBOLS = {
     "cg_prepare_batch_staged": (C.c_int32, [_P, C.POINTER(IntegratorConfig), C.c_size_t, _P,
                                             C.c_int32, _P, C.c_int32, C.c_int32]),
     "cg_integrate_prepared": (C.c_int32, [_P, C.c_int32, C.POINTER(IntegrateStats)]),
+    "cg_integrate_depth_batch": (C.c_int32, [_P, C.POINTER(IntegratorConfig), C.c_size_t, _P,
+                                             C.POINTER(DepthCamera), _P, _P,
+                                             C.POINTER(IntegrateStats)]),
+    "cg_integrate_depth_batch_device": (C.c_int32, [_P, C.POINTER(IntegratorConfig), C.c_size_t, _P,
+                                                    C.POINTER(DepthCamera), _P, _P,
+                                                    C.POINTER(IntegrateStats)]),
+    "cg_stage_depth_async": (C.c_int32, [_P, C.c_int32, C.POINTER(DepthCamera), C.c_size_t, _P, _P]),
+    "cg_integrate_depth_staged": (C.c_int32, [_P, C.POINTER(IntegratorConfig), C.c_size_t, _P,
+                                              C.POINTER(DepthCamera), C.c_int32,
+                                              C.POINTER(IntegrateStats)]),
+    "cg_prepare_depth_device": (C.c_int32, [_P, C.POINTER(IntegratorConfig), C.c_size_t, _P,
+                                            C.POINTER(DepthCamera), _P, _P, C.c_int32]),
+    "cg_prepare_depth_staged": (C.c_int32, [_P, C.POINTER(IntegratorConfig), C.c_size_t, _P,
+                                            C.POINTER(DepthCamera), C.c_int32, C.c_int32]),
     "cg_mesh_to_frames": (C.c_int32, [_P, C.POINTER(Mesh), C.c_float, C.c_size_t, _P, _P, _P, _P, _P,
                                       C.c_size_t]),
     "cg_recover_mesh": (C.c_int32, [_P, C.POINTER(IntegratorConfig), C.POINTER(Mesh), C.c_float,

@@ -177,6 +177,8 @@ struct CallCounters {
   unsigned long long far_dropped;  // ... of the front half the host has just synchronised on
   int err;
   int num_blocks;
+  unsigned long long points_kept;  // depth jobs: kept points of the group (sum of the count table)
+  int hole_sentinel;               // depth jobs: the sentinel ray exists only for the slab holes
 };
 
 // named stages (the reference wraps the same path in voxblox::timing::Timer scopes,
@@ -203,6 +205,7 @@ enum Stage {
   kStageMergeMark,
   kStageMergeResample,
   kStageTransfer,
+  kStageDepthPoints,
   kNumStages
 };
 const char* stage_name(int s);
@@ -233,6 +236,9 @@ struct FrontBufs {
   int* d_key_bounds = nullptr;              // [6] running min / max of the bundle voxel fields
   uint32_t* d_select_count = nullptr;       // output count of the stream compactions
   int32_t* d_front_err = nullptr;           // error bits of a prepared front half (sets > 0)
+  // depth jobs (integrate_depth.cu): a slab of W*H point slots per frame, the kept count of each
+  // frame, and the per-tile counts of the unprojection
+  DevBuf depth_pts, depth_cols, depth_counts, depth_tiles;
   // independent stages of one job side by side (gather || bundle heads + order; short || long
   // update lists): a second stream forked from / joined to the job's stream by events
   cudaStream_t side = nullptr;
@@ -261,6 +267,10 @@ struct cg_context : cg::FrontBufs {
   cg::DevBuf stage_pts[2], stage_cols[2];   // cg_stage_batch_async double buffer
   cudaEvent_t stage_ready[2] = {nullptr, nullptr};
   size_t stage_points[2] = {0, 0};
+  // a slot staged by cg_stage_depth_async holds images (depth in stage_pts, colour in stage_cols)
+  bool stage_is_depth[2] = {false, false};
+  cg_depth_camera stage_cam[2] = {};
+  size_t stage_frames[2] = {0, 0};
   int num_sms = 148;
   // integration scratch
   cg::DevBuf points, colors;
@@ -312,6 +322,7 @@ struct cg_context : cg::FrontBufs {
     std::vector<uint64_t> offs;  // relative to the job's first point
     const float* d_points = nullptr;
     const uint8_t* d_colors = nullptr;
+    const uint32_t* d_counts = nullptr;  // depth jobs: kept points per frame (prep[slot])
     int freespace = 0;
     float voxel_size = 0.0f;
     bool front_queued = false;   // false: the job did not fit the one-group fast path

@@ -73,10 +73,12 @@ cudaError_t fill_bytes(void* p, int byte, size_t bytes, cudaStream_t s);
 // stream `s` into the set `fb`: nothing here touches the layer.  The counters the back half needs
 // (rays, voxel visits, segments, key extent, errors) are copied to fb.h_counters at the end; the
 // caller synchronises.  *need_split: the bundle keys do not fit, the caller halves the group.
+// `d_counts` (depth jobs, else null): the points of job frame f are the first d_counts[f] of its
+// slots [offs[f], offs[f + 1]); the rest are holes.
 int32_t front_enqueue(cg_context* ctx, FrontBufs& fb, cudaStream_t s, int32_t* d_err,
                       const cg_layer* L, const cg_integrator_config* cfg, const IntegratorParams& P,
                       const float* d_points, const uint8_t* d_colors, const uint64_t* offs,
-                      size_t f0, size_t f1, int attempt, bool* need_split);
+                      const uint32_t* d_counts, size_t f0, size_t f1, int attempt, bool* need_split);
 
 enum FrontVerdict { kFrontOk, kFrontRetry, kFrontSplit, kFrontFail };
 
@@ -94,5 +96,17 @@ int32_t upload_frame_tables(FrontBufs& fb, size_t F, const float* h_poses, const
 int32_t run_back_half(cg_context* ctx, const FrontBufs& fb, cg_layer* L, const IntegratorParams& P,
                       uint32_t num_rays, size_t num_pairs, size_t num_segments,
                       cg_integrate_stats* stats);
+
+// ---- depth jobs (integrate_depth.cu)
+// pixels of one depth job at most (F * W * H): the point slots of a job are indexed like a group's
+constexpr size_t kMaxDepthJobPixels = 0x7FFFFFF0ull;
+// CG_OK, or CG_ERR_INVALID_ARG with the error text naming `who`
+int32_t check_depth_camera(const char* who, const cg_depth_camera* cam, size_t F);
+size_t depth_pixel_bytes(const cg_depth_camera& cam);
+size_t color_pixel_bytes(const cg_depth_camera& cam);
+// F frames of images (device memory) -> fb.depth_pts / depth_cols, a slab of W*H slots per frame,
+// and fb.depth_counts[f] = kept points of frame f; two kernels on stream s, stage depth_points
+int32_t unproject_depth(cg_context* ctx, FrontBufs& fb, const cg_depth_camera& cam, size_t F,
+                        const void* d_depth, const uint8_t* d_color, cudaStream_t s);
 
 }  // namespace cg

@@ -96,12 +96,18 @@ __device__ __forceinline__ V3 load_point(const float* pts, size_t i) {
 }
 
 // Frames of one group: offs points at the group's first entry of the job's offset table (F + 1
-// entries are read), base = offs[0]; slots and point indices are relative to the group.
+// entries are read), base = offs[0]; slots and point indices are relative to the group.  counts
+// (depth jobs, else null): the group's entries of the job's kept-count table; frame f's points
+// are then the first counts[f] of its slots, the others are holes.
 struct FrameTable {
   const uint64_t* offs;
   uint64_t base;
   int F;
+  const uint32_t* counts;
   __device__ __forceinline__ uint64_t start(int f) const { return offs[f] - base; }
+  __device__ __forceinline__ int count(int f) const {
+    return counts ? static_cast<int>(counts[f]) : static_cast<int>(start(f + 1) - start(f));
+  }
   __device__ __forceinline__ int frame_of(uint64_t g) const {
     int lo = 0, hi = F;  // start(lo) <= g < start(hi)
     while (hi - lo > 1) {
@@ -137,13 +143,14 @@ __global__ void k_point_keys(IntegratorParams P, KeyLayout kl, const float* __re
     int f = s_first_frame;
     while (f + 1 < ft.F && ft.start(f + 1) <= g) ++f;
     const uint64_t base = ft.start(f);
-    const int n = static_cast<int>(ft.start(f + 1) - base);
+    const int n = ft.count(f);
     const int i = static_cast<int>(g - base);
+    // (a hole, i >= n, keeps its slot: visit_rank(i) = i there)
     const uint32_t k = static_cast<uint32_t>(visit_rank(i, n, P.order_mode));
-    const V3 pc = load_point(pts, g);
+    const V3 pc = i < n ? load_point(pts, g) : V3{0.0f, 0.0f, 0.0f};
     bool clearing = false;
     uint64_t key = kInvalidPointKey;
-    if (point_valid(P, pc, &clearing)) {
+    if (i < n && point_valid(P, pc, &clearing)) {
       const Xform T = make_xform(poses + 7 * f);
       const V3 pg = apply(T, pc);
       const float lim = 524000.0f * P.voxel_size;
@@ -220,7 +227,7 @@ __global__ void k_gather_sorted(KeyLayout kl, int order_mode, const uint64_t* __
   if (key == kInvalidPointKey) return;
   const int f = static_cast<int>(kl.frame(key));
   const uint64_t base = ft.start(f);
-  const int n = static_cast<int>(ft.start(f + 1) - base);
+  const int n = ft.count(f);
   const size_t i = base + order_index(static_cast<int>(kl.rank(key)), n, order_mode);
   out[j] = make_float4(pts[3 * i], pts[3 * i + 1], pts[3 * i + 2], __uint_as_float(cols[i]));
 }
@@ -628,7 +635,8 @@ struct ValidSlot {
   __device__ __forceinline__ bool operator()(uint32_t g) const {
     const int f = ft.frame_of(g);
     const uint64_t base = ft.start(f);
-    const int n = static_cast<int>(ft.start(f + 1) - base);
+    const int n = ft.count(f);
+    if (static_cast<int>(g - base) >= n) return false;  // a hole of a depth job's slab
     bool clearing;
     return point_valid(P, load_point(pts, base + order_index(static_cast<int>(g - base), n,
                                                              P.order_mode)), &clearing);
@@ -645,7 +653,7 @@ __global__ void k_simple_rays(IntegratorParams P, const float* __restrict__ pose
   const uint32_t g = slots[r];
   const int f = ft.frame_of(g);
   const uint64_t base = ft.start(f);
-  const int n = static_cast<int>(ft.start(f + 1) - base);
+  const int n = ft.count(f);
   const size_t i = base + order_index(static_cast<int>(g - base), n, P.order_mode);
   const V3 pc = load_point(pts, i);
   bool clearing = false;
@@ -674,9 +682,16 @@ __device__ __forceinline__ void scan_range(uint32_t n, uint32_t& lo, uint32_t& h
   lo = min(n, blockIdx.x * per);
   hi = min(n, lo + per);
 }
+// CTA 0 also sums a depth job's kept points of the group (kept_counts[0, F)) into
+// c->points_kept (0 for a cloud job, whose count the host knows).  Merged depth jobs: when every
+// dropped key of the group is a hole of a slab (the sentinel bundle starts at slot `kept`), the
+// cloud of the same images has no dropped point and no sentinel ray; c->hole_sentinel = 1 tells
+// the host to leave that ray out of the stats.
 __global__ void __launch_bounds__(kScanThreads)
 k_scan_partials(const uint32_t* __restrict__ num_rays, const unsigned long long* __restrict__ in,
-                unsigned long long* __restrict__ partials) {
+                unsigned long long* __restrict__ partials, const uint32_t* __restrict__ kept_counts,
+                int F, const uint64_t* __restrict__ sorted_keys, const uint32_t* __restrict__ heads,
+                CallCounters* c) {
   typedef cub::BlockReduce<unsigned long long, kScanThreads> Reduce;
   __shared__ typename Reduce::TempStorage tmp;
   uint32_t lo, hi;
@@ -685,6 +700,19 @@ k_scan_partials(const uint32_t* __restrict__ num_rays, const unsigned long long*
   for (uint32_t i = lo + threadIdx.x; i < hi; i += kScanThreads) sum += in[i];
   sum = Reduce(tmp).Sum(sum);
   if (threadIdx.x == 0) partials[blockIdx.x] = sum;
+  if (blockIdx.x != 0) return;
+  unsigned long long kept = 0;
+  if (kept_counts) {
+    __syncthreads();  // tmp is reused
+    for (int f = threadIdx.x; f < F; f += kScanThreads) kept += kept_counts[f];
+    kept = Reduce(tmp).Sum(kept);
+  }
+  if (threadIdx.x == 0) {
+    c->points_kept = kept;
+    const uint32_t nb = *num_rays;
+    c->hole_sentinel = kept_counts && sorted_keys && nb > 0 && heads[nb - 1] == kept &&
+                       sorted_keys[heads[nb - 1]] == kInvalidPointKey;
+  }
 }
 // one CTA: exclusive scan of the partials in place; totals -> counters
 __global__ void __launch_bounds__(1024)
@@ -764,7 +792,7 @@ __global__ void k_grazing_build(KeyLayout kl, const uint64_t* __restrict__ keys,
 int32_t front_enqueue(cg_context* ctx, FrontBufs& fb, cudaStream_t s, int32_t* d_err,
                       const cg_layer* L, const cg_integrator_config* cfg, const IntegratorParams& P,
                       const float* d_points, const uint8_t* d_colors, const uint64_t* offs,
-                      size_t f0, size_t f1, int attempt, bool* need_split) {
+                      const uint32_t* d_counts, size_t f0, size_t f1, int attempt, bool* need_split) {
   *need_split = false;
   const size_t F = f1 - f0;
   const size_t total = offs[f1] - offs[f0];  // points of the group = upper bound on rays
@@ -831,7 +859,9 @@ int32_t front_enqueue(cg_context* ctx, FrontBufs& fb, cudaStream_t s, int32_t* d
   // the job's poses and frame offsets were uploaded once by integrate_job
   const float* pts = d_points + 3 * offs[f0];
   const uint32_t* cols = reinterpret_cast<const uint32_t*>(d_colors) + offs[f0];
-  const FrameTable ft{fb.frame_base.as<uint64_t>() + f0, offs[f0] - offs[0], static_cast<int>(F)};
+  const uint32_t* group_counts = d_counts ? d_counts + f0 : nullptr;
+  const FrameTable ft{fb.frame_base.as<uint64_t>() + f0, offs[f0] - offs[0], static_cast<int>(F),
+                      group_counts};
   fb.group_poses = fb.poses.as<float>() + 7 * f0;
   fb.group_frames = static_cast<int>(F);
   ValidSlot valid{P, ft, pts};
@@ -945,7 +975,10 @@ int32_t front_enqueue(cg_context* ctx, FrontBufs& fb, cudaStream_t s, int32_t* d
     const int sgrid = std::min(1024, ctx->num_sms * 4);
     CG_CUDA(fb.scan_partials.reserve(1024 * sizeof(unsigned long long)));
     k_scan_partials<<<sgrid, kScanThreads, 0, s>>>(d_num, fb.ray_count.as<unsigned long long>(),
-                                                   fb.scan_partials.as<unsigned long long>());
+                                                   fb.scan_partials.as<unsigned long long>(),
+                                                   group_counts, static_cast<int>(F),
+                                                   merged ? dk.Current() : nullptr,
+                                                   fb.scan.as<uint32_t>(), fb.d_counters);
     k_scan_totals<<<1, 1024, 0, s>>>(d_num, fb.scan_partials.as<unsigned long long>(), sgrid,
                                      fb.d_counters, d_err, fb.d_key_bounds);
     k_scan_apply<<<sgrid, kScanThreads, 0, s>>>(d_num, fb.ray_count.as<unsigned long long>(),

@@ -31,7 +31,8 @@ const char* stage_name(int s) {
       "point_keys",    "bundle_sort",  "bundle_scan",      "gather_sorted", "bundle_order",
       "fold_wide",     "fold_bundles", "bundle_rays",      "ray_scan",      "walk_segments",
       "segment_sort",  "block_accumulate", "pair_sort",    "segments",   "visits",   "voxel_update",
-      "replay_wide",   "finalize",     "merge_mark",       "merge_resample", "transfer"};
+      "replay_wide",   "finalize",     "merge_mark",       "merge_resample", "transfer",
+      "depth_points"};
   return (s >= 0 && s < kNumStages) ? names[s] : "?";
 }
 
@@ -432,7 +433,8 @@ void release_front(FrontBufs& fb) {
   DevBuf* bufs[] = {&fb.poses, &fb.frame_base, &fb.key_a, &fb.key_b, &fb.scan, &fb.cub_tmp, &fb.rays,
                     &fb.ray_count, &fb.ray_offset, &fb.sorted_pts, &fb.scan_partials, &fb.ray_id,
                     &fb.frame_count,
-                    &fb.grazing_keys, &fb.grazing_ray_key};
+                    &fb.grazing_keys, &fb.grazing_ray_key, &fb.depth_pts, &fb.depth_cols,
+                    &fb.depth_counts, &fb.depth_tiles};
   for (DevBuf* b : bufs) b->release();
   if (fb.h_counters) cudaFreeHost(fb.h_counters);
   if (fb.d_counters) cudaFree(fb.d_counters);

@@ -23,6 +23,7 @@
 #include <cstdint>
 #include <cstdio>
 #include <cstdlib>
+#include <cstring>
 #include <functional>
 #include <memory>
 #include <stdexcept>
@@ -252,6 +253,46 @@ class TsdfIntegratorBase {
     check(cg_integrate_batch(layer_->handle(), &config_, F, poses.data(),
                              pts.empty() ? nullptr : &pts[0].x, cols.empty() ? nullptr : &cols[0].r,
                              offs.data(), freespace_points ? 1 : 0, &stats_));
+  }
+  // Registered depth + colour images (sensor_msgs/Image pairs of one CameraInfo): the same
+  // layer as depth_image_proc point_cloud_xyzrgb followed by TsdfServer's insertion of that cloud
+  // (its non-finite points dropped).  depth: W*H uint16 (16UC1) or float (32FC1) per frame,
+  // tightly packed; colour: W*H pixels of the camera's colour encoding.
+  struct DepthImage {
+    const void* data;
+  };
+  struct ColorImage {
+    const uint8_t* data;
+  };
+  void integrateDepthImage(const Transformation& T_G_C, const DepthImage& depth,
+                           const ColorImage& color, const cg_depth_camera& camera) {
+    check(cg_integrate_depth_batch(layer_->handle(), &config_, 1, T_G_C.data(), &camera, depth.data,
+                                   color.data, &stats_));
+  }
+  // F frames as one job: depth / colour of frame f at depth[f] / color[f]
+  void integrateDepthImages(const std::vector<Transformation>& T_G_C,
+                            const std::vector<DepthImage>& depth,
+                            const std::vector<ColorImage>& color, const cg_depth_camera& camera) {
+    const size_t F = T_G_C.size();
+    if (depth.size() != F || color.size() != F)
+      fatal_handler()(CG_ERR_INVALID_ARG, "integrateDepthImages: one image pair per pose expected");
+    if (camera.width <= 0 || camera.height <= 0)
+      fatal_handler()(CG_ERR_INVALID_ARG, "integrateDepthImages: invalid image size");
+    const size_t px = static_cast<size_t>(camera.width) * static_cast<size_t>(camera.height);
+    const size_t dsize = camera.depth_encoding == CG_DEPTH_16UC1 ? 2 : 4;
+    const size_t csize = camera.color_encoding == CG_COLOR_MONO8 ? 1
+                         : (camera.color_encoding == CG_COLOR_RGBA8 ||
+                            camera.color_encoding == CG_COLOR_BGRA8) ? 4 : 3;
+    std::vector<uint8_t> d(F * px * dsize), c(F * px * csize);
+    std::vector<float> poses(7 * F);
+    for (size_t f = 0; f < F; ++f) {
+      std::memcpy(&d[f * px * dsize], depth[f].data, px * dsize);
+      std::memcpy(&c[f * px * csize], color[f].data, px * csize);
+      std::copy(T_G_C[f].data(), T_G_C[f].data() + 7, poses.begin() + 7 * f);
+    }
+    check(cg_integrate_depth_batch(layer_->handle(), &config_, F, poses.data(), &camera,
+                                   d.empty() ? nullptr : d.data(), c.empty() ? nullptr : c.data(),
+                                   &stats_));
   }
   // Pipelined jobs for a host that knows its next job (the recover loop does: tsdf_recover.h:
   // 71-86): prepareDevice queues the layer-independent first half of a LATER job — points already

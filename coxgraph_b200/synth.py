@@ -201,6 +201,29 @@ def render_frame(T_G_C, cam=CAM_640x480, device="cpu", near_box=False, stride=1,
     return p_c.contiguous(), colors.contiguous()
 
 
+def render_depth_frame(T_G_C, cam=CAM_640x480, stride=1, scene="room", depth_encoding="16UC1"):
+    """The frame render_frame casts, as the registered images a depth camera driver publishes.
+    Returns (depth, rgb8 uint8 [H,W,3], camera dict): depth is z in millimetres rounded to nearest
+    (uint16 [H,W], 16UC1) or z in metres (float32 [H,W], 32FC1); the colours are the hash colours
+    of render_frame.  With stride > 1 the image is subsampled and the camera's intrinsics are
+    scaled to match (pixel u of the result is pixel u * stride of the full image)."""
+    pts, cols = render_frame(T_G_C, cam=cam, stride=stride, scene=scene)
+    W = len(range(0, cam["width"], stride))
+    H = len(range(0, cam["height"], stride))
+    z = pts[:, 2].numpy().reshape(H, W)
+    if depth_encoding == "16UC1":
+        depth = np.clip(np.rint(z.astype(np.float64) * 1000.0), 0, 65535).astype(np.uint16)
+    elif depth_encoding == "32FC1":
+        depth = z.astype(np.float32)
+    else:
+        raise ValueError(f"unknown depth encoding {depth_encoding}")
+    rgb = cols[:, :3].numpy().reshape(H, W, 3).copy()
+    camera = dict(width=W, height=H, fx=cam["fx"] / stride, fy=cam["fy"] / stride,
+                  cx=cam["cx"] / stride, cy=cam["cy"] / stride, depth_encoding=depth_encoding,
+                  color_encoding="rgb8")
+    return depth, rgb, camera
+
+
 def submap_frames(robot, submap, frames, cam=CAM_640x480, device="cpu", stride=1):
     """Poses + rendered frames of one submap of one robot (robot map frame == world here)."""
     poses = trajectory(frames, robot=robot, submap=submap, frames_per_submap=frames)

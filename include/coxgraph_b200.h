@@ -262,6 +262,62 @@ int32_t cg_prepare_batch_staged(cg_layer* layer, const cg_integrator_config* cfg
                                 int32_t slot);
 int32_t cg_integrate_prepared(cg_layer* layer, int32_t slot, cg_integrate_stats* stats);
 
+/* --- integration of registered depth + colour images: replaces depth_image_proc
+ * point_cloud_xyzrgb (depth_conversions.h convert<T>) followed by voxblox_ros TsdfServer's
+ * insertion (convertPointcloud drops the points with a non-finite coordinate, then
+ * integratePointCloud).  The result is bit-identical, stats included, to cg_integrate_batch_device
+ * on that cloud: per pixel (u, v) in row-major order, a valid depth d (16UC1: d != 0, millimetres;
+ * 32FC1: finite, metres) gives x = ((u - float(cx)) * d) * float(unit / fx), y likewise, z = d in
+ * metres, colour (r, g, b, 255) from the encoding's byte offsets; invalid pixels and points with a
+ * non-finite coordinate are dropped.  Lens distortion is ignored (as depth_image_proc does), the
+ * colour image has the depth image's size and both are tightly packed.  stats.points_in counts
+ * the kept points.  The entry points mirror the cloud family above one to one. */
+enum cg_depth_encoding { CG_DEPTH_16UC1 = 0, CG_DEPTH_32FC1 = 1 };
+enum cg_color_encoding {
+  CG_COLOR_RGB8 = 0,  /* r, g, b offsets 0, 1, 2; 3 bytes a pixel */
+  CG_COLOR_RGBA8 = 1, /* 0, 1, 2; 4 bytes */
+  CG_COLOR_BGR8 = 2,  /* 2, 1, 0; 3 bytes */
+  CG_COLOR_BGRA8 = 3, /* 2, 1, 0; 4 bytes */
+  CG_COLOR_MONO8 = 4  /* 0, 0, 0; 1 byte */
+};
+/* sensor_msgs/CameraInfo as image_geometry::PinholeCameraModel reports it (fx = P[0], fy = P[5],
+ * cx = P[2], cy = P[6]) plus the two image encodings. */
+typedef struct cg_depth_camera {
+  int32_t width, height;
+  double fx, fy, cx, cy;
+  int32_t depth_encoding; /* cg_depth_encoding */
+  int32_t color_encoding; /* cg_color_encoding */
+} cg_depth_camera;
+/* F frames: depth [F][H][W] (uint16 or float), colour [F][H][W][pixel bytes]; host memory
+ * (pageable or pinned) or, for _device, device memory on the context's GPU. */
+int32_t cg_integrate_depth_batch(cg_layer* layer, const cg_integrator_config* cfg,
+                                 size_t num_frames, const float* T_G_C_poses,
+                                 const cg_depth_camera* camera, const void* depth,
+                                 const uint8_t* color, cg_integrate_stats* stats);
+int32_t cg_integrate_depth_batch_device(cg_layer* layer, const cg_integrator_config* cfg,
+                                        size_t num_frames, const float* T_G_C_poses,
+                                        const cg_depth_camera* camera, const void* d_depth,
+                                        const uint8_t* d_color, cg_integrate_stats* stats);
+/* Staging of images into slot 0 or 1 (pinned host memory; returns at once).  The slots are those
+ * of cg_stage_batch_async: staging replaces what the slot held, and a slot that holds images is
+ * only usable by the _depth_ calls (and one that holds a cloud only by the cloud calls);
+ * otherwise CG_ERR_INVALID_ARG.  The camera and frame count must be those staged. */
+int32_t cg_stage_depth_async(cg_context* ctx, int32_t slot, const cg_depth_camera* camera,
+                             size_t num_frames, const void* depth, const uint8_t* color);
+int32_t cg_integrate_depth_staged(cg_layer* layer, const cg_integrator_config* cfg,
+                                  size_t num_frames, const float* T_G_C_poses,
+                                  const cg_depth_camera* camera, int32_t slot,
+                                  cg_integrate_stats* stats);
+/* Pipelined depth jobs, completed by cg_integrate_prepared.  The unprojected points are kept in
+ * the prepare slot, so a job the fast path cannot take runs the plain way from them. */
+int32_t cg_prepare_depth_device(cg_layer* layer, const cg_integrator_config* cfg,
+                                size_t num_frames, const float* T_G_C_poses,
+                                const cg_depth_camera* camera, const void* d_depth,
+                                const uint8_t* d_color, int32_t slot);
+int32_t cg_prepare_depth_staged(cg_layer* layer, const cg_integrator_config* cfg,
+                                size_t num_frames, const float* T_G_C_poses,
+                                const cg_depth_camera* camera, int32_t stage_slot, int32_t slot);
+
 /* --- mesh recovery: the recover node's front end (SURVEY §8f N3) ----------------------
  * voxblox_msgs/Mesh (the fork's "mesh with observation history") flattened into plain arrays:
  * block b owns vertices [vertex_begin[b], vertex_begin[b+1]) (triangles: multiples of 3), x/y/z
