@@ -17,8 +17,9 @@ OBJS = $(OBJ)/layer.o $(OBJ)/integrate.o $(OBJ)/integrate_front.o $(OBJ)/integra
 
 HOSTCHK = build/host_api_check
 DEPTHCHK = build/depth_api_check
+ESDFCHK = build/esdf_update_check
 
-all: $(LIB) oracle $(HOSTCHK) $(DEPTHCHK)
+all: $(LIB) oracle $(HOSTCHK) $(DEPTHCHK) $(ESDFCHK)
 
 $(OBJ)/%.o: $(SRC)/%.cu $(HDRS)
 	@mkdir -p $(OBJ)
@@ -39,6 +40,11 @@ $(HOSTCHK): tests/host/host_api_check.cc coxgraph_b200/host/coxgraph_b200.hpp in
 # C++ depth-image driver (tests/test_host_depth.py)
 $(DEPTHCHK): tests/host/depth_api_check.cc coxgraph_b200/host/coxgraph_b200.hpp include/coxgraph_b200.h $(LIB)
 	g++ -std=c++17 -O1 -Wall -Wextra tests/host/depth_api_check.cc -o $@ -Lcoxgraph_b200/lib \
+	    -lcoxgraph_b200 -Wl,-rpath,'$$ORIGIN/../coxgraph_b200/lib'
+
+# C++ incremental-ESDF driver (tests/test_host_esdf_update.py)
+$(ESDFCHK): tests/host/esdf_update_check.cc coxgraph_b200/host/coxgraph_b200.hpp include/coxgraph_b200.h $(LIB)
+	g++ -std=c++17 -O1 -Wall -Wextra tests/host/esdf_update_check.cc -o $@ -Lcoxgraph_b200/lib \
 	    -lcoxgraph_b200 -Wl,-rpath,'$$ORIGIN/../coxgraph_b200/lib'
 
 clean:

@@ -246,6 +246,26 @@ class Layer:
         capi.check(lib.cg_layer_esdf_batch(self._h, C.byref(cfg), C.byref(st)))
         if not fetch:
             return st
+        return self._fetch_esdf(st)
+
+    def updateEsdf(self, config=None, fetch=True):
+        """voxblox::EsdfIntegrator::updateFromTsdfLayer on the device: brings the ESDF retained in
+        the context up to date with this layer, re-solving only the blocks within reach of what
+        changed; the result is bit-identical to updateEsdfBatch(config).  Changes are found by
+        content (the `updated` flags are left alone).  -> updateEsdfBatch's dict plus
+        "update" (capi.EsdfUpdateStats); with fetch=False -> (stats, update stats)."""
+        lib = capi.load()
+        cfg = config if config is not None else esdfConfig()
+        st, ust = capi.EsdfStats(), capi.EsdfUpdateStats()
+        capi.check(lib.cg_layer_esdf_update(self._h, C.byref(cfg), C.byref(st), C.byref(ust)))
+        if not fetch:
+            return st, ust
+        out = self._fetch_esdf(st)
+        out["update"] = ust
+        return out
+
+    def _fetch_esdf(self, st):
+        lib = capi.load()
         B = st.blocks
         idx = np.zeros((B, 3), np.int32)
         dist = np.zeros((B, capi.VOXELS_PER_BLOCK), np.float32)

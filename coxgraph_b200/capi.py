@@ -135,6 +135,11 @@ class EsdfStats(C.Structure):
                 ("fixed_voxels", C.c_uint64), ("sweeps", C.c_uint64), ("block_passes", C.c_uint64)]
 
 
+class EsdfUpdateStats(C.Structure):
+    _fields_ = [("blocks_changed", C.c_uint64), ("blocks_removed", C.c_uint64),
+                ("blocks_region", C.c_uint64), ("full_rebuild", C.c_int32), ("reserved", C.c_int32)]
+
+
 # every symbol include/coxgraph_b200.h declares: name -> (restype, argtypes)
 _P = C.c_void_p
 SYMBOLS = {
@@ -208,6 +213,8 @@ SYMBOLS = {
                                     C.POINTER(C.c_size_t), C.POINTER(C.c_size_t)]),
     "cg_esdf_config_default": (None, [C.POINTER(EsdfConfig)]),
     "cg_layer_esdf_batch": (C.c_int32, [_P, C.POINTER(EsdfConfig), C.POINTER(EsdfStats)]),
+    "cg_layer_esdf_update": (C.c_int32, [_P, C.POINTER(EsdfConfig), C.POINTER(EsdfStats),
+                                         C.POINTER(EsdfUpdateStats)]),
     "cg_esdf_fetch": (C.c_int32, [_P, C.c_size_t, _P, _P, _P, C.POINTER(C.c_size_t)]),
     "cg_esdf_free_points": (C.c_int32, [_P, C.c_float, C.c_size_t, _P, C.POINTER(C.c_size_t)]),
     "cg_reproject_submaps": (C.c_int32, [_P, _P, _P, C.c_size_t, C.c_float, C.c_float, _P, _P,

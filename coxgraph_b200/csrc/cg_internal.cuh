@@ -303,11 +303,18 @@ struct cg_context : cg::FrontBufs {
   size_t mc_blocks = 0, mc_total = 0;  // size of the retained result (cg_mesh_fetch)
   cg::DevBuf weld_keys, weld_words, weld_out;  // vertex welding (mesh_connect.cu)
   // ESDF of a layer (esdf.cu): working / result planes in (z, y, x) block order, retained until
-  // the next cg_layer_esdf_batch on this context
+  // the next cg_layer_esdf_batch / cg_layer_esdf_update on this context
   cg::DevBuf esdf_keys, esdf_slots, esdf_dist, esdf_packed, esdf_fixed, esdf_slot_to_b,
       esdf_dirty, esdf_list, esdf_index, esdf_counters;
+  // cg_layer_esdf_update: the planes of the next block list while the retained ones are read,
+  // new -> retained block position, changed / removed block keys, region mask and list
+  cg::DevBuf esdf_dist_next, esdf_packed_next, esdf_old_b, esdf_sources, esdf_region,
+      esdf_region_list;
   size_t esdf_blocks = 0;
   float esdf_voxel_size = 0.0f, esdf_block_size = 0.0f;
+  // what the retained ESDF was computed from: cg_layer::serial (0: nothing retained) and config
+  uint64_t esdf_serial = 0;
+  cg_esdf_config esdf_cfg = {};
   // instrumentation
   bool profiling = false;
   uint64_t own_launches = 0;  // kernels of this library launched (library sorts/scans excluded)
@@ -342,6 +349,8 @@ struct cg_layer {
   size_t hash_cap = 0;
   size_t max_blocks = 0;
   int64_t num_blocks = 0;  // host mirror, refreshed at the end of every mutating call
+  // unique per process (cg_layer_create), never reused: a destroyed layer's address can come back
+  uint64_t serial = 0;
 };
 
 namespace cg {

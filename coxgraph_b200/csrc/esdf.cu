@@ -24,10 +24,17 @@
 // With min_diff_m > 0 upstream stops early and may stay above this fixed point by less than
 // min_diff_m per hop (tests bound it); `parent` follows upstream's queue order there and a fixed
 // neighbour order here (faces, edges, corners; first neighbour that attains the distance).
+//
+// cg_layer_esdf_update (updateFromTsdfLayer) starts from the retained result instead: it finds the
+// voxels whose init state changed (k_esdf_compare), re-initialises every block within reach of them
+// (k_esdf_dilate) and runs the same sweeps and finish over those blocks only; DESIGN §4.6 has the
+// argument that this ends in the batch's bits.
 #include <cub/cub.cuh>
 
 #include <algorithm>
+#include <cmath>
 #include <cstring>
+#include <utility>
 
 #include "cg_internal.cuh"
 
@@ -53,12 +60,16 @@ struct NeighborTable {
 };
 __constant__ NeighborTable c_nb;
 
-__global__ void k_esdf_init(LayerView L, const uint32_t* __restrict__ slots, uint32_t n,
-                            EsdfParams P, float* __restrict__ dist, uint32_t* __restrict__ fixed_bits,
+// the init state of a block's voxels; `list` (may be null: all n blocks) names the blocks,
+// `counters` (may be null) receives the observed / fixed totals
+__global__ void k_esdf_init(LayerView L, const uint32_t* __restrict__ slots,
+                            const uint32_t* __restrict__ list, uint32_t n, EsdfParams P,
+                            float* __restrict__ dist, uint32_t* __restrict__ fixed_bits,
                             int32_t* __restrict__ slot_to_b, uint8_t* __restrict__ dirty,
                             unsigned long long* __restrict__ counters) {
   unsigned long long n_obs = 0, n_fixed = 0;
-  for (uint32_t b = blockIdx.x; b < n; b += gridDim.x) {
+  for (uint32_t item = blockIdx.x; item < n; item += gridDim.x) {
+    const uint32_t b = list ? list[item] : item;
     const int slot = static_cast<int>(slots[b]);
     const float* td = L.dist_plane(slot);
     const float* tw = L.weight_plane(slot);
@@ -84,6 +95,7 @@ __global__ void k_esdf_init(LayerView L, const uint32_t* __restrict__ slots, uin
       if ((threadIdx.x & 31) == 0) fixed_bits[static_cast<size_t>(b) * 128 + (i >> 5)] = bits;
     }
   }
+  if (!counters) return;
   n_obs = __reduce_add_sync(0xFFFFFFFFu, static_cast<unsigned>(n_obs));
   n_fixed = __reduce_add_sync(0xFFFFFFFFu, static_cast<unsigned>(n_fixed));
   if ((threadIdx.x & 31) == 0) {
@@ -160,7 +172,7 @@ __global__ void __launch_bounds__(kEsdfThreads)
 k_esdf_sweep(LayerView L, const uint64_t* __restrict__ keys, const uint32_t* __restrict__ list,
              const uint32_t* __restrict__ count, EsdfParams P, float* __restrict__ dist,
              const uint32_t* __restrict__ fixed_bits, const int32_t* __restrict__ slot_to_b,
-             uint8_t* __restrict__ dirty) {
+             const uint8_t* __restrict__ region, uint8_t* __restrict__ dirty) {
   __shared__ float tile[kTileVoxels];
   __shared__ int table[27];
   __shared__ uint32_t face_flags;
@@ -208,7 +220,8 @@ k_esdf_sweep(LayerView L, const uint64_t* __restrict__ keys, const uint32_t* __r
       }
       if (!__syncthreads_or(changed)) break;
     }
-    // write back what changed; a changed face wakes the blocks behind it
+    // write back what changed; a changed face wakes the blocks behind it (those of the region
+    // only, when one is given: the values outside it are final)
     uint32_t faces = 0;
     float* own = dist + static_cast<size_t>(b) * kVoxelsPerBlock;
     for (int z = 0; z < kVps; ++z) {
@@ -228,7 +241,7 @@ k_esdf_sweep(LayerView L, const uint64_t* __restrict__ keys, const uint32_t* __r
       const int dx = t % 3 - 1, dy = (t / 3) % 3 - 1, dz = t / 9 - 1;
       const uint32_t need = (dx < 0 ? 1u : dx > 0 ? 2u : 0u) | (dy < 0 ? 4u : dy > 0 ? 8u : 0u) |
                             (dz < 0 ? 16u : dz > 0 ? 32u : 0u);
-      if ((face_flags & need) == need) dirty[table[t]] = 1;
+      if ((face_flags & need) == need && (!region || region[table[t]])) dirty[table[t]] = 1;
     }
   }
 }
@@ -239,13 +252,15 @@ k_esdf_sweep(LayerView L, const uint64_t* __restrict__ keys, const uint32_t* __r
 // serializeToIntegers' second word); flags: 1 observed, 2 hallucinated, 4 in_queue, 8 fixed
 __global__ void __launch_bounds__(kEsdfThreads)
 k_esdf_finish(LayerView L, const uint64_t* __restrict__ keys, const uint32_t* __restrict__ slots,
-              uint32_t n, EsdfParams P, float* dist, const uint32_t* __restrict__ fixed_bits,
-              const int32_t* __restrict__ slot_to_b, uint32_t* __restrict__ packed) {
+              const uint32_t* __restrict__ list, uint32_t n, EsdfParams P, float* dist,
+              const uint32_t* __restrict__ fixed_bits, const int32_t* __restrict__ slot_to_b,
+              uint32_t* __restrict__ packed) {
   __shared__ float tile[kTileVoxels];
   __shared__ int table[27];
   const int x = threadIdx.x & 15, y = threadIdx.x >> 4;
   const int col = (y + 1) * kTileRow + x + 1;
-  for (uint32_t b = blockIdx.x; b < n; b += gridDim.x) {
+  for (uint32_t item = blockIdx.x; item < n; item += gridDim.x) {
+    const uint32_t b = list ? list[item] : item;
     __syncthreads();
     load_neighbor_table(L, keys[b], slot_to_b, table);
     __syncthreads();
@@ -341,6 +356,136 @@ __global__ void k_esdf_unpack_idx(const uint64_t* __restrict__ keys, uint32_t n,
   idx[3 * i + 2] = z;
 }
 
+// ------------------------------------------------------------------ incremental update
+// Counters of one update (uint32 words after the batch's counters): see cg_layer_esdf_update.
+enum UpdateCount { kUcSources = 0, kUcRemoved, kUcMoved, kUcChanged, kUcRegion, kUcWords = 8 };
+
+// position of `key` in the sorted `keys[0, n)`, or -1
+__device__ __forceinline__ int32_t find_sorted(const uint64_t* __restrict__ keys, uint32_t n,
+                                               uint64_t key) {
+  uint32_t lo = 0, hi = n;
+  while (lo < hi) {
+    const uint32_t mid = (lo + hi) >> 1;
+    if (keys[mid] < key) lo = mid + 1; else hi = mid;
+  }
+  return lo < n && keys[lo] == key ? static_cast<int32_t>(lo) : -1;
+}
+
+// Matches the new block list with the retained one by key (slots are not stable: removing blocks
+// compacts the pool).  New block b -> old_b[b] (-1: new block); retained blocks the layer no
+// longer has are sources of the region.
+__global__ void k_esdf_match(const uint64_t* __restrict__ keys, const uint32_t* __restrict__ slots,
+                             uint32_t n, const uint64_t* __restrict__ old_keys, uint32_t n_old,
+                             int32_t* __restrict__ old_b, int32_t* __restrict__ slot_to_b,
+                             uint64_t* __restrict__ sources, uint32_t* __restrict__ ucount) {
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) {
+    const int32_t ob = find_sorted(old_keys, n_old, keys[i]);
+    old_b[i] = ob;
+    slot_to_b[slots[i]] = static_cast<int32_t>(i);
+    if (ob != static_cast<int32_t>(i)) atomicAdd(&ucount[kUcMoved], 1u);
+  }
+  if (i < n_old && find_sorted(keys, n, old_keys[i]) < 0) {
+    sources[atomicAdd(&ucount[kUcSources], 1u)] = old_keys[i];
+    atomicAdd(&ucount[kUcRemoved], 1u);
+  }
+}
+
+// One pass over every block: the new init state of each voxel (k_esdf_init's rule) against the
+// one the retained result implies — fixed voxels kept their distance, other observed voxels
+// started at sign(result) * default (0 stays 0), unobserved ones have packed & 1 == 0 and the
+// hallucinated bit is packed & 2.  A block with any difference, or without a retained block, is a
+// source of the region.  Also counts the observed / fixed voxels of the whole map.
+__global__ void __launch_bounds__(kEsdfThreads)
+k_esdf_compare(LayerView L, const uint64_t* __restrict__ keys, const uint32_t* __restrict__ slots,
+               uint32_t n, EsdfParams P, const int32_t* __restrict__ old_b,
+               const float* __restrict__ old_dist, const uint32_t* __restrict__ old_packed,
+               uint64_t* __restrict__ sources, uint32_t* __restrict__ ucount,
+               unsigned long long* __restrict__ counters) {
+  unsigned long long n_obs = 0, n_fixed = 0;
+  for (uint32_t b = blockIdx.x; b < n; b += gridDim.x) {
+    const int slot = static_cast<int>(slots[b]);
+    const int32_t ob = old_b[b];
+    const float* td = L.dist_plane(slot);
+    const float* tw = L.weight_plane(slot);
+    bool changed = ob < 0;
+    for (int i = threadIdx.x; i < kVoxelsPerBlock; i += kEsdfThreads) {
+      const float d = td[i], w = tw[i];
+      uint32_t flags;  // 1 observed, 2 hallucinated, 8 fixed
+      float init = 0.0f;
+      if (w < P.min_weight) {
+        flags = P.crust ? 3u : 0u;
+        init = -P.default_distance;
+      } else {
+        const bool fixed = fabsf(d) < P.min_distance;
+        const float sgn = d == 0.0f ? 0.0f : (d < 0.0f ? -1.0f : 1.0f);
+        init = fixed ? d : sgn * P.default_distance;
+        flags = fixed ? 9u : 1u;
+        ++n_obs;
+        n_fixed += fixed ? 1 : 0;
+      }
+      if (ob >= 0) {
+        const size_t o = static_cast<size_t>(ob) * kVoxelsPerBlock + i;
+        const uint32_t op = __ldcs(old_packed + o) & 11u;
+        const float od = __ldcs(old_dist + o);
+        const float oinit = (op & 8u) ? od : (od == 0.0f ? 0.0f : (od < 0.0f ? -P.default_distance : P.default_distance));
+        if (op != flags || ((flags & 1u) && __float_as_uint(oinit) != __float_as_uint(init))) changed = true;
+      }
+    }
+    if (__syncthreads_or(changed) && threadIdx.x == 0) {
+      sources[atomicAdd(&ucount[kUcSources], 1u)] = keys[b];
+      atomicAdd(&ucount[kUcChanged], 1u);
+    }
+  }
+  n_obs = __reduce_add_sync(0xFFFFFFFFu, static_cast<unsigned>(n_obs));
+  n_fixed = __reduce_add_sync(0xFFFFFFFFu, static_cast<unsigned>(n_fixed));
+  if ((threadIdx.x & 31) == 0) {
+    atomicAdd(&counters[0], n_obs);
+    atomicAdd(&counters[1], n_fixed);
+  }
+}
+
+// region: every current block within block-Chebyshev distance r of a source key, probed in the
+// layer's hash
+__global__ void k_esdf_dilate(LayerView L, const uint64_t* __restrict__ sources,
+                              const uint32_t* __restrict__ ucount, int r,
+                              const int32_t* __restrict__ slot_to_b, uint8_t* __restrict__ region) {
+  const uint32_t n = ucount[kUcSources];
+  const int side = 2 * r + 1, cube = side * side * side;
+  for (uint32_t s = blockIdx.x; s < n; s += gridDim.x) {
+    int bx, by, bz;
+    unpack_block_key(sources[s], bx, by, bz);
+    for (int o = threadIdx.x; o < cube; o += blockDim.x) {
+      const int slot = L.find_slot(pack_block_key(bx + o % side - r, by + (o / side) % side - r,
+                                                  bz + o / (side * side) - r));
+      if (slot >= 0) region[slot_to_b[slot]] = 1;
+    }
+  }
+}
+
+__global__ void k_esdf_region_list(const uint8_t* __restrict__ region, uint32_t n,
+                                   uint32_t* __restrict__ list, uint32_t* __restrict__ ucount) {
+  const uint32_t b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b < n && region[b]) list[atomicAdd(&ucount[kUcRegion], 1u)] = b;
+}
+
+// the retained distance and packed planes of the blocks outside the region to their new positions
+// (every block outside the region has a retained block: new blocks are sources)
+__global__ void __launch_bounds__(kEsdfThreads)
+k_esdf_remap(const uint8_t* __restrict__ region, const int32_t* __restrict__ old_b, uint32_t n,
+             const float4* __restrict__ old_dist, const uint4* __restrict__ old_packed,
+             float4* __restrict__ dist, uint4* __restrict__ packed) {
+  constexpr int kVec = kVoxelsPerBlock / 4;
+  for (uint32_t b = blockIdx.x; b < n; b += gridDim.x) {
+    if (region[b]) continue;
+    const size_t src = static_cast<size_t>(old_b[b]) * kVec, dst = static_cast<size_t>(b) * kVec;
+    for (int i = threadIdx.x; i < kVec; i += kEsdfThreads) {
+      dist[dst + i] = __ldcs(old_dist + src + i);
+      packed[dst + i] = __ldcs(old_packed + src + i);
+    }
+  }
+}
+
 static float float_from_bits(uint32_t u) {
   float f;
   memcpy(&f, &u, sizeof(f));
@@ -370,6 +515,95 @@ static cudaError_t upload_neighbor_table() {
   return e;
 }
 
+static int32_t check_config(const cg_esdf_config* cfg, const char* fn) {
+  if (cfg->full_euclidean_distance) {
+    set_error("%s: full_euclidean_distance is not implemented (upstream default: off)", fn);
+    return CG_ERR_UNSUPPORTED;
+  }
+  if (!(cfg->max_distance_m > 0.0f) || !(cfg->default_distance_m >= cfg->max_distance_m) ||
+      !(cfg->min_distance_m >= 0.0f)) {
+    set_error("%s: need max_distance_m > 0, default_distance_m >= max_distance_m "
+              "(as voxblox_ros' parameter loader enforces), min_distance_m >= 0", fn);
+    return CG_ERR_INVALID_ARG;
+  }
+  return CG_OK;
+}
+
+static EsdfParams make_params(const cg_layer* L, const cg_esdf_config* cfg) {
+  EsdfParams P;
+  P.max_distance = cfg->max_distance_m;
+  P.default_distance = cfg->default_distance_m;
+  P.min_distance = cfg->min_distance_m;
+  P.min_weight = cfg->min_weight;
+  P.w1 = 1.0f * L->v.voxel_size;
+  P.w2 = float_from_bits(0x3FB504F3) * L->v.voxel_size;  // float(sqrt(2))
+  P.w3 = float_from_bits(0x3FDDB3D7) * L->v.voxel_size;  // float(sqrt(3))
+  P.crust = cfg->add_occupied_crust ? 1 : 0;
+  return P;
+}
+
+// the config fields the result depends on, compared bit for bit
+static bool same_result_config(const cg_esdf_config& a, const cg_esdf_config& b) {
+  return memcmp(&a.max_distance_m, &b.max_distance_m, sizeof(float)) == 0 &&
+         memcmp(&a.default_distance_m, &b.default_distance_m, sizeof(float)) == 0 &&
+         memcmp(&a.min_distance_m, &b.min_distance_m, sizeof(float)) == 0 &&
+         memcmp(&a.min_weight, &b.min_weight, sizeof(float)) == 0 &&
+         (a.add_occupied_crust != 0) == (b.add_occupied_crust != 0);
+}
+
+// Block radius R of the region around a changed block (DESIGN §4.6).  A voxel feeds a neighbour
+// only while |d| < max_distance and every hop adds at least w1 = voxel_size, so a voxel's result
+// depends on the init states within L = ceil(max / w1) + 1 hops; one more hop covers the rounding
+// of fl(a + w) (k hops lose less than k * 2^-24 relative, under one hop while k < 4096), and the
+// packed word also reads the 26 neighbours' results: L + 2 voxels, R = ceil((L + 2) / 16) blocks.
+static int region_reach(const cg_layer* L, const cg_esdf_config* cfg) {
+  const double hops = std::ceil(static_cast<double>(cfg->max_distance_m) /
+                                static_cast<double>(L->v.voxel_size)) + 2.0;
+  return static_cast<int>(std::ceil((hops + 1.0) / kVps));
+}
+
+// the retained ESDF is now that of `L` under `cfg`
+static int32_t retain(cg_context* ctx, const cg_layer* L, const cg_esdf_config* cfg, size_t n) {
+  ctx->esdf_blocks = n;
+  ctx->esdf_serial = L->serial;
+  ctx->esdf_cfg = *cfg;
+  ctx->esdf_voxel_size = L->v.voxel_size;
+  ctx->esdf_block_size = L->v.block_size;
+  return CG_OK;
+}
+
+// Sweeps over the dirty blocks until none is left.  With `region`, only region blocks are woken.
+static int32_t run_sweeps(cg_context* ctx, const cg_layer* L, const uint64_t* keys, size_t n,
+                          const EsdfParams& P, const uint8_t* region, uint64_t* sweeps,
+                          uint64_t* passes, const char* fn) {
+  cudaStream_t s = ctx->stream;
+  uint32_t* d_count = reinterpret_cast<uint32_t*>(ctx->esdf_counters.as<unsigned long long>() + 2);
+  for (;;) {
+    CG_CUDA(cudaMemsetAsync(d_count, 0, sizeof(uint32_t), s));
+    k_esdf_collect<<<grid_for(n, 256), 256, 0, s>>>(ctx->esdf_dirty.as<uint8_t>(),
+                                                    static_cast<uint32_t>(n),
+                                                    ctx->esdf_list.as<uint32_t>(), d_count);
+    uint32_t h_count = 0;
+    CG_CUDA(cudaMemcpyAsync(&h_count, d_count, sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+    CG_CUDA(cudaStreamSynchronize(s));
+    ctx->own_launches += 1;
+    if (h_count == 0) break;
+    if (++*sweeps > 100000) {
+      set_error("%s: no convergence", fn);
+      return CG_ERR_CUDA;
+    }
+    *passes += h_count;
+    const unsigned grid = std::min<unsigned>(h_count, static_cast<unsigned>(ctx->num_sms) * 8u);
+    ctx->own_launches += 1;
+    k_esdf_sweep<<<grid, kEsdfThreads, 0, s>>>(L->v, keys, ctx->esdf_list.as<uint32_t>(), d_count, P,
+                                               ctx->esdf_dist.as<float>(),
+                                               ctx->esdf_fixed.as<uint32_t>(),
+                                               ctx->esdf_slot_to_b.as<int32_t>(), region,
+                                               ctx->esdf_dirty.as<uint8_t>());
+  }
+  return CG_OK;
+}
+
 }  // namespace cg
 
 using namespace cg;
@@ -394,26 +628,19 @@ int32_t cg_layer_esdf_batch(const cg_layer* L, const cg_esdf_config* cfg, cg_esd
   cg_context* ctx = L->ctx;
   CG_CUDA(cudaSetDevice(ctx->device));
   if (stats) memset(stats, 0, sizeof(*stats));
-  if (cfg->full_euclidean_distance) {
-    set_error("cg_layer_esdf_batch: full_euclidean_distance is not implemented (upstream default: off)");
-    return CG_ERR_UNSUPPORTED;
-  }
-  if (!(cfg->max_distance_m > 0.0f) || !(cfg->default_distance_m >= cfg->max_distance_m) ||
-      !(cfg->min_distance_m >= 0.0f)) {
-    set_error("cg_layer_esdf_batch: need max_distance_m > 0, default_distance_m >= max_distance_m "
-              "(as voxblox_ros' parameter loader enforces), min_distance_m >= 0");
-    return CG_ERR_INVALID_ARG;
-  }
+  int32_t rc = check_config(cfg, "cg_layer_esdf_batch");
+  if (rc) return rc;
   cudaStream_t s = ctx->stream;
   const size_t n = static_cast<size_t>(L->num_blocks);
   ctx->esdf_blocks = 0;
+  ctx->esdf_serial = 0;
   ctx->esdf_voxel_size = L->v.voxel_size;
   ctx->esdf_block_size = L->v.block_size;
-  if (n == 0) return CG_OK;
+  if (n == 0) return retain(ctx, L, cfg, 0);
   CG_CUDA(upload_neighbor_table());
   const uint64_t* keys;
   const uint32_t* slots;
-  int32_t rc = sort_blocks(L, &keys, &slots);
+  rc = sort_blocks(L, &keys, &slots);
   if (rc) return rc;
   // sort_blocks leaves its result in scratch other calls reuse: keep our own copy
   CG_CUDA(ctx->esdf_keys.reserve(n * sizeof(uint64_t)));
@@ -430,52 +657,22 @@ int32_t cg_layer_esdf_batch(const cg_layer* L, const cg_esdf_config* cfg, cg_esd
   CG_CUDA(ctx->esdf_list.reserve(n * sizeof(uint32_t)));
   CG_CUDA(ctx->esdf_index.reserve(n * 3 * sizeof(int32_t)));
   CG_CUDA(ctx->esdf_counters.reserve(4 * sizeof(unsigned long long)));
-  EsdfParams P;
-  P.max_distance = cfg->max_distance_m;
-  P.default_distance = cfg->default_distance_m;
-  P.min_distance = cfg->min_distance_m;
-  P.min_weight = cfg->min_weight;
-  P.w1 = 1.0f * L->v.voxel_size;
-  P.w2 = float_from_bits(0x3FB504F3) * L->v.voxel_size;  // float(sqrt(2))
-  P.w3 = float_from_bits(0x3FDDB3D7) * L->v.voxel_size;  // float(sqrt(3))
-  P.crust = cfg->add_occupied_crust ? 1 : 0;
+  const EsdfParams P = make_params(L, cfg);
   unsigned long long* counters = ctx->esdf_counters.as<unsigned long long>();
-  uint32_t* d_count = reinterpret_cast<uint32_t*>(counters + 2);
   CG_CUDA(cudaMemsetAsync(counters, 0, 4 * sizeof(unsigned long long), s));
   const unsigned wide = static_cast<unsigned>(std::min<size_t>(n, static_cast<size_t>(ctx->num_sms) * 16));
   ctx->own_launches += 2;
-  k_esdf_init<<<wide, kEsdfThreads, 0, s>>>(L->v, slots, static_cast<uint32_t>(n), P,
+  k_esdf_init<<<wide, kEsdfThreads, 0, s>>>(L->v, slots, nullptr, static_cast<uint32_t>(n), P,
                                             ctx->esdf_dist.as<float>(), ctx->esdf_fixed.as<uint32_t>(),
                                             ctx->esdf_slot_to_b.as<int32_t>(),
                                             ctx->esdf_dirty.as<uint8_t>(), counters);
   k_esdf_unpack_idx<<<grid_for(n, 256), 256, 0, s>>>(keys, static_cast<uint32_t>(n),
                                                      ctx->esdf_index.as<int32_t>());
   uint64_t sweeps = 0, passes = 0;
-  for (;;) {
-    CG_CUDA(cudaMemsetAsync(d_count, 0, sizeof(uint32_t), s));
-    k_esdf_collect<<<grid_for(n, 256), 256, 0, s>>>(ctx->esdf_dirty.as<uint8_t>(),
-                                                    static_cast<uint32_t>(n),
-                                                    ctx->esdf_list.as<uint32_t>(), d_count);
-    uint32_t h_count = 0;
-    CG_CUDA(cudaMemcpyAsync(&h_count, d_count, sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
-    CG_CUDA(cudaStreamSynchronize(s));
-    ctx->own_launches += 1;
-    if (h_count == 0) break;
-    if (++sweeps > 100000) {
-      set_error("cg_layer_esdf_batch: no convergence");
-      return CG_ERR_CUDA;
-    }
-    passes += h_count;
-    const unsigned grid = std::min<unsigned>(h_count, static_cast<unsigned>(ctx->num_sms) * 8u);
-    ctx->own_launches += 1;
-    k_esdf_sweep<<<grid, kEsdfThreads, 0, s>>>(L->v, keys, ctx->esdf_list.as<uint32_t>(), d_count, P,
-                                               ctx->esdf_dist.as<float>(),
-                                               ctx->esdf_fixed.as<uint32_t>(),
-                                               ctx->esdf_slot_to_b.as<int32_t>(),
-                                               ctx->esdf_dirty.as<uint8_t>());
-  }
+  rc = run_sweeps(ctx, L, keys, n, P, nullptr, &sweeps, &passes, "cg_layer_esdf_batch");
+  if (rc) return rc;
   ctx->own_launches += 1;
-  k_esdf_finish<<<wide, kEsdfThreads, 0, s>>>(L->v, keys, slots, static_cast<uint32_t>(n), P,
+  k_esdf_finish<<<wide, kEsdfThreads, 0, s>>>(L->v, keys, slots, nullptr, static_cast<uint32_t>(n), P,
                                               ctx->esdf_dist.as<float>(),
                                               ctx->esdf_fixed.as<uint32_t>(),
                                               ctx->esdf_slot_to_b.as<int32_t>(),
@@ -484,7 +681,6 @@ int32_t cg_layer_esdf_batch(const cg_layer* L, const cg_esdf_config* cfg, cg_esd
   CG_CUDA(cudaMemcpyAsync(h_counters, counters, sizeof(h_counters), cudaMemcpyDeviceToHost, s));
   CG_CUDA(cudaStreamSynchronize(s));
   CG_CUDA(cudaGetLastError());
-  ctx->esdf_blocks = n;
   if (stats) {
     stats->blocks = n;
     stats->observed_voxels = h_counters[0];
@@ -492,7 +688,126 @@ int32_t cg_layer_esdf_batch(const cg_layer* L, const cg_esdf_config* cfg, cg_esd
     stats->sweeps = sweeps;
     stats->block_passes = passes;
   }
-  return CG_OK;
+  return retain(ctx, L, cfg, n);
+}
+
+int32_t cg_layer_esdf_update(const cg_layer* L, const cg_esdf_config* cfg, cg_esdf_stats* stats,
+                             cg_esdf_update_stats* ust) {
+  if (!L || !cfg) return CG_ERR_INVALID_ARG;
+  cg_context* ctx = L->ctx;
+  CG_CUDA(cudaSetDevice(ctx->device));
+  if (stats) memset(stats, 0, sizeof(*stats));
+  if (ust) memset(ust, 0, sizeof(*ust));
+  int32_t rc = check_config(cfg, "cg_layer_esdf_update");
+  if (rc) return rc;
+  const size_t n = static_cast<size_t>(L->num_blocks), n_old = ctx->esdf_blocks;
+  if (ctx->esdf_serial != L->serial || n_old == 0 || n == 0 || !same_result_config(ctx->esdf_cfg, *cfg)) {
+    rc = cg_layer_esdf_batch(L, cfg, stats);
+    if (rc == CG_OK && ust) {
+      ust->blocks_changed = ust->blocks_region = n;
+      ust->full_rebuild = 1;
+    }
+    return rc;
+  }
+  cudaStream_t s = ctx->stream;
+  ctx->esdf_blocks = 0;  // until the update is complete
+  ctx->esdf_serial = 0;
+  CG_CUDA(upload_neighbor_table());
+  const uint64_t* keys;
+  const uint32_t* slots;
+  rc = sort_blocks(L, &keys, &slots);
+  if (rc) return rc;
+  CG_CUDA(ctx->esdf_old_b.reserve(n * sizeof(int32_t)));
+  CG_CUDA(ctx->esdf_sources.reserve((n + n_old) * sizeof(uint64_t)));
+  CG_CUDA(ctx->esdf_region.reserve(n));
+  CG_CUDA(ctx->esdf_region_list.reserve(n * sizeof(uint32_t)));
+  CG_CUDA(ctx->esdf_fixed.reserve(n * 128 * sizeof(uint32_t)));  // read for region blocks only
+  CG_CUDA(ctx->esdf_slot_to_b.reserve(n * sizeof(int32_t)));
+  CG_CUDA(ctx->esdf_dirty.reserve(n));
+  CG_CUDA(ctx->esdf_list.reserve(n * sizeof(uint32_t)));
+  CG_CUDA(ctx->esdf_counters.reserve((4 + kUcWords / 2) * sizeof(unsigned long long)));
+  const EsdfParams P = make_params(L, cfg);
+  unsigned long long* counters = ctx->esdf_counters.as<unsigned long long>();
+  uint32_t* ucount = reinterpret_cast<uint32_t*>(counters + 4);
+  uint8_t* region = ctx->esdf_region.as<uint8_t>();
+  int32_t* old_b = ctx->esdf_old_b.as<int32_t>();
+  uint64_t* sources = ctx->esdf_sources.as<uint64_t>();
+  uint32_t* region_list = ctx->esdf_region_list.as<uint32_t>();
+  int32_t* slot_to_b = ctx->esdf_slot_to_b.as<int32_t>();
+  CG_CUDA(cudaMemsetAsync(counters, 0, (4 + kUcWords / 2) * sizeof(unsigned long long), s));
+  CG_CUDA(cudaMemsetAsync(region, 0, n, s));
+  CG_CUDA(cudaMemsetAsync(ctx->esdf_dirty.p, 0, n, s));
+  const unsigned wide = static_cast<unsigned>(std::min<size_t>(n, static_cast<size_t>(ctx->num_sms) * 16));
+  ctx->own_launches += 4;
+  k_esdf_match<<<grid_for(std::max(n, n_old), 256), 256, 0, s>>>(
+      keys, slots, static_cast<uint32_t>(n), ctx->esdf_keys.as<uint64_t>(),
+      static_cast<uint32_t>(n_old), old_b, slot_to_b, sources, ucount);
+  k_esdf_compare<<<wide, kEsdfThreads, 0, s>>>(L->v, keys, slots, static_cast<uint32_t>(n), P, old_b,
+                                               ctx->esdf_dist.as<float>(), ctx->esdf_packed.as<uint32_t>(),
+                                               sources, ucount, counters);
+  k_esdf_dilate<<<static_cast<unsigned>(std::min<size_t>(n + n_old, static_cast<size_t>(ctx->num_sms) * 8)),
+                  kEsdfThreads, 0, s>>>(L->v, sources, ucount, region_reach(L, cfg), slot_to_b, region);
+  k_esdf_region_list<<<grid_for(n, 256), 256, 0, s>>>(region, static_cast<uint32_t>(n), region_list, ucount);
+  unsigned long long h_counters[4 + kUcWords / 2];
+  CG_CUDA(cudaMemcpyAsync(h_counters, counters, sizeof(h_counters), cudaMemcpyDeviceToHost, s));
+  CG_CUDA(cudaStreamSynchronize(s));
+  uint32_t h_ucount[kUcWords];
+  memcpy(h_ucount, h_counters + 4, sizeof(h_ucount));
+  const uint32_t n_region = h_ucount[kUcRegion];
+  if (h_ucount[kUcMoved] != 0 || n != n_old) {
+    // the block list changed: the blocks outside the region move to their new positions in a
+    // second pair of planes, which then becomes the retained one
+    CG_CUDA(ctx->esdf_dist_next.reserve(n * kVoxelsPerBlock * sizeof(float)));
+    CG_CUDA(ctx->esdf_packed_next.reserve(n * kVoxelsPerBlock * sizeof(uint32_t)));
+    if (n_region < n) {
+      ctx->own_launches += 1;
+      k_esdf_remap<<<wide, kEsdfThreads, 0, s>>>(region, old_b, static_cast<uint32_t>(n),
+                                                 ctx->esdf_dist.as<float4>(), ctx->esdf_packed.as<uint4>(),
+                                                 ctx->esdf_dist_next.as<float4>(),
+                                                 ctx->esdf_packed_next.as<uint4>());
+    }
+    std::swap(ctx->esdf_dist, ctx->esdf_dist_next);
+    std::swap(ctx->esdf_packed, ctx->esdf_packed_next);
+    // k_esdf_match has read the retained keys (stream order) before they are replaced
+    CG_CUDA(ctx->esdf_keys.reserve(n * sizeof(uint64_t)));
+    CG_CUDA(ctx->esdf_index.reserve(n * 3 * sizeof(int32_t)));
+    CG_CUDA(cudaMemcpyAsync(ctx->esdf_keys.p, keys, n * sizeof(uint64_t), cudaMemcpyDeviceToDevice, s));
+    ctx->own_launches += 1;
+    k_esdf_unpack_idx<<<grid_for(n, 256), 256, 0, s>>>(ctx->esdf_keys.as<uint64_t>(),
+                                                       static_cast<uint32_t>(n),
+                                                       ctx->esdf_index.as<int32_t>());
+  }
+  // the sweeps read the layer's hash and these keys; the slots stay sort_blocks' (this call only)
+  keys = ctx->esdf_keys.as<uint64_t>();
+  uint64_t sweeps = 0, passes = 0;
+  if (n_region) {
+    const unsigned grid = std::min<unsigned>(n_region, static_cast<unsigned>(ctx->num_sms) * 16u);
+    ctx->own_launches += 1;
+    k_esdf_init<<<grid, kEsdfThreads, 0, s>>>(L->v, slots, region_list, n_region, P,
+                                              ctx->esdf_dist.as<float>(), ctx->esdf_fixed.as<uint32_t>(),
+                                              slot_to_b, ctx->esdf_dirty.as<uint8_t>(), nullptr);
+    rc = run_sweeps(ctx, L, keys, n, P, region, &sweeps, &passes, "cg_layer_esdf_update");
+    if (rc) return rc;
+    ctx->own_launches += 1;
+    k_esdf_finish<<<grid, kEsdfThreads, 0, s>>>(L->v, keys, slots, region_list, n_region, P,
+                                                ctx->esdf_dist.as<float>(), ctx->esdf_fixed.as<uint32_t>(),
+                                                slot_to_b, ctx->esdf_packed.as<uint32_t>());
+    CG_CUDA(cudaStreamSynchronize(s));
+  }
+  CG_CUDA(cudaGetLastError());
+  if (stats) {
+    stats->blocks = n;
+    stats->observed_voxels = h_counters[0];
+    stats->fixed_voxels = h_counters[1];
+    stats->sweeps = sweeps;
+    stats->block_passes = passes;
+  }
+  if (ust) {
+    ust->blocks_changed = h_ucount[kUcChanged];
+    ust->blocks_removed = h_ucount[kUcRemoved];
+    ust->blocks_region = n_region;
+  }
+  return retain(ctx, L, cfg, n);
 }
 
 int32_t cg_esdf_fetch(cg_context* ctx, size_t capacity_blocks, int32_t* block_idx, float* distance,

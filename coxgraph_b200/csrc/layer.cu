@@ -7,6 +7,7 @@
 #include <thrust/iterator/counting_iterator.h>
 
 #include <algorithm>
+#include <atomic>
 
 #include "cg_internal.cuh"
 #include "host_stage.cuh"
@@ -559,7 +560,9 @@ int32_t cg_context_destroy(cg_context* ctx) {
                     &ctx->mesh_cols_c, &ctx->mesh_frames, &ctx->esdf_keys, &ctx->esdf_slots,
                     &ctx->esdf_dist, &ctx->esdf_packed, &ctx->esdf_fixed,
                     &ctx->esdf_slot_to_b, &ctx->esdf_dirty, &ctx->esdf_list, &ctx->esdf_index,
-                    &ctx->esdf_counters, &ctx->weld_keys, &ctx->weld_words, &ctx->weld_out};
+                    &ctx->esdf_counters, &ctx->esdf_dist_next, &ctx->esdf_packed_next,
+                    &ctx->esdf_old_b, &ctx->esdf_sources, &ctx->esdf_region,
+                    &ctx->esdf_region_list, &ctx->weld_keys, &ctx->weld_words, &ctx->weld_out};
   for (DevBuf* b : bufs) b->release();
   drain_events(ctx);
   for (cudaEvent_t e : ctx->event_pool) cudaEventDestroy(e);
@@ -650,6 +653,8 @@ int32_t cg_layer_create(cg_context* ctx, float voxel_size, int32_t vps, size_t m
   *out = nullptr;
   CG_CUDA(cudaSetDevice(ctx->device));
   cg_layer* L = new cg_layer();
+  static std::atomic<uint64_t> next_serial{1};
+  L->serial = next_serial.fetch_add(1);
   L->ctx = ctx;
   L->max_blocks = max_blocks;
   size_t cap = 1024;

@@ -519,6 +519,15 @@ class EsdfIntegrator {
   void updateFromTsdfLayerBatch(cg_esdf_stats* stats = nullptr) {
     check(cg_layer_esdf_batch(tsdf_layer_->handle(), &config_, stats));
   }
+  // updateFromTsdfLayer: re-solves only the blocks within reach of what changed in the TSDF layer
+  // since the ESDF retained in the context was computed; bit-identical to the batch.  Changes are
+  // found by content, so `clear_updated_flag` is accepted and ignored (the layer's updated flags
+  // belong to the mesher and the serialiser), as min_diff_m is.
+  void updateFromTsdfLayer(bool clear_updated_flag = false, cg_esdf_stats* stats = nullptr,
+                           cg_esdf_update_stats* update_stats = nullptr) {
+    (void)clear_updated_flag;
+    check(cg_layer_esdf_update(tsdf_layer_->handle(), &config_, stats, update_stats));
+  }
   // Layer<EsdfVoxel>: blocks in (z, y, x) order, 4096 voxels each
   void getEsdfLayer(BlockIndexList* block_indices, std::vector<EsdfVoxel>* voxels) const {
     size_t nb = 0;

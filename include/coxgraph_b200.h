@@ -437,6 +437,26 @@ void cg_esdf_config_default(cg_esdf_config* cfg);
  * stays in the layer's context until the next call. */
 int32_t cg_layer_esdf_batch(const cg_layer* tsdf_layer, const cg_esdf_config* cfg,
                             cg_esdf_stats* stats);
+/* voxblox::EsdfIntegrator::updateFromTsdfLayer(), the incremental form: brings the ESDF retained in
+ * the context up to date with `tsdf_layer`, re-solving only the blocks within reach of what
+ * changed.  On return the retained ESDF is bit-identical to what cg_layer_esdf_batch(tsdf_layer,
+ * cfg) leaves (block list and order, distances, packed words).  Changes are found by comparing the
+ * layer's content with the retained result, so the layer's `updated` flags are neither read nor
+ * cleared and any writer of the layer is covered.  When there is nothing to start from — no ESDF
+ * retained (or an empty one), one of another layer, one computed under other max_distance_m,
+ * default_distance_m, min_distance_m, min_weight or add_occupied_crust, or a layer without
+ * blocks — the call runs the batch and sets full_rebuild.  Config rules and errors are the batch's; a rejected call leaves the
+ * retained ESDF untouched.  `stats`: blocks / observed_voxels / fixed_voxels are whole-map totals,
+ * sweeps / block_passes this call's.  Either stats pointer may be NULL. */
+typedef struct cg_esdf_update_stats {
+  uint64_t blocks_changed;   /* current blocks whose init state changed, new blocks included */
+  uint64_t blocks_removed;   /* retained blocks the layer no longer has */
+  uint64_t blocks_region;    /* blocks re-solved: those within reach of a changed or removed one */
+  int32_t full_rebuild;      /* 1: ran as the batch (all blocks changed and re-solved) */
+  int32_t reserved;
+} cg_esdf_update_stats;
+int32_t cg_layer_esdf_update(const cg_layer* tsdf_layer, const cg_esdf_config* cfg,
+                             cg_esdf_stats* stats, cg_esdf_update_stats* update_stats);
 /* Copies the retained ESDF out: blocks in (z, y, x) order, distance float[B*4096] and
  * packed uint32[B*4096] by linear voxel index — the two words Block<EsdfVoxel>::serializeToIntegers
  * emits per voxel: packed = parent.x << 24 | parent.y << 16 | parent.z << 8 | flags (int8 parent
