@@ -199,23 +199,7 @@ class Layer:
         """voxblox::MeshIntegrator<TsdfVoxel>::generateMesh on the device (marching cubes per
         block) -> (block_idx int32 [B,3] in (z,y,x) order, vertex_begin u32 [B+1], vertices f32
         [V,3], normals f32 [V,3], colors u8 [V,4]); three consecutive vertices = one triangle."""
-        lib = capi.load()
-        nb, nv = C.c_size_t(0), C.c_size_t(0)
-        capi.check(lib.cg_layer_mesh(self._h, min_weight, int(use_color), int(only_updated), 0, 0,
-                                     None, None, None, None, None, C.byref(nb), C.byref(nv)))
-        B, V = nb.value, nv.value
-        if not fetch:  # the mesh stays on the device (cg_mesh_fetch copies it out later)
-            return B, V
-        idx = np.zeros((B, 3), np.int32)
-        begin = np.zeros(B + 1, np.uint32)
-        v = np.zeros((V, 3), np.float32)
-        n = np.zeros((V, 3), np.float32)
-        c = np.zeros((V, 4), np.uint8)
-        if B:
-            capi.check(lib.cg_mesh_fetch(self.ctx._h, B, V, _ptr(idx), _ptr(begin),
-                                         _ptr(v) if V else None, _ptr(n) if V else None,
-                                         _ptr(c) if V else None))
-        return idx, begin, v, n, c
+        return _mesh(capi.load().cg_layer_mesh, self, min_weight, use_color, only_updated, fetch)
 
     def getConnectedMesh(self, fetch=True):
         """MeshLayer::getConnectedMesh (voxblox::createConnectedMesh) of the mesh the last
@@ -325,6 +309,26 @@ class Layer:
         fl = None if flags is None else np.ascontiguousarray(flags, np.uint8)
         capi.check(capi.load().cg_layer_upload(self._h, len(idx), _ptr(idx), _ptr(vox),
                                                None if fl is None else _ptr(fl)))
+
+
+def _mesh(entry, layer, min_weight, use_color, only_updated, fetch):
+    """cg_layer_mesh or cg_layer_mesh_sharded (`entry`), then cg_mesh_fetch: Layer.generateMesh."""
+    nb, nv = C.c_size_t(0), C.c_size_t(0)
+    capi.check(entry(layer._h, min_weight, int(use_color), int(only_updated), 0, 0, None, None,
+                     None, None, None, C.byref(nb), C.byref(nv)))
+    B, V = nb.value, nv.value
+    if not fetch:  # the mesh stays on the device (cg_mesh_fetch copies it out later)
+        return B, V
+    idx = np.zeros((B, 3), np.int32)
+    begin = np.zeros(B + 1, np.uint32)
+    v = np.zeros((V, 3), np.float32)
+    n = np.zeros((V, 3), np.float32)
+    c = np.zeros((V, 4), np.uint8)
+    if B:
+        capi.check(capi.load().cg_mesh_fetch(layer.ctx._h, B, V, _ptr(idx), _ptr(begin),
+                                             _ptr(v) if V else None, _ptr(n) if V else None,
+                                             _ptr(c) if V else None))
+    return idx, begin, v, n, c
 
 
 class TsdfIntegrator:
@@ -645,6 +649,23 @@ def getProjectedMapSharded(submap_layers, submap_poses, partial_layer, owned_lay
     arr = (C.c_void_p * max(n, 1))(*[l._h for l in submap_layers])
     capi.check(capi.load().cg_project_submaps_sharded(arr, _ptr(P) if n else None, n,
                                                       partial_layer._h, owned_layer._h, None))
+
+
+def generateMeshSharded(owned_layer, min_weight=1e-4, use_color=True, only_updated=False,
+                        fetch=True):
+    """Collective: generateMesh over the sharded global map, every rank with its owned layer.  Each
+    rank gets the meshes of the blocks it holds, byte for byte what generateMesh gives for them on
+    one layer holding every rank's owned blocks (neighbour and colour blocks are read from the
+    peers).  Same tuple as Layer.generateMesh."""
+    return _mesh(capi.load().cg_layer_mesh_sharded, owned_layer, min_weight, use_color,
+                 only_updated, fetch)
+
+
+def commPeerMappings(ctx):
+    """(peer mappings opened since commInit, open now) of the context's communicator."""
+    opened, now = C.c_uint64(0), C.c_uint64(0)
+    capi.check(capi.load().cg_comm_peer_mappings(ctx._h, C.byref(opened), C.byref(now)))
+    return int(opened.value), int(now.value)
 
 
 def reprojectSubmaps(submap_layers, poses_old, poses_new, global_layer, eps_translation=0.0,

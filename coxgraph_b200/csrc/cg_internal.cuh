@@ -127,6 +127,32 @@ struct LayerView {
   }
 };
 
+// Block lookup of cg_layer_mesh_sharded (the interface of mesh.cu's LocalBlocks): this rank's own
+// hash first, then the key map that comm.cu builds over every rank's owned layer, whose entries
+// point at the block's planes in its holder's pool (a peer pool is read over NVLink through its
+// CUDA IPC mapping).  A reference is a pool slot of this layer (>= 0), -1 for a block no rank
+// holds, or -2 - (map entry) for a block found in the map.
+struct ShardedBlocks {
+  const unsigned long long* keys;  // [cap_mask + 1] block key or kEmptyKey
+  const float* const* planes_of;   // [cap_mask + 1] the block's distance plane
+  uint32_t cap_mask;
+
+  __device__ __forceinline__ int find(const LayerView& L, uint64_t key) const {
+    const int s = L.find_slot(key);
+    if (s >= 0) return s;
+    uint32_t h = hash_key(key) & cap_mask;
+    for (;;) {
+      const unsigned long long k = keys[h];
+      if (k == key) return -2 - static_cast<int>(h);
+      if (k == kEmptyKey) return -1;
+      h = (h + 1) & cap_mask;
+    }
+  }
+  __device__ __forceinline__ const float* planes(const LayerView& L, int ref) const {
+    return ref >= 0 ? L.dist_plane(ref) : planes_of[-2 - ref];
+  }
+};
+
 // ------------------------------------------------------------------ host-side state
 struct DevBuf {
   void* p = nullptr;
@@ -364,6 +390,13 @@ int32_t sort_blocks(const cg_layer* layer, const uint64_t** keys, const uint32_t
 // Layer::removeBlock for every slot with d_remove[slot] != 0 (device flags, one per claimed slot):
 // compacts the pool, rebuilds the hash; enqueued on the context's stream, host mirror updated
 int32_t remove_flagged_blocks(cg_layer* layer, const uint8_t* d_remove, uint64_t* removed_out);
+// comm.cu: the collective steps of cg_layer_mesh_sharded.  sharded_mesh_open binds the owned layer
+// (collective, once per layer), publishes its block count, waits at a barrier for every rank and
+// builds the key map over every rank's owned layer; the smallest key two ranks hold goes to the
+// device word *dup_key (kEmptyKey: none).  All of it is stream-ordered.  sharded_mesh_close is the
+// closing barrier: no rank changes its owned layer while a peer still reads it.
+int32_t sharded_mesh_open(const cg_layer* owned, unsigned long long* dup_key, ShardedBlocks* out);
+int32_t sharded_mesh_close(cg_context* ctx);
 
 #define CG_CUDA(expr)                                         \
   do {                                                        \

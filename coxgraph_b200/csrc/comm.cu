@@ -20,6 +20,13 @@
 // one-word all-reduce on the stream before and after the kernels (all partial layers complete /
 // all peers done reading).  The fold order is fixed, so the result is deterministic and equal to
 // the packed exchange of exchange.cu (hash owner, NCCL all-to-all) block for block.
+//
+// cg_layer_mesh_sharded (mesh.cu) meshes the owned layers where they lie.  Its collective half is
+// here: the owned layer is bound like the partial one (its own binding, so alternating gather and
+// mesh calls map nothing again), and k_build_holders, run over every rank's owned keys, also
+// records where each block's planes are.  The mesh kernel resolves the one-block halo (the +x/+y/+z
+// neighbours and a vertex's colour block) through that map and reads the peer's planes over
+// NVLink; a key two ranks hold is found while the map is built.
 #include <dlfcn.h>
 #include <string.h>
 
@@ -79,12 +86,12 @@ static int32_t load_nccl() {
     }                                                                        \
   } while (0)
 
-// What a peer needs of a rank's partial layer (device pointers valid in the READER's process).
+// What a peer needs of a rank's bound layer (device pointers valid in the READER's process).
 struct PeerLayer {
   const float* pool;
   const uint64_t* block_keys;
   const uint8_t* has_data;
-  const uint32_t* shared;  // [0] number of blocks of the partial layer (written per call)
+  const uint32_t* shared;  // [0] number of blocks of the layer (written per call)
 };
 constexpr int kMaxRanks = 64;
 
@@ -96,17 +103,34 @@ struct IpcRecord {  // one per rank, all-gathered
   int pad;
 };
 
+// One role a layer of this rank plays for its peers (the partial layer of cg_gather_global, the
+// owned layer of cg_layer_mesh_sharded): its block count published in `shared`, and every rank's
+// buffers as this process sees them.  Pools are allocated once in cg_layer_create, so a binding
+// holds for the layer's lifetime; it is made again only when a layer of another serial takes the
+// role.
+struct Binding {
+  uint64_t serial = 0;            // cg_layer::serial of the bound layer (0: none)
+  uint32_t* shared = nullptr;     // peer-visible: [0] blocks of this rank's layer (written per call)
+  PeerLayer* d_peers = nullptr;   // [nranks]
+  std::vector<char*> held;        // peer mappings this binding uses (one reference each)
+};
+// A peer allocation mapped into this process.  Small buffers of different layers can share one
+// allocation, and a handle can be opened once only, so the bindings share the mappings.
+struct Mapping {
+  int rank;
+  cudaIpcMemHandle_t handle;
+  char* p;
+  int refs;
+};
 }  // namespace cg
 
 struct cg_comm {
   cg::ncclComm_t comm = nullptr;
   int rank = 0, nranks = 1;
   int* d_token = nullptr;             // barrier word
-  // binding of one partial layer
-  const cg_layer* bound = nullptr;
-  uint32_t* shared = nullptr;         // peer-visible: [0] blocks of this rank's partial layer
-  std::vector<void*> opened;          // peer mappings to close
-  cg::PeerLayer* d_peers = nullptr;   // [nranks]
+  cg::Binding partial, owned;
+  std::vector<cg::Mapping> maps;
+  uint64_t maps_opened = 0;           // cudaIpcOpenMemHandle calls since cg_comm_init
   // the holder map (scratch, rebuilt every call): block key -> set of ranks holding the block
   unsigned long long* hkeys = nullptr;
   unsigned long long* hmask = nullptr;
@@ -115,6 +139,12 @@ struct cg_comm {
   uint32_t* slots = nullptr;          // pool slots of the holders' copies, per owned block
   uint32_t* counters = nullptr;       // [0] owned entries, [1] slot list cursor, [2] overflow
   size_t hcap = 0, list_cap = 0;
+  // the key map of cg_layer_mesh_sharded over every rank's owned layer (rebuilt every call)
+  unsigned long long* mkeys = nullptr;
+  unsigned long long* mmask = nullptr;
+  const float** mplanes = nullptr;    // the block's distance plane in its holder's pool
+  uint32_t* mcounters = nullptr;      // k_build_holders' words ([2] overflow: cannot happen)
+  size_t mcap = 0;
 };
 
 namespace cg {
@@ -134,10 +164,13 @@ __device__ __forceinline__ int pick_owner(unsigned long long key, unsigned long 
   return __ffsll(static_cast<long long>(m)) - 1;
 }
 
-// Every block key of every rank's partial layer (read through the peer mappings) enters the map
-// with its rank's bit.  Grid y = rank.
+// Every block key of every rank's layer (read through the peer mappings) enters the map with its
+// rank's bit.  Grid y = rank.  With `planes` (the key map of cg_layer_mesh_sharded) the entry also
+// records where the block's planes are, and a key that reaches an entry another rank has already
+// marked is held twice: the smallest such key goes to *dup_key.
 __global__ void k_build_holders(const PeerLayer* __restrict__ peers, unsigned long long* hkeys,
-                                unsigned long long* hmask, uint32_t hcap_mask, uint32_t* counters) {
+                                unsigned long long* hmask, uint32_t hcap_mask, uint32_t* counters,
+                                const float** planes, unsigned long long* dup_key) {
   const int r = blockIdx.y;
   const PeerLayer P = peers[r];
   const uint32_t n = P.shared[0];
@@ -157,7 +190,11 @@ __global__ void k_build_holders(const PeerLayer* __restrict__ peers, unsigned lo
         return;
       }
     }
-    atomicOr(&hmask[h], 1ull << r);
+    const unsigned long long held = atomicOr(&hmask[h], 1ull << r);
+    if (planes) {
+      planes[h] = P.pool + static_cast<size_t>(i) * (3 * kVoxelsPerBlock);
+      if (held) atomicMin(dup_key, key);
+    }
   }
 }
 // entries this rank owns, each with room for its holders' slots
@@ -326,15 +363,37 @@ static int32_t ipc_of(const void* p, cudaIpcMemHandle_t* h, unsigned long long* 
   return CG_OK;
 }
 
+static void release(cg_comm* c, Binding& b) {
+  for (char* p : b.held) {
+    for (size_t i = 0; i < c->maps.size(); ++i) {
+      if (c->maps[i].p != p) continue;
+      if (--c->maps[i].refs == 0) {
+        cudaIpcCloseMemHandle(p);
+        c->maps.erase(c->maps.begin() + static_cast<long>(i));
+      }
+      break;
+    }
+  }
+  b.held.clear();
+  b.serial = 0;
+}
+
 static void unbind(cg_comm* c) {
-  for (void* p : c->opened) cudaIpcCloseMemHandle(p);
-  c->opened.clear();
-  void* bufs[] = {c->shared, c->hkeys, c->hmask, c->hbase, c->mine, c->slots, c->counters};
-  for (void* b : bufs)
-    if (b) cudaFree(b);
-  c->shared = c->hbase = c->mine = c->slots = c->counters = nullptr;
-  c->hkeys = c->hmask = nullptr;
-  c->bound = nullptr;
+  for (Binding* b : {&c->partial, &c->owned}) {
+    release(c, *b);
+    if (b->shared) cudaFree(b->shared);
+    if (b->d_peers) cudaFree(b->d_peers);
+    b->shared = nullptr;
+    b->d_peers = nullptr;
+  }
+  void* bufs[] = {c->hkeys, c->hmask, c->hbase, c->mine, c->slots, c->counters,
+                  c->mkeys, c->mmask, c->mplanes, c->mcounters};
+  for (void* p : bufs)
+    if (p) cudaFree(p);
+  c->hbase = c->mine = c->slots = c->counters = c->mcounters = nullptr;
+  c->hkeys = c->hmask = c->mkeys = c->mmask = nullptr;
+  c->mplanes = nullptr;
+  c->hcap = c->list_cap = c->mcap = 0;
 }
 
 static int32_t barrier(cg_context* ctx) {
@@ -343,34 +402,33 @@ static int32_t barrier(cg_context* ctx) {
   return CG_OK;
 }
 
-// All ranks call this with their own partial layer (collective): IPC handles exchanged, peer
-// mappings opened, scratch of the holder map sized for every block of every rank.  Done once per
-// partial layer (it stays bound until another one is used).
-static int32_t bind_partial(cg_context* ctx, const cg_layer* partial) {
+// the block key map of every layer of one role over all ranks: twice the blocks all ranks can hold
+static size_t map_capacity(size_t max_blocks, int nranks) {
+  size_t cap = 1024;
+  while (cap < 2 * max_blocks * static_cast<size_t>(nranks)) cap <<= 1;
+  return cap;
+}
+
+// All ranks call this with their own layer of one role (collective): IPC handles all-gathered, the
+// layers checked against each other (same voxel size and max_blocks; every rank sees every record,
+// so every rank rejects a mismatch), then the peers' buffers mapped.
+static int32_t bind(cg_context* ctx, const cg_layer* layer, Binding& b, const char* who) {
   cg_comm* c = ctx->comm;
-  unbind(c);
+  release(c, b);
   cudaStream_t s = ctx->stream;
   const int R = c->nranks;
-  c->list_cap = partial->max_blocks * static_cast<size_t>(R);  // blocks over all ranks
-  c->hcap = 1024;
-  while (c->hcap < 2 * c->list_cap) c->hcap <<= 1;
-  CG_CUDA(cudaMalloc(&c->shared, 64));
-  CG_CUDA(cudaMalloc(&c->hkeys, c->hcap * sizeof(unsigned long long)));
-  CG_CUDA(cudaMalloc(&c->hmask, c->hcap * sizeof(unsigned long long)));
-  CG_CUDA(cudaMalloc(&c->hbase, c->hcap * sizeof(uint32_t)));
-  CG_CUDA(cudaMalloc(&c->mine, c->list_cap * sizeof(uint32_t)));
-  CG_CUDA(cudaMalloc(&c->slots, c->list_cap * sizeof(uint32_t)));
-  CG_CUDA(cudaMalloc(&c->counters, 4 * sizeof(uint32_t)));
-  CG_CUDA(cudaMemsetAsync(c->shared, 0, 64, s));
+  if (!b.shared) CG_CUDA(cudaMalloc(&b.shared, 64));
+  if (!b.d_peers) CG_CUDA(cudaMalloc(&b.d_peers, sizeof(PeerLayer) * R));
+  CG_CUDA(cudaMemsetAsync(b.shared, 0, 64, s));
   IpcRecord mine;
   memset(&mine, 0, sizeof(mine));
   int32_t rc;
-  if ((rc = ipc_of(partial->v.pool, &mine.pool, &mine.off_pool))) return rc;
-  if ((rc = ipc_of(partial->v.block_keys, &mine.keys, &mine.off_keys))) return rc;
-  if ((rc = ipc_of(partial->v.has_data, &mine.flags, &mine.off_flags))) return rc;
-  if ((rc = ipc_of(c->shared, &mine.shared, &mine.off_shared))) return rc;
-  mine.max_blocks = partial->max_blocks;
-  mine.voxel_size = partial->v.voxel_size;
+  if ((rc = ipc_of(layer->v.pool, &mine.pool, &mine.off_pool))) return rc;
+  if ((rc = ipc_of(layer->v.block_keys, &mine.keys, &mine.off_keys))) return rc;
+  if ((rc = ipc_of(layer->v.has_data, &mine.flags, &mine.off_flags))) return rc;
+  if ((rc = ipc_of(b.shared, &mine.shared, &mine.off_shared))) return rc;
+  mine.max_blocks = layer->max_blocks;
+  mine.voxel_size = layer->v.voxel_size;
   void* d_all = nullptr;
   CG_CUDA(cudaMalloc(&d_all, sizeof(IpcRecord) * R));
   CG_CUDA(cudaMemcpyAsync(static_cast<char*>(d_all) + sizeof(IpcRecord) * c->rank, &mine,
@@ -381,46 +439,125 @@ static int32_t bind_partial(cg_context* ctx, const cg_layer* partial) {
   CG_CUDA(cudaMemcpyAsync(all.data(), d_all, sizeof(IpcRecord) * R, cudaMemcpyDeviceToHost, s));
   CG_CUDA(cudaStreamSynchronize(s));
   cudaFree(d_all);
-  std::vector<PeerLayer> peers(R);
   for (int r = 0; r < R; ++r) {
-    if (all[r].max_blocks != partial->max_blocks || all[r].voxel_size != partial->v.voxel_size) {
-      set_error("cg_gather_global: rank %d's partial layer differs (max_blocks / voxel size)", r);
+    if (all[r].max_blocks != layer->max_blocks || all[r].voxel_size != layer->v.voxel_size) {
+      set_error("%s: rank %d's layer differs from rank %d's (max_blocks %llu / %zu, voxel size %g / %g)",
+                who, r, c->rank, all[r].max_blocks, layer->max_blocks,
+                static_cast<double>(all[r].voxel_size), static_cast<double>(layer->v.voxel_size));
       return CG_ERR_INVALID_ARG;
     }
+  }
+  std::vector<PeerLayer> peers(R);
+  for (int r = 0; r < R; ++r) {
     if (r == c->rank) {
-      peers[r] = PeerLayer{partial->v.pool, partial->v.block_keys, partial->v.has_data, c->shared};
+      peers[r] = PeerLayer{layer->v.pool, layer->v.block_keys, layer->v.has_data, b.shared};
       continue;
     }
-    // several buffers of a peer may live in one allocation: a handle can be opened once only
     const cudaIpcMemHandle_t* hs[4] = {&all[r].pool, &all[r].keys, &all[r].flags, &all[r].shared};
     const unsigned long long offs[4] = {all[r].off_pool, all[r].off_keys, all[r].off_flags,
                                         all[r].off_shared};
     char* mapped[4] = {nullptr, nullptr, nullptr, nullptr};
     for (int k = 0; k < 4; ++k) {
-      for (int j = 0; j < k; ++j)
-        if (memcmp(hs[j], hs[k], sizeof(cudaIpcMemHandle_t)) == 0) mapped[k] = mapped[j];
+      for (Mapping& m : c->maps) {
+        if (m.rank == r && memcmp(&m.handle, hs[k], sizeof(cudaIpcMemHandle_t)) == 0) {
+          ++m.refs;
+          mapped[k] = m.p;
+          break;
+        }
+      }
       if (!mapped[k]) {
         void* p = nullptr;
         const cudaError_t e = cudaIpcOpenMemHandle(&p, *hs[k], cudaIpcMemLazyEnablePeerAccess);
         if (e != cudaSuccess) {
-          set_error("cudaIpcOpenMemHandle (rank %d's partial layer) failed: %s", r,
-                    cudaGetErrorString(e));
+          set_error("cudaIpcOpenMemHandle (rank %d's layer) failed: %s", r, cudaGetErrorString(e));
           return CG_ERR_CUDA;
         }
-        c->opened.push_back(p);
+        ++c->maps_opened;
         mapped[k] = static_cast<char*>(p);
+        c->maps.push_back(Mapping{r, *hs[k], mapped[k], 1});
       }
+      b.held.push_back(mapped[k]);
     }
     peers[r] = PeerLayer{reinterpret_cast<const float*>(mapped[0] + offs[0]),
                          reinterpret_cast<const uint64_t*>(mapped[1] + offs[1]),
                          reinterpret_cast<const uint8_t*>(mapped[2] + offs[2]),
                          reinterpret_cast<const uint32_t*>(mapped[3] + offs[3])};
   }
-  CG_CUDA(cudaMemcpyAsync(c->d_peers, peers.data(), sizeof(PeerLayer) * R, cudaMemcpyHostToDevice, s));
+  CG_CUDA(cudaMemcpyAsync(b.d_peers, peers.data(), sizeof(PeerLayer) * R, cudaMemcpyHostToDevice, s));
   CG_CUDA(cudaStreamSynchronize(s));
-  c->bound = partial;
+  b.serial = layer->serial;
   return CG_OK;
 }
+
+// the partial layer of cg_gather_global, with the holder map's scratch sized for it
+static int32_t bind_partial(cg_context* ctx, const cg_layer* partial) {
+  cg_comm* c = ctx->comm;
+  const size_t list_cap = partial->max_blocks * static_cast<size_t>(c->nranks);
+  const size_t hcap = map_capacity(partial->max_blocks, c->nranks);
+  if (hcap != c->hcap || list_cap != c->list_cap) {
+    void* bufs[] = {c->hkeys, c->hmask, c->hbase, c->mine, c->slots, c->counters};
+    for (void* p : bufs)
+      if (p) cudaFree(p);
+    c->hkeys = c->hmask = nullptr;
+    c->hbase = c->mine = c->slots = c->counters = nullptr;
+    c->hcap = c->list_cap = 0;
+    CG_CUDA(cudaMalloc(&c->hkeys, hcap * sizeof(unsigned long long)));
+    CG_CUDA(cudaMalloc(&c->hmask, hcap * sizeof(unsigned long long)));
+    CG_CUDA(cudaMalloc(&c->hbase, hcap * sizeof(uint32_t)));
+    CG_CUDA(cudaMalloc(&c->mine, list_cap * sizeof(uint32_t)));
+    CG_CUDA(cudaMalloc(&c->slots, list_cap * sizeof(uint32_t)));
+    CG_CUDA(cudaMalloc(&c->counters, 4 * sizeof(uint32_t)));
+    c->hcap = hcap;
+    c->list_cap = list_cap;
+  }
+  return bind(ctx, partial, c->partial, "cg_gather_global");
+}
+
+// the owned layer of cg_layer_mesh_sharded, with the key map's scratch sized for it
+static int32_t bind_owned(cg_context* ctx, const cg_layer* owned) {
+  cg_comm* c = ctx->comm;
+  const size_t mcap = map_capacity(owned->max_blocks, c->nranks);
+  if (mcap != c->mcap) {
+    void* bufs[] = {c->mkeys, c->mmask, c->mplanes, c->mcounters};
+    for (void* p : bufs)
+      if (p) cudaFree(p);
+    c->mkeys = c->mmask = nullptr;
+    c->mplanes = nullptr;
+    c->mcounters = nullptr;
+    c->mcap = 0;
+    CG_CUDA(cudaMalloc(&c->mkeys, mcap * sizeof(unsigned long long)));
+    CG_CUDA(cudaMalloc(&c->mmask, mcap * sizeof(unsigned long long)));
+    CG_CUDA(cudaMalloc(&c->mplanes, mcap * sizeof(const float*)));
+    CG_CUDA(cudaMalloc(&c->mcounters, 4 * sizeof(uint32_t)));
+    c->mcap = mcap;
+  }
+  return bind(ctx, owned, c->owned, "cg_layer_mesh_sharded");
+}
+
+int32_t sharded_mesh_open(const cg_layer* owned, unsigned long long* dup_key, ShardedBlocks* out) {
+  cg_context* ctx = owned->ctx;
+  cg_comm* c = ctx->comm;
+  cudaStream_t s = ctx->stream;
+  int32_t rc;
+  if (c->owned.serial != owned->serial && (rc = bind_owned(ctx, owned))) return rc;
+  ctx->own_launches += 2;
+  k_publish_blocks<<<1, 1, 0, s>>>(c->owned.shared, static_cast<int>(owned->num_blocks));
+  CG_CUDA(cudaMemsetAsync(c->mkeys, 0xFF, c->mcap * sizeof(unsigned long long), s));
+  CG_CUDA(cudaMemsetAsync(c->mmask, 0, c->mcap * sizeof(unsigned long long), s));
+  CG_CUDA(cudaMemsetAsync(c->mcounters, 0, 4 * sizeof(uint32_t), s));
+  CG_CUDA(cudaMemsetAsync(dup_key, 0xFF, sizeof(unsigned long long), s));
+  // every rank's owned layer is complete and its block count published (stream-ordered)
+  if ((rc = barrier(ctx))) return rc;
+  const uint32_t cap_mask = static_cast<uint32_t>(c->mcap - 1);
+  const dim3 per_rank(static_cast<unsigned>(ctx->num_sms), static_cast<unsigned>(c->nranks));
+  k_build_holders<<<per_rank, 256, 0, s>>>(c->owned.d_peers, c->mkeys, c->mmask, cap_mask,
+                                           c->mcounters, c->mplanes, dup_key);
+  CG_CUDA(cudaGetLastError());
+  *out = ShardedBlocks{c->mkeys, c->mplanes, cap_mask};
+  return CG_OK;
+}
+
+int32_t sharded_mesh_close(cg_context* ctx) { return barrier(ctx); }
 
 }  // namespace cg
 
@@ -462,8 +599,7 @@ int32_t cg_comm_init(cg_context* ctx, const uint8_t id[CG_COMM_ID_BYTES], int32_
     delete c;
     return CG_ERR_CUDA;
   }
-  if (cudaMalloc(&c->d_token, sizeof(int)) != cudaSuccess ||
-      cudaMalloc(&c->d_peers, sizeof(PeerLayer) * nranks) != cudaSuccess) {
+  if (cudaMalloc(&c->d_token, sizeof(int)) != cudaSuccess) {
     set_error("cg_comm_init: out of device memory");
     return CG_ERR_CUDA;
   }
@@ -480,10 +616,19 @@ int32_t cg_comm_destroy(cg_context* ctx) {
   cudaStreamSynchronize(ctx->stream);
   unbind(c);
   if (c->d_token) cudaFree(c->d_token);
-  if (c->d_peers) cudaFree(c->d_peers);
   if (c->comm) g_nccl.CommDestroy(c->comm);
   delete c;
   ctx->comm = nullptr;
+  return CG_OK;
+}
+
+int32_t cg_comm_peer_mappings(const cg_context* ctx, uint64_t* opened_total, uint64_t* open_now) {
+  if (!ctx || !ctx->comm) {
+    set_error("cg_comm_peer_mappings: the context has no communicator");
+    return CG_ERR_INVALID_ARG;
+  }
+  if (opened_total) *opened_total = ctx->comm->maps_opened;
+  if (open_now) *open_now = ctx->comm->maps.size();
   return CG_OK;
 }
 
@@ -505,7 +650,7 @@ int32_t cg_gather_global(const cg_layer* partial, cg_layer* owned, uint64_t* blo
   CG_CUDA(cudaSetDevice(ctx->device));
   cudaStream_t s = ctx->stream;
   int32_t rc;
-  if (c->bound != partial && (rc = bind_partial(ctx, partial))) return rc;
+  if (c->partial.serial != partial->serial && (rc = bind_partial(ctx, partial))) return rc;
   // CG_TRACE_COMM=1: per-phase device times of the exchange on stderr (diagnostics only)
   static const bool trace = getenv("CG_TRACE_COMM") != nullptr;
   cudaEvent_t tev[6] = {};
@@ -521,7 +666,7 @@ int32_t cg_gather_global(const cg_layer* partial, cg_layer* owned, uint64_t* blo
   const uint32_t hmask_cap = static_cast<uint32_t>(c->hcap - 1);
   const uint32_t list_cap = static_cast<uint32_t>(std::min<size_t>(c->list_cap, 0xFFFFFFF0u));
   ctx->own_launches += 6;
-  k_publish_blocks<<<1, 1, 0, s>>>(c->shared, static_cast<int>(partial->num_blocks));
+  k_publish_blocks<<<1, 1, 0, s>>>(c->partial.shared, static_cast<int>(partial->num_blocks));
   CG_CUDA(cudaMemsetAsync(c->hkeys, 0xFF, c->hcap * sizeof(unsigned long long), s));
   CG_CUDA(cudaMemsetAsync(c->hmask, 0, c->hcap * sizeof(unsigned long long), s));
   CG_CUDA(cudaMemsetAsync(c->counters, 0, 4 * sizeof(uint32_t), s));
@@ -530,10 +675,11 @@ int32_t cg_gather_global(const cg_layer* partial, cg_layer* owned, uint64_t* blo
   if ((rc = barrier(ctx))) return rc;
   mark();
   const dim3 per_rank(static_cast<unsigned>(ctx->num_sms), static_cast<unsigned>(R));
-  k_build_holders<<<per_rank, 256, 0, s>>>(c->d_peers, c->hkeys, c->hmask, hmask_cap, c->counters);
+  k_build_holders<<<per_rank, 256, 0, s>>>(c->partial.d_peers, c->hkeys, c->hmask, hmask_cap,
+                                           c->counters, nullptr, nullptr);
   k_list_owned<<<ctx->num_sms * 4, 256, 0, s>>>(c->hkeys, c->hmask, static_cast<uint32_t>(c->hcap),
                                                 c->rank, c->hbase, c->mine, list_cap, c->counters);
-  k_holder_slots<<<per_rank, 256, 0, s>>>(c->d_peers, c->hkeys, c->hmask, c->hbase, hmask_cap,
+  k_holder_slots<<<per_rank, 256, 0, s>>>(c->partial.d_peers, c->hkeys, c->hmask, c->hbase, hmask_cap,
                                           c->rank, c->slots, list_cap);
   mark();
   const size_t smem = 3 * kVoxelsPerBlock * sizeof(uint32_t);
@@ -544,7 +690,7 @@ int32_t cg_gather_global(const cg_layer* partial, cg_layer* owned, uint64_t* blo
     if (ctx->device >= 0 && ctx->device < 64) attr_set[ctx->device] = true;
   }
   k_fold_owned<<<ctx->num_sms * 4, kFoldThreads, smem, s>>>(
-      owned->v, c->d_peers, c->hkeys, c->hmask, c->hbase, c->mine, c->slots, c->counters, list_cap,
+      owned->v, c->partial.d_peers, c->hkeys, c->hmask, c->hbase, c->mine, c->slots, c->counters, list_cap,
       static_cast<int>(owned->num_blocks), &ctx->d_counters->blocks_out);
   k_comm_overflow<<<1, 1, 0, s>>>(c->counters, owned->v.err);
   mark();

@@ -20,6 +20,9 @@
 // scan numbers the triangles, and the vertices land at their final position — the output is
 // byte-identical whatever the launch geometry.  Two passes (count, then write) with a scan over
 // the blocks in between give every block its vertex range in (z, y, x) block order.
+// cg_layer_mesh_sharded runs the same kernel over one rank's owned layer of a sharded global map;
+// only the block lookup differs (ShardedBlocks: the +x/+y/+z neighbours and the colour block may
+// live on a peer rank and are read from its pool over NVLink).
 #include <cub/cub.cuh>
 
 #include <algorithm>
@@ -335,9 +338,21 @@ __device__ __forceinline__ V3 mc_interpolate(V3 v1, V3 v2, float sdf1, float sdf
   return (v1 + v2) * 0.5f;
 }
 
-template <bool kWrite>
+// How the kernel finds a block: find() turns a key into a reference (-1: no such block), planes()
+// a reference into the block's distance plane (weight and colour planes follow, kVoxelsPerBlock
+// words apart).  cg_layer_mesh looks in the layer's own hash: the reference is the pool slot.
+struct LocalBlocks {
+  __device__ __forceinline__ int find(const LayerView& L, uint64_t key) const {
+    return L.find_slot(key);
+  }
+  __device__ __forceinline__ const float* planes(const LayerView& L, int ref) const {
+    return L.dist_plane(ref);
+  }
+};
+
+template <bool kWrite, class Blocks>
 __global__ void __launch_bounds__(kMcThreads)
-k_mesh_blocks(LayerView L, const uint64_t* __restrict__ sorted_keys,
+k_mesh_blocks(LayerView L, Blocks blocks, const uint64_t* __restrict__ sorted_keys,
               const uint32_t* __restrict__ sorted_slots, uint32_t num_blocks, float min_weight,
               int use_color, int only_updated, uint32_t* __restrict__ counts,
               const uint32_t* __restrict__ vertex_begin, float* __restrict__ vertices,
@@ -360,17 +375,18 @@ k_mesh_blocks(LayerView L, const uint64_t* __restrict__ sorted_keys,
     if (threadIdx.x < 8) {
       const int k = threadIdx.x;
       s_nb[k] = k == 0 ? slot
-                       : L.find_slot(pack_block_key(bx + (k & 1), by + ((k >> 1) & 1), bz + (k >> 2)));
+                       : blocks.find(L, pack_block_key(bx + (k & 1), by + ((k >> 1) & 1), bz + (k >> 2)));
     }
     __syncthreads();
     for (int t = threadIdx.x; t < kMcTileVox; t += kMcThreads) {
       const int x = t % kMcTile, y = (t / kMcTile) % kMcTile, z = t / (kMcTile * kMcTile);
       const int nb = s_nb[(x >> 4) | ((y >> 4) << 1) | ((z >> 4) << 2)];
       float d = 0.0f, w = -1.0f;  // a missing neighbour block: the corner is not observed
-      if (nb >= 0) {
+      if (nb != -1) {
         const int lin = (x & 15) + kVps * ((y & 15) + kVps * (z & 15));
-        d = L.dist_plane(nb)[lin];
-        w = L.weight_plane(nb)[lin];
+        const float* p = blocks.planes(L, nb);
+        d = p[lin];
+        w = p[kVoxelsPerBlock + lin];
       }
       s_d[t] = d;
       s_w[t] = w;
@@ -473,7 +489,7 @@ k_mesh_blocks(LayerView L, const uint64_t* __restrict__ sorted_keys,
               // getBlockPtrByCoordinates(vertex)->getVoxelByCoordinates(vertex)
               const int nbx = grid_index(p[k].x, L.block_size_inv), nby = grid_index(p[k].y, L.block_size_inv),
                         nbz = grid_index(p[k].z, L.block_size_inv);
-              cs = L.find_slot(pack_block_key(nbx, nby, nbz));
+              cs = blocks.find(L, pack_block_key(nbx, nby, nbz));
               const V3 no = V3{static_cast<float>(nbx) * L.block_size, static_cast<float>(nby) * L.block_size,
                                static_cast<float>(nbz) * L.block_size};
               const V3 nr = p[k] - no;
@@ -481,9 +497,11 @@ k_mesh_blocks(LayerView L, const uint64_t* __restrict__ sorted_keys,
               cy = max(min(grid_index(nr.y, L.voxel_size_inv), kVps - 1), 0);
               cz = max(min(grid_index(nr.z, L.voxel_size_inv), kVps - 1), 0);
             }
-            if (cs >= 0) {
+            if (cs != -1) {
               const int lin = cx + kVps * (cy + kVps * cz);
-              if (L.weight_plane(cs)[lin] > min_weight) col = L.color_plane(cs)[lin];
+              const float* p = blocks.planes(L, cs);
+              if (p[kVoxelsPerBlock + lin] > min_weight)
+                col = reinterpret_cast<const uint32_t*>(p)[2 * kVoxelsPerBlock + lin];
             }
           }
           colors[out] = col;
@@ -508,9 +526,24 @@ __global__ void k_mesh_unpack_idx(const uint64_t* __restrict__ keys, uint32_t n,
 
 using namespace cg;
 
-// runs both passes; the result stays in the context's buffers (mc_*, stage_b) until the next call
+template <bool kWrite, class Blocks>
+static void launch_mesh(unsigned grid, cudaStream_t s, const cg_layer* L, const Blocks& blocks,
+                        const uint64_t* keys, const uint32_t* slots, uint32_t n, float min_weight,
+                        int32_t use_color, int32_t only_updated, uint32_t* counts,
+                        const uint32_t* begin, float* vertices, float* normals, uint32_t* colors) {
+  k_mesh_blocks<kWrite, Blocks><<<grid, kMcThreads, 0, s>>>(L->v, blocks, keys, slots, n, min_weight,
+                                                            use_color, only_updated, counts, begin,
+                                                            vertices, normals, colors);
+}
+
+// Runs both passes; the result stays in the context's buffers (mc_*, stage_b) until the next call.
+// `sharded` (cg_layer_mesh_sharded): blocks this rank does not hold are looked up across the ranks.
+// The collective opening comes after the local scratch is reserved, and from there every exit
+// passes the closing barrier, so no rank leaves while a peer still waits for it.  The one host
+// synchronisation reads the vertex total and the duplicate-key word together.
 static int32_t mesh_to_device(const cg_layer* L, float min_weight, int32_t use_color,
-                              int32_t only_updated, size_t* n_blocks, size_t* n_vertices) {
+                              int32_t only_updated, bool sharded, size_t* n_blocks,
+                              size_t* n_vertices) {
   cg_context* ctx = L->ctx;
   cudaStream_t s = ctx->stream;
   const size_t n = static_cast<size_t>(L->num_blocks);
@@ -518,45 +551,77 @@ static int32_t mesh_to_device(const cg_layer* L, float min_weight, int32_t use_c
   *n_vertices = 0;
   ctx->mc_blocks = 0;
   ctx->mc_total = 0;
-  if (n == 0) return CG_OK;
-  const uint64_t* keys;
-  const uint32_t* slots;
-  int32_t rc = sort_blocks(L, &keys, &slots);
-  if (rc) return rc;
-  CG_CUDA(ctx->mc_counts.reserve(2 * (n + 1) * sizeof(uint32_t)));
+  if (n == 0 && !sharded) return CG_OK;  // a rank without blocks still takes part in the exchange
+  const uint64_t* keys = nullptr;
+  const uint32_t* slots = nullptr;
+  int32_t rc;
+  if (n > 0 && (rc = sort_blocks(L, &keys, &slots))) return rc;
+  // counts [n + 1] | vertex_begin [n + 1] | duplicate key (sharded: 8-byte aligned, read back with
+  // the total that ends vertex_begin)
+  CG_CUDA(ctx->mc_counts.reserve((2 * (n + 1) + 2) * sizeof(uint32_t)));
   CG_CUDA(ctx->mc_index.reserve(n * 3 * sizeof(int32_t)));
   uint32_t* counts = ctx->mc_counts.as<uint32_t>();
   uint32_t* begin = counts + (n + 1);
+  unsigned long long* dup_key = reinterpret_cast<unsigned long long*>(counts + 2 * (n + 1));
   size_t tmp = 0;
   CG_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, tmp, counts, begin, static_cast<int>(n + 1), s));
   CG_CUDA(ctx->cub_tmp.reserve(tmp));
   const unsigned grid = static_cast<unsigned>(std::min<size_t>(n, static_cast<size_t>(ctx->num_sms) * 16));
-  ctx->own_launches += 2;
-  CG_CUDA(cudaMemsetAsync(counts + n, 0, sizeof(uint32_t), s));
-  k_mesh_blocks<false><<<grid, kMcThreads, 0, s>>>(L->v, keys, slots, static_cast<uint32_t>(n),
-                                                   min_weight, use_color, only_updated, counts,
-                                                   nullptr, nullptr, nullptr, nullptr);
-  k_mesh_unpack_idx<<<grid_for(n, 256), 256, 0, s>>>(keys, static_cast<uint32_t>(n),
-                                                     ctx->mc_index.as<int32_t>());
-  CG_CUDA(cub::DeviceScan::ExclusiveSum(ctx->cub_tmp.p, tmp, counts, begin, static_cast<int>(n + 1), s));
-  uint32_t total = 0;
-  CG_CUDA(cudaMemcpyAsync(&total, begin + n, sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
-  CG_CUDA(cudaStreamSynchronize(s));
-  CG_CUDA(cudaGetLastError());
-  if (total > 0) {
-    CG_CUDA(ctx->mc_vertices.reserve(static_cast<size_t>(total) * 3 * sizeof(float)));
-    CG_CUDA(ctx->mc_normals.reserve(static_cast<size_t>(total) * 3 * sizeof(float)));
-    CG_CUDA(ctx->mc_colors.reserve(static_cast<size_t>(total) * sizeof(uint32_t)));
-    ctx->own_launches += 1;
-    k_mesh_blocks<true><<<grid, kMcThreads, 0, s>>>(
-        L->v, keys, slots, static_cast<uint32_t>(n), min_weight, use_color, only_updated, counts,
-        begin, ctx->mc_vertices.as<float>(), ctx->mc_normals.as<float>(), ctx->mc_colors.as<uint32_t>());
+  ShardedBlocks sb{};
+  if (sharded && (rc = sharded_mesh_open(L, dup_key, &sb))) return rc;
+  const uint32_t nb = static_cast<uint32_t>(n);
+  rc = [&]() -> int32_t {
+    CG_CUDA(cudaMemsetAsync(counts + n, 0, sizeof(uint32_t), s));
+    if (n > 0) {
+      ctx->own_launches += 2;
+      if (sharded)
+        launch_mesh<false>(grid, s, L, sb, keys, slots, nb, min_weight, use_color, only_updated,
+                           counts, nullptr, nullptr, nullptr, nullptr);
+      else
+        launch_mesh<false>(grid, s, L, LocalBlocks{}, keys, slots, nb, min_weight, use_color,
+                           only_updated, counts, nullptr, nullptr, nullptr, nullptr);
+      k_mesh_unpack_idx<<<grid_for(n, 256), 256, 0, s>>>(keys, nb, ctx->mc_index.as<int32_t>());
+    }
+    CG_CUDA(cub::DeviceScan::ExclusiveSum(ctx->cub_tmp.p, tmp, counts, begin, static_cast<int>(n + 1), s));
+    uint32_t back[3] = {0u, 0u, 0u};  // total, duplicate key (low, high word)
+    CG_CUDA(cudaMemcpyAsync(back, begin + n, (sharded ? 3 : 1) * sizeof(uint32_t),
+                            cudaMemcpyDeviceToHost, s));
+    CG_CUDA(cudaStreamSynchronize(s));
     CG_CUDA(cudaGetLastError());
+    const uint32_t total = back[0];
+    const unsigned long long dup = (static_cast<unsigned long long>(back[2]) << 32) | back[1];
+    if (sharded && dup != kEmptyKey) {  // the same key map on every rank: every rank stops here
+      int x, y, z;
+      unpack_block_key(dup, x, y, z);
+      set_error("cg_layer_mesh_sharded: block (%d, %d, %d) is held by more than one rank", x, y, z);
+      return CG_ERR_INVALID_ARG;
+    }
+    if (total > 0) {
+      CG_CUDA(ctx->mc_vertices.reserve(static_cast<size_t>(total) * 3 * sizeof(float)));
+      CG_CUDA(ctx->mc_normals.reserve(static_cast<size_t>(total) * 3 * sizeof(float)));
+      CG_CUDA(ctx->mc_colors.reserve(static_cast<size_t>(total) * sizeof(uint32_t)));
+      ctx->own_launches += 1;
+      float* v = ctx->mc_vertices.as<float>();
+      float* nrm = ctx->mc_normals.as<float>();
+      uint32_t* col = ctx->mc_colors.as<uint32_t>();
+      if (sharded)
+        launch_mesh<true>(grid, s, L, sb, keys, slots, nb, min_weight, use_color, only_updated,
+                          counts, begin, v, nrm, col);
+      else
+        launch_mesh<true>(grid, s, L, LocalBlocks{}, keys, slots, nb, min_weight, use_color,
+                          only_updated, counts, begin, v, nrm, col);
+      CG_CUDA(cudaGetLastError());
+    }
+    ctx->mc_blocks = n;
+    ctx->mc_total = total;
+    *n_vertices = total;
+    return CG_OK;
+  }();
+  if (sharded) {
+    const int32_t rb = sharded_mesh_close(ctx);
+    if (rc == CG_OK) rc = rb;
   }
-  ctx->mc_blocks = n;
-  ctx->mc_total = total;
-  *n_vertices = total;
-  return CG_OK;
+  return rc;
 }
 
 static int32_t mesh_fetch(cg_context* ctx, size_t capacity_blocks, size_t capacity_vertices,
@@ -603,13 +668,34 @@ int32_t cg_layer_mesh(const cg_layer* L, float min_weight, int32_t use_color, in
   if (!L) return CG_ERR_INVALID_ARG;
   CG_CUDA(cudaSetDevice(L->ctx->device));
   size_t nb = 0, nv = 0;
-  int32_t rc = mesh_to_device(L, min_weight, use_color, only_updated, &nb, &nv);
+  int32_t rc = mesh_to_device(L, min_weight, use_color, only_updated, false, &nb, &nv);
   if (num_blocks_out) *num_blocks_out = nb;
   if (num_vertices_out) *num_vertices_out = nv;
   if (rc) return rc;
   if (!block_idx && !vertex_begin && !vertices && !normals && !colors) return CG_OK;
   return mesh_fetch(L->ctx, capacity_blocks, capacity_vertices, block_idx, vertex_begin, vertices,
                     normals, colors);
+}
+
+int32_t cg_layer_mesh_sharded(const cg_layer* owned, float min_weight, int32_t use_color,
+                              int32_t only_updated, size_t capacity_blocks, size_t capacity_vertices,
+                              int32_t* block_idx, uint32_t* vertex_begin, float* vertices,
+                              float* normals, uint8_t* colors, size_t* num_blocks_out,
+                              size_t* num_vertices_out) {
+  if (!owned) return CG_ERR_INVALID_ARG;
+  if (!owned->ctx->comm) {
+    set_error("cg_layer_mesh_sharded: call cg_comm_init first");
+    return CG_ERR_INVALID_ARG;
+  }
+  CG_CUDA(cudaSetDevice(owned->ctx->device));
+  size_t nb = 0, nv = 0;
+  int32_t rc = mesh_to_device(owned, min_weight, use_color, only_updated, true, &nb, &nv);
+  if (num_blocks_out) *num_blocks_out = nb;
+  if (num_vertices_out) *num_vertices_out = nv;
+  if (rc) return rc;
+  if (!block_idx && !vertex_begin && !vertices && !normals && !colors) return CG_OK;
+  return mesh_fetch(owned->ctx, capacity_blocks, capacity_vertices, block_idx, vertex_begin,
+                    vertices, normals, colors);
 }
 
 int32_t cg_mesh_fetch(cg_context* ctx, size_t capacity_blocks, size_t capacity_vertices,

@@ -441,13 +441,15 @@ struct LayerMesh {
   std::vector<Point> vertices, normals;
   std::vector<Color> colors;
 };
-inline void generateMesh(const TsdfLayer& layer, LayerMesh* mesh,
-                         const MeshIntegratorConfig& config = MeshIntegratorConfig(),
-                         bool only_mesh_updated_blocks = false) {
+namespace detail {
+// cg_layer_mesh or cg_layer_mesh_sharded (same arguments), then cg_mesh_fetch
+template <class MeshEntry>
+inline void meshAndFetch(MeshEntry entry, const TsdfLayer& layer, LayerMesh* mesh,
+                         const MeshIntegratorConfig& config, bool only_mesh_updated_blocks) {
   size_t nb = 0, nv = 0;
-  check(cg_layer_mesh(layer.handle(), config.min_weight, config.use_color ? 1 : 0,
-                      only_mesh_updated_blocks ? 1 : 0, 0, 0, nullptr, nullptr, nullptr, nullptr,
-                      nullptr, &nb, &nv));
+  check(entry(layer.handle(), config.min_weight, config.use_color ? 1 : 0,
+              only_mesh_updated_blocks ? 1 : 0, 0, 0, nullptr, nullptr, nullptr, nullptr, nullptr,
+              &nb, &nv));
   mesh->block_indices.resize(nb);
   mesh->vertex_begin.assign(nb + 1, 0);
   mesh->vertices.resize(nv);
@@ -457,6 +459,20 @@ inline void generateMesh(const TsdfLayer& layer, LayerMesh* mesh,
   check(cg_mesh_fetch(layer.context(), nb, nv, &mesh->block_indices[0].x, mesh->vertex_begin.data(),
                       nv ? &mesh->vertices[0].x : nullptr, nv ? &mesh->normals[0].x : nullptr,
                       nv ? &mesh->colors[0].r : nullptr));
+}
+}  // namespace detail
+inline void generateMesh(const TsdfLayer& layer, LayerMesh* mesh,
+                         const MeshIntegratorConfig& config = MeshIntegratorConfig(),
+                         bool only_mesh_updated_blocks = false) {
+  detail::meshAndFetch(cg_layer_mesh, layer, mesh, config, only_mesh_updated_blocks);
+}
+// The same over the sharded global map that getProjectedMapSharded leaves, every rank with its
+// owned layer (collective): each rank gets the meshes of its own blocks, byte for byte what
+// generateMesh gives for them on the gathered map; the halo blocks are read from the peers.
+inline void generateMeshSharded(const TsdfLayer& owned_layer, LayerMesh* mesh,
+                                const MeshIntegratorConfig& config = MeshIntegratorConfig(),
+                                bool only_mesh_updated_blocks = false) {
+  detail::meshAndFetch(cg_layer_mesh_sharded, owned_layer, mesh, config, only_mesh_updated_blocks);
 }
 
 // ---- MeshLayer::getConnectedMesh + io::outputMeshAsPly: what saveAndPubCombinedMesh does with a

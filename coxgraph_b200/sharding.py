@@ -145,3 +145,12 @@ def project_sharded_native(local_submaps, local_poses, partial_layer, owned_laye
     NVLink peer memory, no torch in the data path.  Needs init_native(ctx) once."""
     from .api import getProjectedMapSharded
     getProjectedMapSharded(local_submaps, local_poses, partial_layer, owned_layer)
+
+
+def mesh_sharded(owned_layer, min_weight=1e-4, use_color=True, only_updated=False, fetch=True):
+    """The mesh half of saveAndPubCombinedMesh over all ranks (cg_layer_mesh_sharded), after
+    project_sharded_native: every rank meshes the blocks of its owned layer where they lie, reading
+    the one-block halo from the peers.  Returns Layer.generateMesh's tuple for this rank's blocks;
+    merged by block index, the ranks' results equal generateMesh of the gathered map."""
+    from .api import generateMeshSharded
+    return generateMeshSharded(owned_layer, min_weight, use_color, only_updated, fetch)

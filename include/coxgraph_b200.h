@@ -538,6 +538,34 @@ int32_t cg_project_submaps_sharded(const cg_layer* const* submaps, const float* 
                                    size_t num_submaps, cg_layer* partial_layer,
                                    cg_layer* owned_layer, cg_merge_stats* stats);
 
+/* MeshIntegrator::generateMesh over the sharded global map, where it lies (the mesh half of
+ * saveAndPubCombinedMesh on several GPUs).  Collective: every rank of the context's communicator
+ * passes its owned layer (cg_gather_global's `owned`; all ranks' owned layers have the same voxel
+ * size and max_blocks) and gets the block meshes of the blocks that layer holds, in (z, y, x)
+ * order, with cg_layer_mesh's conventions and arguments; the result stays in the context for
+ * cg_mesh_fetch and the NULL-array count query.  Every block lookup of the mesher — the +x/+y/+z
+ * neighbours a block's border cubes read, and the block of a vertex's colour — is resolved across
+ * the ranks (the peer's block is read over NVLink), so for every block the rank holding it produces
+ * byte for byte what cg_layer_mesh produces for that block on ONE layer holding the union of all
+ * ranks' owned layers (voxels and `updated` flags).  A block no rank holds is missing, as in
+ * cg_layer_mesh.
+ * Errors: no communicator (cg_comm_init) -> CG_ERR_INVALID_ARG; owned layers of different voxel
+ * size or max_blocks, or a block key held by more than one rank (two cg_gather_global calls into
+ * owned layers not cleared in between can leave one) -> CG_ERR_INVALID_ARG on every rank, the
+ * message names the rank or the key.  The call ends with a barrier: a rank may clear or refill its
+ * owned layer as soon as it returns.  The owned layer's buffers are mapped into the peers the first
+ * time it is used and stay mapped until every rank has passed another owned layer or destroyed its
+ * communicator; destroy an owned layer only after that.  cg_mesh_connect stays rank-local (the
+ * first-occurrence order over the global block order would need a gather). */
+int32_t cg_layer_mesh_sharded(const cg_layer* owned_layer, float min_weight, int32_t use_color,
+                              int32_t only_updated, size_t capacity_blocks, size_t capacity_vertices,
+                              int32_t* block_idx_xyz, uint32_t* vertex_begin, float* vertices_xyz,
+                              float* normals_xyz, uint8_t* colors_rgba,
+                              size_t* num_blocks_out, size_t* num_vertices_out);
+/* Peer mappings (cudaIpcOpenMemHandle) of the context's communicator: opened since cg_comm_init,
+ * and open now.  A layer is mapped once per role (partial, owned), not once per call. */
+int32_t cg_comm_peer_mappings(const cg_context* ctx, uint64_t* opened_total, uint64_t* open_now);
+
 /* --- self checks of device arithmetic shortcuts (which: 0 = exact division through a
  * precomputed reciprocal, 1 = round-half-away, 2 = RayCaster state at block entries computed
  * without walking, `samples` random rays); *mismatches must come back 0.  which = 3 runs the same
