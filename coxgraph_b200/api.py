@@ -651,6 +651,27 @@ def getProjectedMapSharded(submap_layers, submap_poses, partial_layer, owned_lay
                                                       partial_layer._h, owned_layer._h, None))
 
 
+def reprojectSubmapsSharded(submap_layers, poses_old, poses_new, partial_layer, owned_layer,
+                            eps_translation=0.0, eps_rotation=0.0):
+    """Collective: reprojectSubmaps over all ranks after getProjectedMapSharded.  This rank's
+    first len(poses_old) submaps are the ones it projected last (with poses_old), the rest are new;
+    poses_new has one pose per submap.  Afterwards partial_layer and owned_layer hold exactly what
+    a fresh getProjectedMapSharded under the effective poses would leave; only the owned blocks
+    whose holders or copies changed are folded again (and flagged updated).  Returns (changed
+    mask, ReprojectShardedStats)."""
+    n = len(submap_layers)
+    Po = np.ascontiguousarray(poses_old, np.float32).reshape(-1, 7)
+    Pn = np.ascontiguousarray(poses_new, np.float32).reshape(n, 7)
+    arr = (C.c_void_p * max(n, 1))(*[l._h for l in submap_layers])
+    changed = np.zeros(max(n, 1), np.uint8)
+    st = capi.ReprojectShardedStats()
+    capi.check(capi.load().cg_reproject_submaps_sharded(
+        arr, n, len(Po), _ptr(Po) if len(Po) else None, _ptr(Pn) if n else None,
+        float(eps_translation), float(eps_rotation), partial_layer._h, owned_layer._h,
+        _ptr(changed), C.byref(st)))
+    return changed[:n].astype(bool), st
+
+
 def generateMeshSharded(owned_layer, min_weight=1e-4, use_color=True, only_updated=False,
                         fetch=True):
     """Collective: generateMesh over the sharded global map, every rank with its owned layer.  Each

@@ -121,6 +121,13 @@ class ReprojectStats(C.Structure):
                 ("blocks_removed", C.c_uint64), ("full_rebuild", C.c_uint64)]
 
 
+class ReprojectShardedStats(C.Structure):
+    _fields_ = [("submaps_moved", C.c_uint64), ("submaps_added", C.c_uint64),
+                ("blocks_dirty_local", C.c_uint64), ("blocks_dirty", C.c_uint64),
+                ("blocks_folded", C.c_uint64), ("blocks_removed", C.c_uint64),
+                ("full_rebuild", C.c_uint64)]
+
+
 class EsdfConfig(C.Structure):
     """cg_esdf_config == voxblox::EsdfIntegrator::Config."""
 
@@ -227,6 +234,9 @@ SYMBOLS = {
     "cg_comm_destroy": (C.c_int32, [_P]),
     "cg_gather_global": (C.c_int32, [_P, _P, C.POINTER(C.c_uint64)]),
     "cg_project_submaps_sharded": (C.c_int32, [_P, _P, C.c_size_t, _P, _P, C.POINTER(MergeStats)]),
+    "cg_reproject_submaps_sharded": (C.c_int32, [_P, C.c_size_t, C.c_size_t, _P, _P, C.c_float,
+                                                 C.c_float, _P, _P, _P,
+                                                 C.POINTER(ReprojectShardedStats)]),
     "cg_layer_mesh_sharded": (C.c_int32, [_P, C.c_float, C.c_int32, C.c_int32, C.c_size_t, C.c_size_t,
                                           _P, _P, _P, _P, _P, C.POINTER(C.c_size_t),
                                           C.POINTER(C.c_size_t)]),

@@ -398,6 +398,27 @@ int32_t remove_flagged_blocks(cg_layer* layer, const uint8_t* d_remove, uint64_t
 int32_t sharded_mesh_open(const cg_layer* owned, unsigned long long* dup_key, ShardedBlocks* out);
 int32_t sharded_mesh_close(cg_context* ctx);
 
+// merge.cu: the re-projection shared by cg_reproject_submaps and cg_reproject_submaps_sharded
+// (the latter also asks for the keys of the dirty blocks the layer holds before and after it,
+// appended at *count, at most `cap` stored), and the block reset / removal steps of both.
+struct DirtyKeysOut {
+  uint64_t* keys;
+  uint32_t* count;  // device cursor
+  uint32_t cap;
+};
+double full_rebuild_fraction();
+int32_t reproject_local(const cg_layer* const* submaps, size_t n, size_t num_known,
+                        const float* poses_old, const float* poses_new, float eps_translation,
+                        float eps_rotation, cg_layer* G, uint8_t* changed_out,
+                        cg_reproject_stats* stats, const DirtyKeysOut* dirty, const char* who);
+// lists the blocks of G whose keys are in the hash set `dirty_keys` (cap entries; slots in
+// slots[0, counts[0])) and resets them to the default state with has_data = 0
+int32_t reset_dirty_blocks(cg_layer* G, const uint64_t* dirty_keys, uint32_t cap, uint32_t* slots,
+                           uint32_t* counts);
+// removes the listed blocks (`listed` = counts[0] of them) that hold no data, then finish_call
+int32_t remove_dead_blocks(cg_layer* G, const uint32_t* slots, const uint32_t* counts,
+                           uint32_t listed, uint64_t* removed);
+
 #define CG_CUDA(expr)                                         \
   do {                                                        \
     cudaError_t _e = (expr);                                  \

@@ -91,13 +91,14 @@ struct PeerLayer {
   const float* pool;
   const uint64_t* block_keys;
   const uint8_t* has_data;
-  const uint32_t* shared;  // [0] number of blocks of the layer (written per call)
+  const uint32_t* shared;  // [0] number of blocks of the layer (written per call), see Binding
+  const uint64_t* dirty_keys;  // partial role: the keys cg_reproject_submaps_sharded publishes
 };
 constexpr int kMaxRanks = 64;
 
 struct IpcRecord {  // one per rank, all-gathered
-  cudaIpcMemHandle_t pool, keys, flags, shared;
-  unsigned long long off_pool, off_keys, off_flags, off_shared;  // pointer - allocation base
+  cudaIpcMemHandle_t pool, keys, flags, shared, dirty;
+  unsigned long long off_pool, off_keys, off_flags, off_shared, off_dirty;  // pointer - allocation base
   unsigned long long max_blocks;
   float voxel_size;
   int pad;
@@ -110,7 +111,12 @@ struct IpcRecord {  // one per rank, all-gathered
 // role.
 struct Binding {
   uint64_t serial = 0;            // cg_layer::serial of the bound layer (0: none)
-  uint32_t* shared = nullptr;     // peer-visible: [0] blocks of this rank's layer (written per call)
+  // peer-visible words, written per call: [0] blocks of this rank's layer; the partial role's
+  // cg_reproject_submaps_sharded also publishes [1] blocks of the owned layer, [2] dirty keys and
+  // [3] the full-rebuild fraction (float bits; rank 0's is the one every rank uses)
+  uint32_t* shared = nullptr;
+  uint64_t* dirty = nullptr;      // partial role: peer-visible dirty keys (2 x max_blocks)
+  uint32_t dirty_cap = 0;
   PeerLayer* d_peers = nullptr;   // [nranks]
   std::vector<char*> held;        // peer mappings this binding uses (one reference each)
 };
@@ -134,6 +140,10 @@ struct cg_comm {
   // the holder map (scratch, rebuilt every call): block key -> set of ranks holding the block
   unsigned long long* hkeys = nullptr;
   unsigned long long* hmask = nullptr;
+  // cg_reproject_submaps_sharded: the union D of every rank's dirty keys (scratch, lazily sized)
+  cg::DevBuf dset;
+  size_t dcap = 0;
+  uint32_t* dcounters = nullptr;      // [0] |D|, [1] owned blocks of all ranks, [2] overflow, [3] fraction
   uint32_t* hbase = nullptr;          // owned entries: first element of the block's slot list
   uint32_t* mine = nullptr;           // entries this rank owns
   uint32_t* slots = nullptr;          // pool slots of the holders' copies, per owned block
@@ -167,15 +177,28 @@ __device__ __forceinline__ int pick_owner(unsigned long long key, unsigned long 
 // Every block key of every rank's layer (read through the peer mappings) enters the map with its
 // rank's bit.  Grid y = rank.  With `planes` (the key map of cg_layer_mesh_sharded) the entry also
 // records where the block's planes are, and a key that reaches an entry another rank has already
-// marked is held twice: the smallest such key goes to *dup_key.
+// marked is held twice: the smallest such key goes to *dup_key.  With `filter` (a key set of
+// filter_mask + 1 entries, cg_reproject_submaps_sharded) only the keys in it enter the map.
+__device__ __forceinline__ bool in_key_set(const unsigned long long* __restrict__ keys, uint32_t mask,
+                                           unsigned long long key) {
+  uint32_t h = hash_key(key) & mask;
+  for (;;) {
+    const unsigned long long k = keys[h];
+    if (k == key) return true;
+    if (k == kEmptyKey) return false;
+    h = (h + 1) & mask;
+  }
+}
 __global__ void k_build_holders(const PeerLayer* __restrict__ peers, unsigned long long* hkeys,
                                 unsigned long long* hmask, uint32_t hcap_mask, uint32_t* counters,
-                                const float** planes, unsigned long long* dup_key) {
+                                const float** planes, unsigned long long* dup_key,
+                                const unsigned long long* __restrict__ filter, uint32_t filter_mask) {
   const int r = blockIdx.y;
   const PeerLayer P = peers[r];
   const uint32_t n = P.shared[0];
   for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
     const unsigned long long key = P.block_keys[i];
+    if (filter && !in_key_set(filter, filter_mask, key)) continue;
     uint32_t h = hash_key(key) & hcap_mask;
     for (uint32_t tries = 0;; ++tries) {
       const unsigned long long k = hkeys[h];
@@ -220,12 +243,14 @@ __global__ void k_holder_slots(const PeerLayer* __restrict__ peers,
                                const unsigned long long* __restrict__ hkeys,
                                const unsigned long long* __restrict__ hmask,
                                const uint32_t* __restrict__ hbase, uint32_t hcap_mask, int me,
-                               uint32_t* __restrict__ slots, uint32_t slots_cap) {
+                               uint32_t* __restrict__ slots, uint32_t slots_cap,
+                               const unsigned long long* __restrict__ filter, uint32_t filter_mask) {
   const int r = blockIdx.y;
   const PeerLayer P = peers[r];
   const uint32_t n = P.shared[0];
   for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
     const unsigned long long key = P.block_keys[i];
+    if (filter && !in_key_set(filter, filter_mask, key)) continue;
     const uint32_t e = holder_find(hkeys, hcap_mask, key);
     const unsigned long long mask = hmask[e];
     if (pick_owner(key, mask) != me) continue;
@@ -336,6 +361,44 @@ __global__ void k_publish_blocks(uint32_t* shared, int n) { shared[0] = static_c
 __global__ void k_comm_overflow(const uint32_t* counters, int32_t* err) {
   if (counters[2]) atomicOr(err, kErrPoolFull);
 }
+// cg_reproject_submaps_sharded: every rank's published dirty keys (read through the peer mappings)
+// enter the set D; counters [0] |D|, [1] owned blocks of all ranks, [2] a rank published more keys
+// than its buffer holds, [3] rank 0's full-rebuild fraction.  Grid y = rank.
+__global__ void k_union_dirty(const PeerLayer* __restrict__ peers, uint32_t dirty_cap,
+                              unsigned long long* set, uint32_t set_mask, uint32_t* counters) {
+  const int r = blockIdx.y;
+  const PeerLayer P = peers[r];
+  const uint32_t published = P.shared[2];
+  if (blockIdx.x == 0 && threadIdx.x == 0) {
+    atomicAdd(&counters[1], P.shared[1]);
+    if (published > dirty_cap) atomicExch(&counters[2], 1u);
+    if (r == 0) counters[3] = P.shared[3];
+  }
+  const uint32_t n = min(published, dirty_cap);
+  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+    const unsigned long long key = P.dirty_keys[i];
+    uint32_t h = hash_key(key) & set_mask;
+    for (;;) {
+      const unsigned long long k = set[h];
+      if (k == key) break;
+      if (k == kEmptyKey) {
+        const unsigned long long old = atomicCAS(&set[h], kEmptyKey, key);
+        if (old == kEmptyKey) {
+          atomicAdd(&counters[0], 1u);
+          break;
+        }
+        if (old == key) break;
+      }
+      h = (h + 1) & set_mask;
+    }
+  }
+}
+__global__ void k_publish_words(uint32_t* shared, uint32_t partial_blocks, uint32_t owned_blocks,
+                                uint32_t fraction_bits) {
+  shared[0] = partial_blocks;
+  shared[1] = owned_blocks;
+  shared[3] = fraction_bits;
+}
 
 // pointer -> (allocation base handle, offset): cudaMalloc may place small buffers inside a larger
 // allocation, and an IPC handle always names the whole allocation
@@ -382,10 +445,17 @@ static void unbind(cg_comm* c) {
   for (Binding* b : {&c->partial, &c->owned}) {
     release(c, *b);
     if (b->shared) cudaFree(b->shared);
+    if (b->dirty) cudaFree(b->dirty);
     if (b->d_peers) cudaFree(b->d_peers);
     b->shared = nullptr;
+    b->dirty = nullptr;
+    b->dirty_cap = 0;
     b->d_peers = nullptr;
   }
+  c->dset.release();
+  c->dcap = 0;
+  if (c->dcounters) cudaFree(c->dcounters);
+  c->dcounters = nullptr;
   void* bufs[] = {c->hkeys, c->hmask, c->hbase, c->mine, c->slots, c->counters,
                   c->mkeys, c->mmask, c->mplanes, c->mcounters};
   for (void* p : bufs)
@@ -427,6 +497,7 @@ static int32_t bind(cg_context* ctx, const cg_layer* layer, Binding& b, const ch
   if ((rc = ipc_of(layer->v.block_keys, &mine.keys, &mine.off_keys))) return rc;
   if ((rc = ipc_of(layer->v.has_data, &mine.flags, &mine.off_flags))) return rc;
   if ((rc = ipc_of(b.shared, &mine.shared, &mine.off_shared))) return rc;
+  if (b.dirty && (rc = ipc_of(b.dirty, &mine.dirty, &mine.off_dirty))) return rc;
   mine.max_blocks = layer->max_blocks;
   mine.voxel_size = layer->v.voxel_size;
   void* d_all = nullptr;
@@ -450,14 +521,15 @@ static int32_t bind(cg_context* ctx, const cg_layer* layer, Binding& b, const ch
   std::vector<PeerLayer> peers(R);
   for (int r = 0; r < R; ++r) {
     if (r == c->rank) {
-      peers[r] = PeerLayer{layer->v.pool, layer->v.block_keys, layer->v.has_data, b.shared};
+      peers[r] = PeerLayer{layer->v.pool, layer->v.block_keys, layer->v.has_data, b.shared, b.dirty};
       continue;
     }
-    const cudaIpcMemHandle_t* hs[4] = {&all[r].pool, &all[r].keys, &all[r].flags, &all[r].shared};
-    const unsigned long long offs[4] = {all[r].off_pool, all[r].off_keys, all[r].off_flags,
-                                        all[r].off_shared};
-    char* mapped[4] = {nullptr, nullptr, nullptr, nullptr};
-    for (int k = 0; k < 4; ++k) {
+    const cudaIpcMemHandle_t* hs[5] = {&all[r].pool, &all[r].keys, &all[r].flags, &all[r].shared,
+                                       &all[r].dirty};
+    const unsigned long long offs[5] = {all[r].off_pool, all[r].off_keys, all[r].off_flags,
+                                        all[r].off_shared, all[r].off_dirty};
+    char* mapped[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
+    for (int k = 0; k < (b.dirty ? 5 : 4); ++k) {
       for (Mapping& m : c->maps) {
         if (m.rank == r && memcmp(&m.handle, hs[k], sizeof(cudaIpcMemHandle_t)) == 0) {
           ++m.refs;
@@ -481,7 +553,8 @@ static int32_t bind(cg_context* ctx, const cg_layer* layer, Binding& b, const ch
     peers[r] = PeerLayer{reinterpret_cast<const float*>(mapped[0] + offs[0]),
                          reinterpret_cast<const uint64_t*>(mapped[1] + offs[1]),
                          reinterpret_cast<const uint8_t*>(mapped[2] + offs[2]),
-                         reinterpret_cast<const uint32_t*>(mapped[3] + offs[3])};
+                         reinterpret_cast<const uint32_t*>(mapped[3] + offs[3]),
+                         b.dirty ? reinterpret_cast<const uint64_t*>(mapped[4] + offs[4]) : nullptr};
   }
   CG_CUDA(cudaMemcpyAsync(b.d_peers, peers.data(), sizeof(PeerLayer) * R, cudaMemcpyHostToDevice, s));
   CG_CUDA(cudaStreamSynchronize(s));
@@ -509,6 +582,16 @@ static int32_t bind_partial(cg_context* ctx, const cg_layer* partial) {
     CG_CUDA(cudaMalloc(&c->counters, 4 * sizeof(uint32_t)));
     c->hcap = hcap;
     c->list_cap = list_cap;
+  }
+  // the dirty keys of cg_reproject_submaps_sharded: the partial layer's blocks before and after a
+  // call, so at most twice its pool
+  const uint32_t dirty_cap = static_cast<uint32_t>(std::min<size_t>(2 * partial->max_blocks, 0xFFFFFFF0u));
+  if (dirty_cap != c->partial.dirty_cap) {
+    if (c->partial.dirty) cudaFree(c->partial.dirty);
+    c->partial.dirty = nullptr;
+    c->partial.dirty_cap = 0;
+    CG_CUDA(cudaMalloc(&c->partial.dirty, dirty_cap * sizeof(uint64_t)));
+    c->partial.dirty_cap = dirty_cap;
   }
   return bind(ctx, partial, c->partial, "cg_gather_global");
 }
@@ -551,13 +634,62 @@ int32_t sharded_mesh_open(const cg_layer* owned, unsigned long long* dup_key, Sh
   const uint32_t cap_mask = static_cast<uint32_t>(c->mcap - 1);
   const dim3 per_rank(static_cast<unsigned>(ctx->num_sms), static_cast<unsigned>(c->nranks));
   k_build_holders<<<per_rank, 256, 0, s>>>(c->owned.d_peers, c->mkeys, c->mmask, cap_mask,
-                                           c->mcounters, c->mplanes, dup_key);
+                                           c->mcounters, c->mplanes, dup_key, nullptr, 0);
   CG_CUDA(cudaGetLastError());
   *out = ShardedBlocks{c->mkeys, c->mplanes, cap_mask};
   return CG_OK;
 }
 
 int32_t sharded_mesh_close(cg_context* ctx) { return barrier(ctx); }
+
+// The holder map of the fold, cleared (before the opening barrier) and built over every rank's
+// partial layer; with `filter` (cg_reproject_submaps_sharded) over the blocks whose keys are in it.
+static int32_t reset_holders(cg_context* ctx) {
+  cg_comm* c = ctx->comm;
+  cudaStream_t s = ctx->stream;
+  CG_CUDA(cudaMemsetAsync(c->hkeys, 0xFF, c->hcap * sizeof(unsigned long long), s));
+  CG_CUDA(cudaMemsetAsync(c->hmask, 0, c->hcap * sizeof(unsigned long long), s));
+  CG_CUDA(cudaMemsetAsync(c->counters, 0, 4 * sizeof(uint32_t), s));
+  CG_CUDA(cudaMemsetAsync(&ctx->d_counters->blocks_out, 0, sizeof(unsigned long long), s));
+  return CG_OK;
+}
+static uint32_t fold_list_cap(const cg_comm* c) {
+  return static_cast<uint32_t>(std::min<size_t>(c->list_cap, 0xFFFFFFF0u));
+}
+static void list_holders(cg_context* ctx, const unsigned long long* filter, uint32_t filter_mask) {
+  cg_comm* c = ctx->comm;
+  cudaStream_t s = ctx->stream;
+  const uint32_t hmask_cap = static_cast<uint32_t>(c->hcap - 1);
+  const uint32_t list_cap = fold_list_cap(c);
+  ctx->own_launches += 3;
+  const dim3 per_rank(static_cast<unsigned>(ctx->num_sms), static_cast<unsigned>(c->nranks));
+  k_build_holders<<<per_rank, 256, 0, s>>>(c->partial.d_peers, c->hkeys, c->hmask, hmask_cap,
+                                           c->counters, nullptr, nullptr, filter, filter_mask);
+  k_list_owned<<<ctx->num_sms * 4, 256, 0, s>>>(c->hkeys, c->hmask, static_cast<uint32_t>(c->hcap),
+                                                c->rank, c->hbase, c->mine, list_cap, c->counters);
+  k_holder_slots<<<per_rank, 256, 0, s>>>(c->partial.d_peers, c->hkeys, c->hmask, c->hbase, hmask_cap,
+                                          c->rank, c->slots, list_cap, filter, filter_mask);
+}
+// every block the holder map gives this rank, folded into `owned` (blocks the layer holds are
+// read as they are: fresh, or reset by cg_reproject_submaps_sharded)
+static int32_t fold_owned(cg_context* ctx, cg_layer* owned) {
+  cg_comm* c = ctx->comm;
+  cudaStream_t s = ctx->stream;
+  const size_t smem = 3 * kVoxelsPerBlock * sizeof(uint32_t);
+  static bool attr_set[64] = {};
+  if (ctx->device < 0 || ctx->device >= 64 || !attr_set[ctx->device]) {
+    CG_CUDA(cudaFuncSetAttribute(k_fold_owned, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                 static_cast<int>(smem)));
+    if (ctx->device >= 0 && ctx->device < 64) attr_set[ctx->device] = true;
+  }
+  ctx->own_launches += 2;
+  k_fold_owned<<<ctx->num_sms * 4, kFoldThreads, smem, s>>>(
+      owned->v, c->partial.d_peers, c->hkeys, c->hmask, c->hbase, c->mine, c->slots, c->counters,
+      fold_list_cap(c), static_cast<int>(owned->num_blocks), &ctx->d_counters->blocks_out);
+  k_comm_overflow<<<1, 1, 0, s>>>(c->counters, owned->v.err);
+  CG_CUDA(cudaGetLastError());
+  return CG_OK;
+}
 
 }  // namespace cg
 
@@ -662,37 +794,15 @@ int32_t cg_gather_global(const cg_layer* partial, cg_layer* owned, uint64_t* blo
     }
   };
   mark();
-  const int R = c->nranks;
-  const uint32_t hmask_cap = static_cast<uint32_t>(c->hcap - 1);
-  const uint32_t list_cap = static_cast<uint32_t>(std::min<size_t>(c->list_cap, 0xFFFFFFF0u));
-  ctx->own_launches += 6;
+  ctx->own_launches += 1;
   k_publish_blocks<<<1, 1, 0, s>>>(c->partial.shared, static_cast<int>(partial->num_blocks));
-  CG_CUDA(cudaMemsetAsync(c->hkeys, 0xFF, c->hcap * sizeof(unsigned long long), s));
-  CG_CUDA(cudaMemsetAsync(c->hmask, 0, c->hcap * sizeof(unsigned long long), s));
-  CG_CUDA(cudaMemsetAsync(c->counters, 0, 4 * sizeof(uint32_t), s));
-  CG_CUDA(cudaMemsetAsync(&ctx->d_counters->blocks_out, 0, sizeof(unsigned long long), s));
+  if ((rc = reset_holders(ctx))) return rc;
   // every rank's partial layer is complete and its block count published (stream-ordered)
   if ((rc = barrier(ctx))) return rc;
   mark();
-  const dim3 per_rank(static_cast<unsigned>(ctx->num_sms), static_cast<unsigned>(R));
-  k_build_holders<<<per_rank, 256, 0, s>>>(c->partial.d_peers, c->hkeys, c->hmask, hmask_cap,
-                                           c->counters, nullptr, nullptr);
-  k_list_owned<<<ctx->num_sms * 4, 256, 0, s>>>(c->hkeys, c->hmask, static_cast<uint32_t>(c->hcap),
-                                                c->rank, c->hbase, c->mine, list_cap, c->counters);
-  k_holder_slots<<<per_rank, 256, 0, s>>>(c->partial.d_peers, c->hkeys, c->hmask, c->hbase, hmask_cap,
-                                          c->rank, c->slots, list_cap);
+  list_holders(ctx, nullptr, 0);
   mark();
-  const size_t smem = 3 * kVoxelsPerBlock * sizeof(uint32_t);
-  static bool attr_set[64] = {};
-  if (ctx->device < 0 || ctx->device >= 64 || !attr_set[ctx->device]) {
-    CG_CUDA(cudaFuncSetAttribute(k_fold_owned, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                 static_cast<int>(smem)));
-    if (ctx->device >= 0 && ctx->device < 64) attr_set[ctx->device] = true;
-  }
-  k_fold_owned<<<ctx->num_sms * 4, kFoldThreads, smem, s>>>(
-      owned->v, c->partial.d_peers, c->hkeys, c->hmask, c->hbase, c->mine, c->slots, c->counters, list_cap,
-      static_cast<int>(owned->num_blocks), &ctx->d_counters->blocks_out);
-  k_comm_overflow<<<1, 1, 0, s>>>(c->counters, owned->v.err);
+  if ((rc = fold_owned(ctx, owned))) return rc;
   mark();
   // nobody clears or refills its partial layer while a peer still reads it
   if ((rc = barrier(ctx))) return rc;
@@ -724,6 +834,177 @@ int32_t cg_project_submaps_sharded(const cg_layer* const* submaps, const float* 
     memset(stats, 0, sizeof(*stats));
   }
   return cg_gather_global(partial, owned, nullptr);
+}
+
+// ---- cg_reproject_submaps_sharded (DESIGN.md §5): the local re-projection of every rank's
+// partial layer, then a fold of only the blocks whose holders or copies may have changed.
+// The opening barrier carries a status word: one 8-bit count per failure kind, summed over the
+// ranks, so that every rank knows whether (and how) some rank's local step failed.
+static uint32_t status_bits(int32_t rc) {
+  if (rc == CG_OK) return 0;
+  const int field = rc == CG_ERR_INVALID_ARG ? 0 : rc == CG_ERR_OUT_OF_RANGE ? 1 : rc == CG_ERR_POOL_FULL ? 2 : 3;
+  return 1u << (8 * field);
+}
+static int32_t status_of(uint32_t word) {  // the most severe failure a rank reported
+  const int32_t kinds[4] = {CG_ERR_INVALID_ARG, CG_ERR_OUT_OF_RANGE, CG_ERR_POOL_FULL, CG_ERR_CUDA};
+  for (int f = 3; f >= 0; --f)
+    if ((word >> (8 * f)) & 0xFFu) return kinds[f];
+  return CG_OK;
+}
+
+int32_t cg_reproject_submaps_sharded(const cg_layer* const* submaps, size_t n, size_t num_known,
+                                     const float* poses_old, const float* poses_new,
+                                     float eps_translation, float eps_rotation, cg_layer* partial,
+                                     cg_layer* owned, uint8_t* changed_out,
+                                     cg_reproject_sharded_stats* stats) {
+  static const char* who = "cg_reproject_submaps_sharded";
+  if (stats) memset(stats, 0, sizeof(*stats));
+  if (!partial || !owned || partial->ctx != owned->ctx || partial == owned) {
+    set_error("%s: partial and owned must be two layers of one context", who);
+    return CG_ERR_INVALID_ARG;
+  }
+  cg_context* ctx = owned->ctx;
+  cg_comm* c = ctx->comm;
+  if (!c) {
+    set_error("%s: call cg_comm_init first", who);
+    return CG_ERR_INVALID_ARG;
+  }
+  CG_CUDA(cudaSetDevice(ctx->device));
+  cudaStream_t s = ctx->stream;
+  // This rank's arguments.  A rejected call still joins the opening barrier, so every rank returns
+  // an error and no rank touches its owned layer.
+  int32_t local = CG_ERR_INVALID_ARG;
+  if (num_known > n) {
+    set_error("%s: num_known (%zu) > num_submaps (%zu)", who, num_known, n);
+  } else if (n && (!submaps || !poses_new || (num_known && !poses_old))) {
+    set_error("%s: null submap or pose array", who);
+  } else if (c->partial.serial == 0 || c->partial.serial != partial->serial) {
+    set_error("%s: `partial` is not the partial layer of the last cg_gather_global on this context",
+              who);
+  } else if (partial->v.voxel_size != owned->v.voxel_size) {
+    set_error("%s: the layers' voxel sizes differ", who);
+  } else {
+    local = CG_OK;
+    for (size_t i = 0; i < n && local == CG_OK; ++i) {
+      if (submaps[i] == owned) {
+        set_error("%s: submap %zu is the owned layer", who, i);
+        local = CG_ERR_INVALID_ARG;
+      }
+    }
+  }
+  cg_reproject_stats rs{};
+  const int64_t owned_before = owned->num_blocks;
+  if (local == CG_OK) {
+    const DirtyKeysOut dk{c->partial.dirty, c->partial.shared + 2, c->partial.dirty_cap};
+    local = cudaMemsetAsync(c->partial.shared + 2, 0, sizeof(uint32_t), s) == cudaSuccess
+                ? CG_OK : cuda_fail(cudaGetLastError(), "cudaMemsetAsync");
+    if (local == CG_OK)
+      local = reproject_local(submaps, n, num_known, poses_old, poses_new, eps_translation,
+                              eps_rotation, partial, changed_out, &rs, &dk, who);
+  }
+  if (local == CG_OK) {
+    const float fraction = static_cast<float>(full_rebuild_fraction());
+    uint32_t fbits;
+    memcpy(&fbits, &fraction, sizeof(fbits));
+    ctx->own_launches += 1;
+    k_publish_words<<<1, 1, 0, s>>>(c->partial.shared, static_cast<uint32_t>(partial->num_blocks),
+                                    static_cast<uint32_t>(owned->num_blocks), fbits);
+  }
+  uint32_t word = status_bits(local);
+  CG_CUDA(cudaMemcpyAsync(c->d_token, &word, sizeof(word), cudaMemcpyHostToDevice, s));
+  int32_t rc;
+  // every rank's partial layer, dirty keys and counts are complete (stream-ordered)
+  if ((rc = barrier(ctx))) return rc;
+  CG_CUDA(cudaMemcpyAsync(&word, c->d_token, sizeof(word), cudaMemcpyDeviceToHost, s));
+  CG_CUDA(cudaMemsetAsync(c->d_token, 0, sizeof(int), s));
+  CG_CUDA(cudaStreamSynchronize(s));
+  if (local) return local;
+  if (word) {
+    set_error("%s: another rank's local step failed (status %d); no owned layer was changed", who,
+              status_of(word));
+    return status_of(word);
+  }
+  // D: the union of every rank's published keys, identical on every rank
+  const int R = c->nranks;
+  const size_t dcap = map_capacity(2 * partial->max_blocks, R);
+  uint32_t h[4] = {0, 0, 0, 0};
+  rc = [&]() -> int32_t {
+    CG_CUDA(c->dset.reserve(dcap * sizeof(unsigned long long)));
+    c->dcap = dcap;
+    if (!c->dcounters) CG_CUDA(cudaMalloc(&c->dcounters, 4 * sizeof(uint32_t)));
+    CG_CUDA(cudaMemsetAsync(c->dset.p, 0xFF, dcap * sizeof(unsigned long long), s));
+    CG_CUDA(cudaMemsetAsync(c->dcounters, 0, 4 * sizeof(uint32_t), s));
+    ctx->own_launches += 1;
+    k_union_dirty<<<dim3(static_cast<unsigned>(ctx->num_sms), static_cast<unsigned>(R)), 256, 0, s>>>(
+        c->partial.d_peers, c->partial.dirty_cap, c->dset.as<unsigned long long>(),
+        static_cast<uint32_t>(dcap - 1), c->dcounters);
+    CG_CUDA(cudaMemcpyAsync(h, c->dcounters, sizeof(h), cudaMemcpyDeviceToHost, s));
+    CG_CUDA(cudaStreamSynchronize(s));
+    return CG_OK;
+  }();
+  if (rc) {
+    barrier(ctx);
+    return rc;
+  }
+  float fraction;
+  memcpy(&fraction, &h[3], sizeof(fraction));
+  const bool full = static_cast<double>(h[0]) > static_cast<double>(fraction) * static_cast<double>(h[1]);
+  if (stats) {
+    stats->submaps_moved = rs.submaps_moved;
+    stats->submaps_added = n - num_known;
+    stats->blocks_dirty_local = rs.blocks_dirty;
+    stats->blocks_dirty = h[0];
+    stats->full_rebuild = full ? 1 : 0;
+  }
+  if (h[2]) {  // cannot happen: a partial layer holds at most max_blocks blocks before and after
+    barrier(ctx);
+    set_error("%s: a rank published more dirty keys than its buffer holds", who);
+    return CG_ERR_CUDA;
+  }
+  if (full) {
+    // the whole gather, into the cleared owned layer (it opens and closes with its own barriers)
+    rc = cg_layer_clear(owned);
+    if (rc) {
+      barrier(ctx);
+      return rc;
+    }
+    rc = cg_gather_global(partial, owned, nullptr);
+    if (stats) stats->blocks_folded = static_cast<uint64_t>(owned->num_blocks);
+    return rc;
+  }
+  // The blocks of D this owned layer holds are reset, the blocks of D it owns now are folded (a
+  // held block as it was reset, a new one fresh), and held blocks that were not folded again —
+  // owned elsewhere now, or without data — are removed.
+  CG_CUDA(ctx->stage_b.reserve((static_cast<size_t>(owned->num_blocks) + 2) * sizeof(uint32_t)));
+  uint32_t* counts = ctx->stage_b.as<uint32_t>();  // [0] blocks of D the owned layer holds
+  uint32_t* slots = counts + 2;
+  const unsigned long long* dset = c->dset.as<unsigned long long>();
+  rc = [&]() -> int32_t {
+    if (h[0] == 0) return CG_OK;
+    int32_t r = reset_dirty_blocks(owned, reinterpret_cast<const uint64_t*>(dset),
+                                   static_cast<uint32_t>(dcap), slots, counts);
+    if (r) return r;
+    if ((r = reset_holders(ctx))) return r;
+    list_holders(ctx, dset, static_cast<uint32_t>(dcap - 1));
+    return fold_owned(ctx, owned);
+  }();
+  // nobody clears or refills its partial layer while a peer still reads it
+  const int32_t rb = barrier(ctx);
+  if (rc) return rc;
+  if (rb) return rb;
+  uint64_t removed = 0;
+  uint32_t listed = 0;
+  if (h[0] > 0) {
+    CG_CUDA(cudaMemcpyAsync(&listed, counts, sizeof(listed), cudaMemcpyDeviceToHost, s));
+    if ((rc = finish_call(owned, nullptr))) return rc;
+    if (listed > 0 && (rc = remove_dead_blocks(owned, slots, counts, listed, &removed))) return rc;
+  }
+  if (stats) {
+    // blocks outside D are untouched: the owned blocks of D now are the ones folded
+    stats->blocks_folded = static_cast<uint64_t>(owned->num_blocks - (owned_before - listed));
+    stats->blocks_removed = removed;
+  }
+  return CG_OK;
 }
 
 }  // extern "C"

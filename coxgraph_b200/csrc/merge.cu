@@ -716,15 +716,24 @@ static int32_t project_batch(const cg_layer* const* submaps, const BatchSubmap* 
 // and folded into them in submap order, and those left without data are removed.  Every other
 // block holds exactly what a full rebuild would produce, so the result is bit-identical to
 // clearing the layer and projecting all submaps again.
+// Lists the slots of the dirty blocks G holds (counts[0] of them; counts[1]: dirty keys).  With
+// `out_keys` (cg_reproject_submaps_sharded) the keys of those blocks are also appended there
+// (cursor *out_count, at most out_cap stored); `slots` / `counts` may then be null.
 __global__ void k_dirty_slots(LayerView G, const uint64_t* __restrict__ dirty_keys, uint32_t cap,
-                              uint32_t* __restrict__ slots, uint32_t* __restrict__ counts) {
+                              uint32_t* __restrict__ slots, uint32_t* __restrict__ counts,
+                              uint64_t* __restrict__ out_keys, uint32_t* out_count, uint32_t out_cap) {
   const uint32_t h = blockIdx.x * blockDim.x + threadIdx.x;
   if (h >= cap) return;
   const uint64_t key = dirty_keys[h];
   if (key == kEmptyKey) return;
-  atomicAdd(&counts[1], 1u);  // dirty destination blocks
+  if (counts) atomicAdd(&counts[1], 1u);  // dirty destination blocks
   const int slot = G.find_slot(key);
-  if (slot >= 0) slots[atomicAdd(&counts[0], 1u)] = static_cast<uint32_t>(slot);
+  if (slot < 0) return;
+  if (slots) slots[atomicAdd(&counts[0], 1u)] = static_cast<uint32_t>(slot);
+  if (out_keys) {
+    const uint32_t at = atomicAdd(out_count, 1u);
+    if (at < out_cap) out_keys[at] = key;
+  }
 }
 __global__ void __launch_bounds__(256)
 k_reset_blocks(LayerView G, const uint32_t* __restrict__ slots, const uint32_t* __restrict__ counts) {
@@ -791,6 +800,225 @@ static bool pose_changed(const float* a, const float* b, float eps_t, float eps_
                               double(b[3]) * b[3]);
   if (na > 0 && nb > 0) dot /= na * nb;
   return 2.0 * std::acos(std::min(1.0, dot)) > eps_rot;
+}
+
+// dirty blocks / blocks of the map above which the re-projections rebuild the whole map
+// (CG_REPROJECT_FULL_FRACTION overrides it; the tests use 2 to force the block-by-block path)
+double full_rebuild_fraction() {
+  const char* e = getenv("CG_REPROJECT_FULL_FRACTION");
+  return (e && *e) ? atof(e) : 0.3;
+}
+
+int32_t reset_dirty_blocks(cg_layer* G, const uint64_t* dirty_keys, uint32_t cap, uint32_t* slots,
+                           uint32_t* counts) {
+  cg_context* ctx = G->ctx;
+  cudaStream_t s = ctx->stream;
+  CG_CUDA(cudaMemsetAsync(counts, 0, 2 * sizeof(uint32_t), s));
+  StageScope sc(ctx, kStageMergeMark, 2);
+  k_dirty_slots<<<grid_for(cap, 256), 256, 0, s>>>(G->v, dirty_keys, cap, slots, counts, nullptr,
+                                                   nullptr, 0);
+  k_reset_blocks<<<ctx->num_sms * 8, 256, 0, s>>>(G->v, slots, counts);
+  CG_CUDA(cudaGetLastError());
+  return CG_OK;
+}
+
+int32_t remove_dead_blocks(cg_layer* G, const uint32_t* slots, const uint32_t* counts,
+                           uint32_t listed, uint64_t* removed) {
+  cg_context* ctx = G->ctx;
+  cudaStream_t s = ctx->stream;
+  CG_CUDA(ctx->flags.reserve(static_cast<size_t>(G->num_blocks) + 1));
+  CG_CUDA(cudaMemsetAsync(ctx->flags.p, 0, static_cast<size_t>(G->num_blocks), s));
+  ctx->own_launches += 1;
+  k_flag_dead<<<grid_for(listed, 256), 256, 0, s>>>(G->v, slots, counts, ctx->flags.as<uint8_t>());
+  const int32_t rc = remove_flagged_blocks(G, ctx->flags.as<uint8_t>(), removed);
+  if (rc) return rc;
+  return finish_call(G, nullptr);
+}
+
+// cg_reproject_submaps, and the local step of cg_reproject_submaps_sharded: submaps [0, num_known)
+// are re-projected (moved ones under poses_new), submaps [num_known, n) are new and projected under
+// poses_new behind them.  The dirty set is every destination block a moved submap marks under
+// either pose and every block a new submap marks.  With `dirty`, the keys of the dirty blocks G
+// holds before the call and those it holds after it are appended to dirty->keys (a key may appear
+// twice).
+int32_t reproject_local(const cg_layer* const* submaps, size_t n, size_t num_known,
+                        const float* poses_old, const float* poses_new, float eps_translation,
+                        float eps_rotation, cg_layer* G, uint8_t* changed_out,
+                        cg_reproject_stats* stats, const DirtyKeysOut* dirty, const char* who) {
+  cg_context* ctx = G->ctx;
+  cudaStream_t s = ctx->stream;
+  if (stats) memset(stats, 0, sizeof(*stats));
+  std::vector<size_t> moved;
+  for (size_t i = 0; i < n; ++i) {
+    const cg_layer* A = submaps[i];
+    if (!A || A == G || A->ctx != ctx) {
+      set_error("%s: submap %zu invalid", who, i);
+      return CG_ERR_INVALID_ARG;
+    }
+    const bool ch = i >= num_known ||
+                    pose_changed(poses_old + 7 * i, poses_new + 7 * i, eps_translation, eps_rotation);
+    if (changed_out) changed_out[i] = ch ? 1 : 0;
+    if (ch && i < num_known) moved.push_back(i);
+  }
+  if (stats) stats->submaps_moved = moved.size();
+  if (moved.empty() && num_known == n) return CG_OK;
+  // descriptor table: [0, num_known) the known submaps under their effective pose and
+  // [num_known, n) the new ones (batch-relative block prefixes, batches start at 0 and at
+  // num_known), then every moved submap under its old and under its new pose and every new submap
+  // (one prefix over the list)
+  const size_t num_new = n - num_known;
+  std::vector<BatchSubmap> h(n + 2 * moved.size() + num_new);
+  {
+    size_t mi = 0;
+    const size_t ranges[2][2] = {{0, num_known}, {num_known, n}};
+    for (const auto& r : ranges) {
+      const size_t end = r[1];
+      for (size_t i0 = r[0]; i0 < end; i0 += kBatchMax) {
+        uint32_t total = 0;
+        for (size_t i = i0; i < std::min(end, i0 + static_cast<size_t>(kBatchMax)); ++i) {
+          const bool ch = i >= num_known || (mi < moved.size() && moved[mi] == i);
+          if (ch && i < num_known) ++mi;
+          fill_desc(h[i], submaps[i], (ch ? poses_new : poses_old) + 7 * i, total);
+          total += h[i].num_blocks;
+        }
+      }
+    }
+  }
+  uint32_t dirty_src = 0;
+  size_t dirty_bound = 0;
+  for (size_t k = 0; k < moved.size(); ++k) {
+    const size_t i = moved[k];
+    fill_desc(h[n + 2 * k], submaps[i], poses_old + 7 * i, dirty_src);
+    dirty_src += h[n + 2 * k].num_blocks;
+    fill_desc(h[n + 2 * k + 1], submaps[i], poses_new + 7 * i, dirty_src);
+    dirty_src += h[n + 2 * k + 1].num_blocks;
+    dirty_bound += 2 * mark_bound(submaps[i], G, h[n + 2 * k].num_blocks);
+  }
+  for (size_t i = num_known; i < n; ++i) {
+    BatchSubmap& d = h[n + 2 * moved.size() + (i - num_known)];
+    fill_desc(d, submaps[i], poses_new + 7 * i, dirty_src);
+    dirty_src += d.num_blocks;
+    dirty_bound += mark_bound(submaps[i], G, d.num_blocks);
+  }
+  int32_t urc = upload_descs(ctx, h.data(), h.size());
+  if (urc) return urc;
+  const BatchSubmap* d_desc = ctx->batch_desc.as<BatchSubmap>();
+  uint32_t dirty_total = 0, dirty_existing = 0;
+  uint64_t removed = 0;
+  if (dirty_src > 0) {
+    // the dirty set: destination blocks a moved submap marks under either pose, or a new one marks
+    size_t cap = 4096;
+    while (cap < 2 * dirty_bound) cap <<= 1;
+    const size_t g_blocks = static_cast<size_t>(G->num_blocks);
+    CG_CUDA(ctx->stage_a.reserve(cap * sizeof(uint64_t)));
+    CG_CUDA(ctx->stage_b.reserve((g_blocks + 2) * sizeof(uint32_t)));
+    uint32_t* counts = ctx->stage_b.as<uint32_t>();  // [0] dirty blocks present in G, [1] dirty blocks
+    uint32_t* slots = counts + 2;
+    const uint64_t* dirty_keys = ctx->stage_a.as<uint64_t>();
+    {
+      StageScope sc(ctx, kStageMergeMark, 3);
+      CG_CUDA(cudaMemsetAsync(ctx->stage_a.p, 0xFF, cap * sizeof(uint64_t), s));
+      CG_CUDA(cudaMemsetAsync(counts, 0, 2 * sizeof(uint32_t), s));
+      k_mark_batch<<<grid_for(dirty_src, 128), 128, 0, s>>>(
+          d_desc + n, static_cast<int>(2 * moved.size() + num_new), dirty_src, G->v.block_size,
+          ctx->stage_a.as<uint64_t>(), nullptr, static_cast<uint32_t>(cap - 1), G->v.err, nullptr, 0);
+      k_dirty_slots<<<grid_for(cap, 256), 256, 0, s>>>(
+          G->v, dirty_keys, static_cast<uint32_t>(cap), slots, counts,
+          dirty ? dirty->keys : nullptr, dirty ? dirty->count : nullptr, dirty ? dirty->cap : 0);
+    }
+    // the dirty blocks G holds once the call is done
+    auto publish_after = [&]() -> int32_t {
+      if (!dirty) return CG_OK;
+      ctx->own_launches += 1;
+      k_dirty_slots<<<grid_for(cap, 256), 256, 0, s>>>(G->v, dirty_keys, static_cast<uint32_t>(cap),
+                                                       nullptr, nullptr, dirty->keys, dirty->count,
+                                                       dirty->cap);
+      CG_CUDA(cudaGetLastError());
+      return CG_OK;
+    };
+    // When the moved submaps dirty a large part of the map (a corridor map where every block is
+    // shared by a few submaps: a tenth of the poses dirties more than half of the blocks),
+    // rebuilding the dirty blocks from ALL submaps that reach them plus the block removal costs
+    // more than the full rebuild, which gives the same layer by definition: take that instead.
+    {
+      uint32_t h_dirty[2] = {0, 0};
+      CG_CUDA(cudaMemcpyAsync(h_dirty, counts, sizeof(h_dirty), cudaMemcpyDeviceToHost, s));
+      CG_CUDA(cudaStreamSynchronize(s));
+      if (static_cast<double>(h_dirty[0]) > full_rebuild_fraction() * static_cast<double>(g_blocks)) {
+        std::vector<float> eff(7 * n);
+        size_t mi = 0;
+        for (size_t i = 0; i < n; ++i) {
+          const bool ch = i >= num_known || (mi < moved.size() && moved[mi] == i);
+          if (ch && i < num_known) ++mi;
+          memcpy(&eff[7 * i], (ch ? poses_new : poses_old) + 7 * i, 7 * sizeof(float));
+        }
+        int32_t rc = cg_layer_clear(G);
+        if (rc) return rc;
+        cg_merge_stats ms;
+        rc = cg_project_submaps(submaps, eff.data(), n, G, &ms);
+        if (stats) {
+          stats->blocks_dirty = h_dirty[1];
+          stats->candidates = ms.blocks_candidate;
+          stats->blocks_folded = ms.blocks_out;
+          stats->full_rebuild = 1;
+        }
+        return rc ? rc : publish_after();
+      }
+    }
+    {
+      StageScope sc(ctx, kStageMergeMark, 1);
+      k_reset_blocks<<<ctx->num_sms * 8, 256, 0, s>>>(G->v, slots, counts);
+    }
+    // every known submap that reaches a dirty block is folded into it again, in submap order; the
+    // new submaps follow as plain batches
+    for (size_t i0 = 0; i0 < num_known; i0 += kBatchMax) {
+      int32_t rc = project_batch(submaps, h.data(), d_desc, i0,
+                                 std::min(num_known, i0 + static_cast<size_t>(kBatchMax)), G,
+                                 dirty_keys, static_cast<uint32_t>(cap - 1));
+      if (rc) return rc;
+    }
+    for (size_t i0 = num_known; i0 < n; i0 += kBatchMax) {
+      int32_t rc = project_batch(submaps, h.data(), d_desc, i0,
+                                 std::min(n, i0 + static_cast<size_t>(kBatchMax)), G);
+      if (rc) return rc;
+    }
+    // dirty blocks that ended up without data leave the layer (a fresh projection would not
+    // have allocated them)
+    uint32_t h_counts[2] = {0, 0};
+    CG_CUDA(cudaMemcpyAsync(h_counts, counts, sizeof(h_counts), cudaMemcpyDeviceToHost, s));
+    CG_CUDA(cudaStreamSynchronize(s));
+    dirty_existing = h_counts[0];
+    dirty_total = h_counts[1];
+    if (dirty_existing > 0) {
+      // new blocks were claimed behind the old ones: flags cover the current block count
+      CallCounters c0;
+      int32_t rc = finish_call(G, &c0);
+      if (rc) return rc;
+      const CallCounters keep = c0;
+      rc = remove_dead_blocks(G, slots, counts, dirty_existing, &removed);
+      if (rc) return rc;
+      if (stats) {
+        stats->candidates = keep.candidates;
+        stats->blocks_folded = keep.blocks_out;
+      }
+    }
+    const int32_t rc = publish_after();
+    if (rc) return rc;
+  }
+  if (dirty_existing == 0) {
+    CallCounters c;
+    const int32_t rc = finish_call(G, &c);
+    if (rc) return rc;
+    if (stats) {
+      stats->candidates = c.candidates;
+      stats->blocks_folded = c.blocks_out;
+    }
+  }
+  if (stats) {
+    stats->blocks_dirty = dirty_total;
+    stats->blocks_removed = removed;
+  }
+  return CG_OK;
 }
 
 }  // namespace cg
@@ -862,165 +1090,14 @@ int32_t cg_project_submaps(const cg_layer* const* submaps, const float* poses, s
   return rc;
 }
 
-// dirty blocks / blocks of the map above which cg_reproject_submaps rebuilds the whole map
-// (CG_REPROJECT_FULL_FRACTION overrides it; the tests use 2 to force the block-by-block path)
-static double full_rebuild_fraction() {
-  const char* e = getenv("CG_REPROJECT_FULL_FRACTION");
-  return (e && *e) ? atof(e) : 0.3;
-}
-
 int32_t cg_reproject_submaps(const cg_layer* const* submaps, const float* poses_old,
                              const float* poses_new, size_t n, float eps_translation,
                              float eps_rotation, cg_layer* G, uint8_t* changed_out,
                              cg_reproject_stats* stats) {
   if (!G || (n && (!submaps || !poses_old || !poses_new))) return CG_ERR_INVALID_ARG;
   CG_CUDA(cudaSetDevice(G->ctx->device));
-  cg_context* ctx = G->ctx;
-  cudaStream_t s = ctx->stream;
-  if (stats) memset(stats, 0, sizeof(*stats));
-  std::vector<size_t> moved;
-  for (size_t i = 0; i < n; ++i) {
-    const cg_layer* A = submaps[i];
-    if (!A || A == G || A->ctx != ctx) {
-      set_error("cg_reproject_submaps: submap %zu invalid", i);
-      return CG_ERR_INVALID_ARG;
-    }
-    const bool ch = pose_changed(poses_old + 7 * i, poses_new + 7 * i, eps_translation, eps_rotation);
-    if (changed_out) changed_out[i] = ch ? 1 : 0;
-    if (ch) moved.push_back(i);
-  }
-  if (stats) stats->submaps_moved = moved.size();
-  if (moved.empty()) return CG_OK;
-  // descriptor table: [0, n) all submaps under their effective pose (batch-relative block prefix),
-  // then every moved submap under its old and under its new pose (one prefix over the list)
-  std::vector<BatchSubmap> h(n + 2 * moved.size());
-  {
-    size_t mi = 0;
-    for (size_t i0 = 0; i0 < n; i0 += kBatchMax) {
-      uint32_t total = 0;
-      for (size_t i = i0; i < std::min(n, i0 + static_cast<size_t>(kBatchMax)); ++i) {
-        const bool ch = mi < moved.size() && moved[mi] == i;
-        if (ch) ++mi;
-        fill_desc(h[i], submaps[i], (ch ? poses_new : poses_old) + 7 * i, total);
-        total += h[i].num_blocks;
-      }
-    }
-  }
-  uint32_t dirty_src = 0;
-  size_t dirty_bound = 0;
-  for (size_t k = 0; k < moved.size(); ++k) {
-    const size_t i = moved[k];
-    fill_desc(h[n + 2 * k], submaps[i], poses_old + 7 * i, dirty_src);
-    dirty_src += h[n + 2 * k].num_blocks;
-    fill_desc(h[n + 2 * k + 1], submaps[i], poses_new + 7 * i, dirty_src);
-    dirty_src += h[n + 2 * k + 1].num_blocks;
-    dirty_bound += 2 * mark_bound(submaps[i], G, h[n + 2 * k].num_blocks);
-  }
-  int32_t urc = upload_descs(ctx, h.data(), h.size());
-  if (urc) return urc;
-  const BatchSubmap* d_desc = ctx->batch_desc.as<BatchSubmap>();
-  uint32_t dirty_total = 0, dirty_existing = 0;
-  uint64_t removed = 0;
-  if (dirty_src > 0) {
-    // the dirty set: destination blocks a moved submap marks under either pose
-    size_t cap = 4096;
-    while (cap < 2 * dirty_bound) cap <<= 1;
-    const size_t g_blocks = static_cast<size_t>(G->num_blocks);
-    CG_CUDA(ctx->stage_a.reserve(cap * sizeof(uint64_t)));
-    CG_CUDA(ctx->stage_b.reserve((g_blocks + 2) * sizeof(uint32_t)));
-    uint32_t* counts = ctx->stage_b.as<uint32_t>();  // [0] dirty blocks present in G, [1] dirty blocks
-    uint32_t* slots = counts + 2;
-    {
-      StageScope sc(ctx, kStageMergeMark, 3);
-      CG_CUDA(cudaMemsetAsync(ctx->stage_a.p, 0xFF, cap * sizeof(uint64_t), s));
-      CG_CUDA(cudaMemsetAsync(counts, 0, 2 * sizeof(uint32_t), s));
-      k_mark_batch<<<grid_for(dirty_src, 128), 128, 0, s>>>(
-          d_desc + n, static_cast<int>(2 * moved.size()), dirty_src, G->v.block_size,
-          ctx->stage_a.as<uint64_t>(), nullptr, static_cast<uint32_t>(cap - 1), G->v.err, nullptr, 0);
-      k_dirty_slots<<<grid_for(cap, 256), 256, 0, s>>>(G->v, ctx->stage_a.as<uint64_t>(),
-                                                       static_cast<uint32_t>(cap), slots, counts);
-    }
-    // When the moved submaps dirty a large part of the map (a corridor map where every block is
-    // shared by a few submaps: a tenth of the poses dirties more than half of the blocks),
-    // rebuilding the dirty blocks from ALL submaps that reach them plus the block removal costs
-    // more than the full rebuild, which gives the same layer by definition: take that instead.
-    {
-      uint32_t h_dirty[2] = {0, 0};
-      CG_CUDA(cudaMemcpyAsync(h_dirty, counts, sizeof(h_dirty), cudaMemcpyDeviceToHost, s));
-      CG_CUDA(cudaStreamSynchronize(s));
-      if (static_cast<double>(h_dirty[0]) > full_rebuild_fraction() * static_cast<double>(g_blocks)) {
-        std::vector<float> eff(7 * n);
-        size_t mi = 0;
-        for (size_t i = 0; i < n; ++i) {
-          const bool ch = mi < moved.size() && moved[mi] == i;
-          if (ch) ++mi;
-          memcpy(&eff[7 * i], (ch ? poses_new : poses_old) + 7 * i, 7 * sizeof(float));
-        }
-        int32_t rc = cg_layer_clear(G);
-        if (rc) return rc;
-        cg_merge_stats ms;
-        rc = cg_project_submaps(submaps, eff.data(), n, G, &ms);
-        if (stats) {
-          stats->blocks_dirty = h_dirty[1];
-          stats->candidates = ms.blocks_candidate;
-          stats->blocks_folded = ms.blocks_out;
-          stats->full_rebuild = 1;
-        }
-        return rc;
-      }
-    }
-    {
-      StageScope sc(ctx, kStageMergeMark, 1);
-      k_reset_blocks<<<ctx->num_sms * 8, 256, 0, s>>>(G->v, slots, counts);
-    }
-    // every submap that reaches a dirty block is folded into it again, in submap order
-    for (size_t i0 = 0; i0 < n; i0 += kBatchMax) {
-      int32_t rc = project_batch(submaps, h.data(), d_desc, i0, std::min(n, i0 + static_cast<size_t>(kBatchMax)),
-                                 G, ctx->stage_a.as<uint64_t>(), static_cast<uint32_t>(cap - 1));
-      if (rc) return rc;
-    }
-    // dirty blocks that ended up without data leave the layer (a fresh projection would not
-    // have allocated them)
-    uint32_t h_counts[2] = {0, 0};
-    CG_CUDA(cudaMemcpyAsync(h_counts, counts, sizeof(h_counts), cudaMemcpyDeviceToHost, s));
-    CG_CUDA(cudaStreamSynchronize(s));
-    dirty_existing = h_counts[0];
-    dirty_total = h_counts[1];
-    if (dirty_existing > 0) {
-      // new blocks were claimed behind the old ones: flags cover the current block count
-      CallCounters c0;
-      int32_t rc = finish_call(G, &c0);
-      if (rc) return rc;
-      const CallCounters keep = c0;
-      CG_CUDA(ctx->flags.reserve(static_cast<size_t>(G->num_blocks) + 1));
-      CG_CUDA(cudaMemsetAsync(ctx->flags.p, 0, static_cast<size_t>(G->num_blocks), s));
-      ctx->own_launches += 1;
-      k_flag_dead<<<grid_for(dirty_existing, 256), 256, 0, s>>>(G->v, slots, counts,
-                                                                ctx->flags.as<uint8_t>());
-      rc = remove_flagged_blocks(G, ctx->flags.as<uint8_t>(), &removed);
-      if (rc) return rc;
-      rc = finish_call(G, nullptr);
-      if (rc) return rc;
-      if (stats) {
-        stats->candidates = keep.candidates;
-        stats->blocks_folded = keep.blocks_out;
-      }
-    }
-  }
-  if (dirty_existing == 0) {
-    CallCounters c;
-    const int32_t rc = finish_call(G, &c);
-    if (rc) return rc;
-    if (stats) {
-      stats->candidates = c.candidates;
-      stats->blocks_folded = c.blocks_out;
-    }
-  }
-  if (stats) {
-    stats->blocks_dirty = dirty_total;
-    stats->blocks_removed = removed;
-  }
-  return CG_OK;
+  return reproject_local(submaps, n, n, poses_old, poses_new, eps_translation, eps_rotation, G,
+                         changed_out, stats, nullptr, "cg_reproject_submaps");
 }
 
 }  // extern "C"

@@ -427,6 +427,32 @@ inline void getProjectedMapSharded(const std::vector<const TsdfLayer*>& my_subma
   check(cg_project_submaps_sharded(handles.data(), poses.data(), handles.size(),
                                    partial_layer->handle(), owned_layer->handle(), stats));
 }
+// The sharded map after a pose-graph update (collective): T_M_S_old holds the poses of the submaps
+// this rank passed last, T_M_S_new one pose per submap, the submaps behind T_M_S_old.size() being
+// new.  Afterwards both layers hold what getProjectedMapSharded under the effective poses would
+// leave.  Returns which submaps counted as moved or new.
+inline std::vector<uint8_t> reprojectSubmapsSharded(
+    const std::vector<const TsdfLayer*>& my_submap_layers,
+    const std::vector<Transformation>& T_M_S_old, const std::vector<Transformation>& T_M_S_new,
+    TsdfLayer* partial_layer, TsdfLayer* owned_layer, float eps_translation = 0.0f,
+    float eps_rotation = 0.0f, cg_reproject_sharded_stats* stats = nullptr) {
+  const size_t n = my_submap_layers.size();
+  if (T_M_S_new.size() != n || T_M_S_old.size() > n)
+    fatal_handler()(CG_ERR_INVALID_ARG,
+                    "reprojectSubmapsSharded: one new pose per submap and at most as many old ones expected");
+  std::vector<const cg_layer*> handles(n);
+  std::vector<float> po(7 * T_M_S_old.size()), pn(7 * n);
+  for (size_t i = 0; i < n; ++i) {
+    handles[i] = my_submap_layers[i]->handle();
+    if (i < T_M_S_old.size()) std::copy(T_M_S_old[i].data(), T_M_S_old[i].data() + 7, po.begin() + 7 * i);
+    std::copy(T_M_S_new[i].data(), T_M_S_new[i].data() + 7, pn.begin() + 7 * i);
+  }
+  std::vector<uint8_t> changed(n, 0);
+  check(cg_reproject_submaps_sharded(handles.data(), n, T_M_S_old.size(), po.data(), pn.data(),
+                                     eps_translation, eps_rotation, partial_layer->handle(),
+                                     owned_layer->handle(), changed.data(), stats));
+  return changed;
+}
 
 // ---- voxblox::MeshIntegrator<TsdfVoxel>::generateMesh over a device-resident layer (what
 // saveAndPubCombinedMesh runs on the projected map, server_visualizer.cpp:123-126): per-block

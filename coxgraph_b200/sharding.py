@@ -147,6 +147,16 @@ def project_sharded_native(local_submaps, local_poses, partial_layer, owned_laye
     getProjectedMapSharded(local_submaps, local_poses, partial_layer, owned_layer)
 
 
+def reproject_sharded_native(local_submaps, poses_old, poses_new, partial_layer, owned_layer,
+                             eps_translation=0.0, eps_rotation=0.0):
+    """After project_sharded_native: bring the sharded global map up to date with new poses and
+    appended submaps (cg_reproject_submaps_sharded), folding only the owned blocks that changed.
+    Returns (changed mask, ReprojectShardedStats)."""
+    from .api import reprojectSubmapsSharded
+    return reprojectSubmapsSharded(local_submaps, poses_old, poses_new, partial_layer, owned_layer,
+                                   eps_translation, eps_rotation)
+
+
 def mesh_sharded(owned_layer, min_weight=1e-4, use_color=True, only_updated=False, fetch=True):
     """The mesh half of saveAndPubCombinedMesh over all ranks (cg_layer_mesh_sharded), after
     project_sharded_native: every rank meshes the blocks of its owned layer where they lie, reading

@@ -538,6 +538,48 @@ int32_t cg_project_submaps_sharded(const cg_layer* const* submaps, const float* 
                                    size_t num_submaps, cg_layer* partial_layer,
                                    cg_layer* owned_layer, cg_merge_stats* stats);
 
+/* cg_reproject_submaps over all ranks: the sharded global map after a pose-graph update (the
+ * server's rebuild trigger, coxgraph/include/coxgraph/server/coxgraph_server.h:275-283), without
+ * projecting every submap again.  Collective, like cg_gather_global: every rank passes its own
+ * submap list.  Precondition: submaps [0, num_known) are the list this rank last passed to
+ * cg_project_submaps_sharded or to this call, with poses_old (num_known x 7), and the rank has kept
+ * `partial` and `owned` since; submaps [num_known, num_submaps) are new and come with poses_new
+ * (num_submaps x 7).  A known submap is moved under cg_reproject_submaps' eps rules;
+ * changed_out[i] (optional) is 1 for moved and new submaps.  With pose_eff[i] = poses_new[i] for
+ * moved and new submaps and poses_old[i] otherwise, every rank's `owned` and `partial` then hold
+ * exactly what cg_layer_clear(owned) + cg_project_submaps_sharded(submaps, pose_eff, partial,
+ * owned) on all ranks leaves: the same blocks per rank, voxels and has_data.  Blocks folded again
+ * get `updated` = 1; every other block keeps its flags, so cg_layer_reset_updated before the call
+ * and cg_layer_mesh_sharded(only_updated) after it mesh only what changed.
+ * Every rank re-projects its partial layer locally (cg_reproject_submaps, then the new submaps)
+ * and publishes the dirty keys its partial layer holds before or after; only the owned blocks of
+ * their union D are folded again, reset, or removed (DESIGN.md §5).  When |D| exceeds
+ * CG_REPROJECT_FULL_FRACTION (default 0.3, rank 0's value) of the global block count, every rank
+ * clears `owned` and runs the whole gather instead (same result).
+ * Errors (CG_ERR_INVALID_ARG, message naming the problem, layers untouched): no communicator,
+ * num_known > num_submaps, null arrays where num_submaps > 0, a submap that is `partial` or
+ * `owned` or of another context, layers of different voxel size, and a `partial` that is not the
+ * layer the last cg_gather_global on this context used.  A rank whose arguments are rejected or
+ * whose local step fails (e.g. CG_ERR_POOL_FULL) makes every rank return an error without
+ * touching `owned`; the chain then has to restart with cg_project_submaps_sharded. */
+typedef struct cg_reproject_sharded_stats {
+  uint64_t submaps_moved;      /* this rank: known submaps whose pose moved beyond eps */
+  uint64_t submaps_added;      /* this rank: num_submaps - num_known */
+  uint64_t blocks_dirty_local; /* destination blocks this rank's moved / new submaps reach */
+  uint64_t blocks_dirty;       /* |D|: dirty blocks some rank's partial layer holds before or
+                                  after the call (the same on every rank) */
+  uint64_t blocks_folded;      /* owned blocks this rank folded (full rebuild: all of them) */
+  uint64_t blocks_removed;     /* owned blocks this rank dropped (no data left, or now owned
+                                  elsewhere; 0 on a full rebuild) */
+  uint64_t full_rebuild;       /* 1 on every rank when the owned layers were gathered whole */
+} cg_reproject_sharded_stats;
+int32_t cg_reproject_submaps_sharded(const cg_layer* const* submaps, size_t num_submaps,
+                                     size_t num_known, const float* poses_old,
+                                     const float* poses_new, float eps_translation,
+                                     float eps_rotation, cg_layer* partial_layer,
+                                     cg_layer* owned_layer, uint8_t* changed_out,
+                                     cg_reproject_sharded_stats* stats);
+
 /* MeshIntegrator::generateMesh over the sharded global map, where it lies (the mesh half of
  * saveAndPubCombinedMesh on several GPUs).  Collective: every rank of the context's communicator
  * passes its owned layer (cg_gather_global's `owned`; all ranks' owned layers have the same voxel
