@@ -60,6 +60,74 @@ __host__ __device__ __forceinline__ uint32_t hash_key(uint64_t k) {
   k ^= k >> 33;
   return static_cast<uint32_t>(k);
 }
+// Which of n candidates owns a block: the rank of the packed exchange (cg_block_owner) and the
+// holder that folds a block of the sharded map (comm.cu) are both picked by this hash.
+__host__ __device__ __forceinline__ uint32_t owner_pick(uint64_t key, uint32_t n) {
+  return (hash_key(key ^ 0x9E3779B97F4A7C15ULL) >> 7) % n;
+}
+
+// ------------------------------------------------------------------ scratch key set
+// Open addressing over mask + 1 entries (a power of two) of 64-bit keys, kEmptyKey = free entry,
+// linear probing from hash_key.  Every scratch set is sized by key_set_capacity to at least twice
+// the keys it can receive, so a probe always ends at the key or at a free entry.  A kernel that
+// fills the set holds a KeySet, one that only probes it a KeyLookup (kernels build theirs from a
+// `const __restrict__` parameter, which lets the probes use the read-only data cache).
+template <class Key>
+struct KeySetOf {
+  Key* keys;
+  uint32_t mask;
+
+  // the entry of `key`, claimed if the key is new (*inserted, if given: this thread claimed it);
+  // -1 after mask + 1 probes found neither the key nor a free entry
+  __device__ __forceinline__ int insert(unsigned long long key, bool* inserted = nullptr) const {
+    if (inserted) *inserted = false;
+    const uint32_t hash = hash_key(key);
+    for (uint32_t n = 0; n <= mask; ++n) {
+      const uint32_t h = (hash + n) & mask;
+      const unsigned long long k = keys[h];
+      if (k == key) return static_cast<int>(h);
+      if (k == kEmptyKey) {
+        const unsigned long long old = atomicCAS(&keys[h], kEmptyKey, key);
+        if (old == kEmptyKey) {
+          if (inserted) *inserted = true;
+          return static_cast<int>(h);
+        }
+        if (old == key) return static_cast<int>(h);
+      }
+    }
+    return -1;
+  }
+  // the entry of `key`, or -1
+  __device__ __forceinline__ int find(unsigned long long key) const {
+    uint32_t h = hash_key(key) & mask;
+    for (;;) {
+      const unsigned long long k = keys[h];
+      if (k == key) return static_cast<int>(h);
+      if (k == kEmptyKey) return -1;
+      h = (h + 1) & mask;
+    }
+  }
+  // a loop of its own rather than find(key) >= 0: the ray walk probes the anti-grazing set with
+  // it, and this form compiles there to the code the walk was tuned with
+  __device__ __forceinline__ bool contains(unsigned long long key) const {
+    uint32_t h = hash_key(key) & mask;
+    for (;;) {
+      const unsigned long long k = keys[h];
+      if (k == key) return true;
+      if (k == kEmptyKey) return false;
+      h = (h + 1) & mask;
+    }
+  }
+};
+using KeySet = KeySetOf<unsigned long long>;
+using KeyLookup = KeySetOf<const unsigned long long>;
+// entries of a key set for n keys: the smallest power of two >= 2 n, and at least `floor` (a power
+// of two)
+inline size_t key_set_capacity(size_t n, size_t floor) {
+  size_t cap = floor;
+  while (cap < 2 * n) cap <<= 1;
+  return cap;
+}
 
 // ------------------------------------------------------------------ device view of a layer
 struct LayerView {
@@ -133,20 +201,14 @@ struct LayerView {
 // CUDA IPC mapping).  A reference is a pool slot of this layer (>= 0), -1 for a block no rank
 // holds, or -2 - (map entry) for a block found in the map.
 struct ShardedBlocks {
-  const unsigned long long* keys;  // [cap_mask + 1] block key or kEmptyKey
-  const float* const* planes_of;   // [cap_mask + 1] the block's distance plane
-  uint32_t cap_mask;
+  KeyLookup map;                  // block keys of every rank's owned layer
+  const float* const* planes_of;  // [map.mask + 1] the block's distance plane
 
   __device__ __forceinline__ int find(const LayerView& L, uint64_t key) const {
     const int s = L.find_slot(key);
     if (s >= 0) return s;
-    uint32_t h = hash_key(key) & cap_mask;
-    for (;;) {
-      const unsigned long long k = keys[h];
-      if (k == key) return -2 - static_cast<int>(h);
-      if (k == kEmptyKey) return -1;
-      h = (h + 1) & cap_mask;
-    }
+    const int e = map.find(key);
+    return e < 0 ? -1 : -2 - e;
   }
   __device__ __forceinline__ const float* planes(const LayerView& L, int ref) const {
     return ref >= 0 ? L.dist_plane(ref) : planes_of[-2 - ref];
@@ -257,7 +319,7 @@ struct FrontBufs {
   DevBuf ray_id, frame_count;               // bundle -> ray id; (frame, chunk) bundle counts
   DevBuf scan_partials;
   DevBuf grazing_keys, grazing_ray_key;     // anti-grazing: the scan's bundle voxels
-  uint32_t grazing_mask = 0;
+  KeySet grazing_set{};                     // over grazing_keys
   uint32_t* d_class_count = nullptr;        // bundle size-class histogram + scatter cursors
   int* d_key_bounds = nullptr;              // [6] running min / max of the bundle voxel fields
   uint32_t* d_select_count = nullptr;       // output count of the stream compactions
@@ -463,5 +525,22 @@ struct StageScope {
 inline unsigned grid_for(size_t n, unsigned block) {
   return static_cast<unsigned>((n + block - 1) / block);
 }
+
+// Lets kKernel take `bytes` of dynamic shared memory (above the default 48 KB) on `device`; the
+// attribute is set once per device ordinal (a process may hold contexts on several GPUs).
+template <auto kKernel>
+cudaError_t allow_dynamic_smem(int device, size_t bytes) {
+  static bool done[64] = {};
+  const bool known = device >= 0 && device < 64;
+  if (known && done[device]) return cudaSuccess;
+  const cudaError_t e = cudaFuncSetAttribute(kKernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                             static_cast<int>(bytes));
+  if (e == cudaSuccess && known) done[device] = true;
+  return e;
+}
+
+// layer.cu: v[i] = i; and packed block keys -> int3 block indices (idx[3 i .. 3 i + 2])
+__global__ void k_iota(uint32_t* v, int n);
+__global__ void k_unpack_idx(const uint64_t* __restrict__ keys, uint32_t n, int32_t* __restrict__ idx);
 
 }  // namespace cg

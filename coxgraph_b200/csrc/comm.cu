@@ -137,38 +137,31 @@ struct cg_comm {
   cg::Binding partial, owned;
   std::vector<cg::Mapping> maps;
   uint64_t maps_opened = 0;           // cudaIpcOpenMemHandle calls since cg_comm_init
-  // the holder map (scratch, rebuilt every call): block key -> set of ranks holding the block
-  unsigned long long* hkeys = nullptr;
-  unsigned long long* hmask = nullptr;
   // cg_reproject_submaps_sharded: the union D of every rank's dirty keys (scratch, lazily sized)
   cg::DevBuf dset;
   size_t dcap = 0;
   uint32_t* dcounters = nullptr;      // [0] |D|, [1] owned blocks of all ranks, [2] overflow, [3] fraction
-  uint32_t* hbase = nullptr;          // owned entries: first element of the block's slot list
-  uint32_t* mine = nullptr;           // entries this rank owns
-  uint32_t* slots = nullptr;          // pool slots of the holders' copies, per owned block
-  uint32_t* counters = nullptr;       // [0] owned entries, [1] slot list cursor, [2] overflow
+  // the holder map (scratch, rebuilt every call): block key -> set of ranks holding the block,
+  // hcap entries of hkeys / hmask / hbase
+  cg::DevBuf hkeys, hmask;
+  cg::DevBuf hbase;                   // owned entries: first element of the block's slot list
+  cg::DevBuf mine;                    // [list_cap] entries this rank owns
+  cg::DevBuf slots;                   // [list_cap] pool slots of the holders' copies, per owned block
+  cg::DevBuf counters;                // [0] owned entries, [1] slot list cursor, [2] overflow
   size_t hcap = 0, list_cap = 0;
-  // the key map of cg_layer_mesh_sharded over every rank's owned layer (rebuilt every call)
-  unsigned long long* mkeys = nullptr;
-  unsigned long long* mmask = nullptr;
-  const float** mplanes = nullptr;    // the block's distance plane in its holder's pool
-  uint32_t* mcounters = nullptr;      // k_build_holders' words ([2] overflow: cannot happen)
+  // the key map of cg_layer_mesh_sharded over every rank's owned layer (rebuilt every call), mcap
+  // entries of mkeys / mmask / mplanes
+  cg::DevBuf mkeys, mmask;
+  cg::DevBuf mplanes;                 // the block's distance plane in its holder's pool
+  cg::DevBuf mcounters;               // k_build_holders' words ([2] overflow: cannot happen)
   size_t mcap = 0;
 };
 
 namespace cg {
 
-__device__ __forceinline__ uint32_t holder_find(const unsigned long long* __restrict__ hkeys,
-                                                uint32_t hmask_cap, unsigned long long key) {
-  uint32_t h = hash_key(key) & hmask_cap;
-  while (hkeys[h] != key) h = (h + 1) & hmask_cap;
-  return h;
-}
 // the owner of a block: one of its holders, picked by a hash of the block index
 __device__ __forceinline__ int pick_owner(unsigned long long key, unsigned long long mask) {
-  int n = static_cast<int>((hash_key(key ^ 0x9E3779B97F4A7C15ULL) >> 7) %
-                           static_cast<uint32_t>(__popcll(mask)));
+  int n = static_cast<int>(owner_pick(key, static_cast<uint32_t>(__popcll(mask))));
   unsigned long long m = mask;
   while (n-- > 0) m &= m - 1;
   return __ffsll(static_cast<long long>(m)) - 1;
@@ -177,41 +170,24 @@ __device__ __forceinline__ int pick_owner(unsigned long long key, unsigned long 
 // Every block key of every rank's layer (read through the peer mappings) enters the map with its
 // rank's bit.  Grid y = rank.  With `planes` (the key map of cg_layer_mesh_sharded) the entry also
 // records where the block's planes are, and a key that reaches an entry another rank has already
-// marked is held twice: the smallest such key goes to *dup_key.  With `filter` (a key set of
+// marked is held twice: the smallest such key goes to *dup_key.  With `filter_keys` (a key set of
 // filter_mask + 1 entries, cg_reproject_submaps_sharded) only the keys in it enter the map.
-__device__ __forceinline__ bool in_key_set(const unsigned long long* __restrict__ keys, uint32_t mask,
-                                           unsigned long long key) {
-  uint32_t h = hash_key(key) & mask;
-  for (;;) {
-    const unsigned long long k = keys[h];
-    if (k == key) return true;
-    if (k == kEmptyKey) return false;
-    h = (h + 1) & mask;
-  }
-}
-__global__ void k_build_holders(const PeerLayer* __restrict__ peers, unsigned long long* hkeys,
-                                unsigned long long* hmask, uint32_t hcap_mask, uint32_t* counters,
+__global__ void k_build_holders(const PeerLayer* __restrict__ peers, KeySet map,
+                                unsigned long long* hmask, uint32_t* counters,
                                 const float** planes, unsigned long long* dup_key,
-                                const unsigned long long* __restrict__ filter, uint32_t filter_mask) {
+                                const unsigned long long* __restrict__ filter_keys,
+                                uint32_t filter_mask) {
+  const KeyLookup filter{filter_keys, filter_mask};
   const int r = blockIdx.y;
   const PeerLayer P = peers[r];
   const uint32_t n = P.shared[0];
   for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
     const unsigned long long key = P.block_keys[i];
-    if (filter && !in_key_set(filter, filter_mask, key)) continue;
-    uint32_t h = hash_key(key) & hcap_mask;
-    for (uint32_t tries = 0;; ++tries) {
-      const unsigned long long k = hkeys[h];
-      if (k == key) break;
-      if (k == kEmptyKey) {
-        const unsigned long long old = atomicCAS(&hkeys[h], kEmptyKey, key);
-        if (old == kEmptyKey || old == key) break;
-      }
-      h = (h + 1) & hcap_mask;
-      if (tries > hcap_mask) {  // cannot happen: the map holds every block of every rank
-        atomicExch(&counters[2], 1u);
-        return;
-      }
+    if (filter.keys && !filter.contains(key)) continue;
+    const int h = map.insert(key);
+    if (h < 0) {  // cannot happen: the map holds every block of every rank
+      atomicExch(&counters[2], 1u);
+      return;
     }
     const unsigned long long held = atomicOr(&hmask[h], 1ull << r);
     if (planes) {
@@ -244,14 +220,17 @@ __global__ void k_holder_slots(const PeerLayer* __restrict__ peers,
                                const unsigned long long* __restrict__ hmask,
                                const uint32_t* __restrict__ hbase, uint32_t hcap_mask, int me,
                                uint32_t* __restrict__ slots, uint32_t slots_cap,
-                               const unsigned long long* __restrict__ filter, uint32_t filter_mask) {
+                               const unsigned long long* __restrict__ filter_keys,
+                               uint32_t filter_mask) {
+  const KeyLookup map{hkeys, hcap_mask}, filter{filter_keys, filter_mask};
   const int r = blockIdx.y;
   const PeerLayer P = peers[r];
   const uint32_t n = P.shared[0];
   for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
     const unsigned long long key = P.block_keys[i];
-    if (filter && !in_key_set(filter, filter_mask, key)) continue;
-    const uint32_t e = holder_find(hkeys, hcap_mask, key);
+    if (filter.keys && !filter.contains(key)) continue;
+    const int e = map.find(key);
+    if (e < 0) continue;  // not in the map: k_build_holders raised its overflow word
     const unsigned long long mask = hmask[e];
     if (pick_owner(key, mask) != me) continue;
     const uint32_t at = hbase[e] + __popcll(mask & ((1ull << r) - 1ull));
@@ -364,8 +343,8 @@ __global__ void k_comm_overflow(const uint32_t* counters, int32_t* err) {
 // cg_reproject_submaps_sharded: every rank's published dirty keys (read through the peer mappings)
 // enter the set D; counters [0] |D|, [1] owned blocks of all ranks, [2] a rank published more keys
 // than its buffer holds, [3] rank 0's full-rebuild fraction.  Grid y = rank.
-__global__ void k_union_dirty(const PeerLayer* __restrict__ peers, uint32_t dirty_cap,
-                              unsigned long long* set, uint32_t set_mask, uint32_t* counters) {
+__global__ void k_union_dirty(const PeerLayer* __restrict__ peers, uint32_t dirty_cap, KeySet set,
+                              uint32_t* counters) {
   const int r = blockIdx.y;
   const PeerLayer P = peers[r];
   const uint32_t published = P.shared[2];
@@ -376,21 +355,9 @@ __global__ void k_union_dirty(const PeerLayer* __restrict__ peers, uint32_t dirt
   }
   const uint32_t n = min(published, dirty_cap);
   for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-    const unsigned long long key = P.dirty_keys[i];
-    uint32_t h = hash_key(key) & set_mask;
-    for (;;) {
-      const unsigned long long k = set[h];
-      if (k == key) break;
-      if (k == kEmptyKey) {
-        const unsigned long long old = atomicCAS(&set[h], kEmptyKey, key);
-        if (old == kEmptyKey) {
-          atomicAdd(&counters[0], 1u);
-          break;
-        }
-        if (old == key) break;
-      }
-      h = (h + 1) & set_mask;
-    }
+    bool inserted;
+    set.insert(P.dirty_keys[i], &inserted);
+    if (inserted) atomicAdd(&counters[0], 1u);
   }
 }
 __global__ void k_publish_words(uint32_t* shared, uint32_t partial_blocks, uint32_t owned_blocks,
@@ -456,13 +423,9 @@ static void unbind(cg_comm* c) {
   c->dcap = 0;
   if (c->dcounters) cudaFree(c->dcounters);
   c->dcounters = nullptr;
-  void* bufs[] = {c->hkeys, c->hmask, c->hbase, c->mine, c->slots, c->counters,
-                  c->mkeys, c->mmask, c->mplanes, c->mcounters};
-  for (void* p : bufs)
-    if (p) cudaFree(p);
-  c->hbase = c->mine = c->slots = c->counters = c->mcounters = nullptr;
-  c->hkeys = c->hmask = c->mkeys = c->mmask = nullptr;
-  c->mplanes = nullptr;
+  for (DevBuf* d : {&c->hkeys, &c->hmask, &c->hbase, &c->mine, &c->slots, &c->counters, &c->mkeys,
+                    &c->mmask, &c->mplanes, &c->mcounters})
+    d->release();
   c->hcap = c->list_cap = c->mcap = 0;
 }
 
@@ -470,13 +433,6 @@ static int32_t barrier(cg_context* ctx) {
   cg_comm* c = ctx->comm;
   CG_NCCL(g_nccl.AllReduce(c->d_token, c->d_token, 1, ncclInt32, ncclSum, c->comm, ctx->stream));
   return CG_OK;
-}
-
-// the block key map of every layer of one role over all ranks: twice the blocks all ranks can hold
-static size_t map_capacity(size_t max_blocks, int nranks) {
-  size_t cap = 1024;
-  while (cap < 2 * max_blocks * static_cast<size_t>(nranks)) cap <<= 1;
-  return cap;
 }
 
 // All ranks call this with their own layer of one role (collective): IPC handles all-gathered, the
@@ -562,27 +518,19 @@ static int32_t bind(cg_context* ctx, const cg_layer* layer, Binding& b, const ch
   return CG_OK;
 }
 
-// the partial layer of cg_gather_global, with the holder map's scratch sized for it
+// the partial layer of cg_gather_global, with the holder map's scratch sized for it (a key map
+// over every rank's blocks)
 static int32_t bind_partial(cg_context* ctx, const cg_layer* partial) {
   cg_comm* c = ctx->comm;
-  const size_t list_cap = partial->max_blocks * static_cast<size_t>(c->nranks);
-  const size_t hcap = map_capacity(partial->max_blocks, c->nranks);
-  if (hcap != c->hcap || list_cap != c->list_cap) {
-    void* bufs[] = {c->hkeys, c->hmask, c->hbase, c->mine, c->slots, c->counters};
-    for (void* p : bufs)
-      if (p) cudaFree(p);
-    c->hkeys = c->hmask = nullptr;
-    c->hbase = c->mine = c->slots = c->counters = nullptr;
-    c->hcap = c->list_cap = 0;
-    CG_CUDA(cudaMalloc(&c->hkeys, hcap * sizeof(unsigned long long)));
-    CG_CUDA(cudaMalloc(&c->hmask, hcap * sizeof(unsigned long long)));
-    CG_CUDA(cudaMalloc(&c->hbase, hcap * sizeof(uint32_t)));
-    CG_CUDA(cudaMalloc(&c->mine, list_cap * sizeof(uint32_t)));
-    CG_CUDA(cudaMalloc(&c->slots, list_cap * sizeof(uint32_t)));
-    CG_CUDA(cudaMalloc(&c->counters, 4 * sizeof(uint32_t)));
-    c->hcap = hcap;
-    c->list_cap = list_cap;
-  }
+  release(c, c->partial);  // nothing uses the binding until bind() has made it again
+  c->list_cap = partial->max_blocks * static_cast<size_t>(c->nranks);
+  c->hcap = key_set_capacity(c->list_cap, 1024);
+  CG_CUDA(c->hkeys.reserve(c->hcap * sizeof(unsigned long long)));
+  CG_CUDA(c->hmask.reserve(c->hcap * sizeof(unsigned long long)));
+  CG_CUDA(c->hbase.reserve(c->hcap * sizeof(uint32_t)));
+  CG_CUDA(c->mine.reserve(c->list_cap * sizeof(uint32_t)));
+  CG_CUDA(c->slots.reserve(c->list_cap * sizeof(uint32_t)));
+  CG_CUDA(c->counters.reserve(4 * sizeof(uint32_t)));
   // the dirty keys of cg_reproject_submaps_sharded: the partial layer's blocks before and after a
   // call, so at most twice its pool
   const uint32_t dirty_cap = static_cast<uint32_t>(std::min<size_t>(2 * partial->max_blocks, 0xFFFFFFF0u));
@@ -599,21 +547,12 @@ static int32_t bind_partial(cg_context* ctx, const cg_layer* partial) {
 // the owned layer of cg_layer_mesh_sharded, with the key map's scratch sized for it
 static int32_t bind_owned(cg_context* ctx, const cg_layer* owned) {
   cg_comm* c = ctx->comm;
-  const size_t mcap = map_capacity(owned->max_blocks, c->nranks);
-  if (mcap != c->mcap) {
-    void* bufs[] = {c->mkeys, c->mmask, c->mplanes, c->mcounters};
-    for (void* p : bufs)
-      if (p) cudaFree(p);
-    c->mkeys = c->mmask = nullptr;
-    c->mplanes = nullptr;
-    c->mcounters = nullptr;
-    c->mcap = 0;
-    CG_CUDA(cudaMalloc(&c->mkeys, mcap * sizeof(unsigned long long)));
-    CG_CUDA(cudaMalloc(&c->mmask, mcap * sizeof(unsigned long long)));
-    CG_CUDA(cudaMalloc(&c->mplanes, mcap * sizeof(const float*)));
-    CG_CUDA(cudaMalloc(&c->mcounters, 4 * sizeof(uint32_t)));
-    c->mcap = mcap;
-  }
+  release(c, c->owned);  // nothing uses the binding until bind() has made it again
+  c->mcap = key_set_capacity(owned->max_blocks * static_cast<size_t>(c->nranks), 1024);
+  CG_CUDA(c->mkeys.reserve(c->mcap * sizeof(unsigned long long)));
+  CG_CUDA(c->mmask.reserve(c->mcap * sizeof(unsigned long long)));
+  CG_CUDA(c->mplanes.reserve(c->mcap * sizeof(const float*)));
+  CG_CUDA(c->mcounters.reserve(4 * sizeof(uint32_t)));
   return bind(ctx, owned, c->owned, "cg_layer_mesh_sharded");
 }
 
@@ -625,18 +564,19 @@ int32_t sharded_mesh_open(const cg_layer* owned, unsigned long long* dup_key, Sh
   if (c->owned.serial != owned->serial && (rc = bind_owned(ctx, owned))) return rc;
   ctx->own_launches += 2;
   k_publish_blocks<<<1, 1, 0, s>>>(c->owned.shared, static_cast<int>(owned->num_blocks));
-  CG_CUDA(cudaMemsetAsync(c->mkeys, 0xFF, c->mcap * sizeof(unsigned long long), s));
-  CG_CUDA(cudaMemsetAsync(c->mmask, 0, c->mcap * sizeof(unsigned long long), s));
-  CG_CUDA(cudaMemsetAsync(c->mcounters, 0, 4 * sizeof(uint32_t), s));
+  CG_CUDA(cudaMemsetAsync(c->mkeys.p, 0xFF, c->mcap * sizeof(unsigned long long), s));
+  CG_CUDA(cudaMemsetAsync(c->mmask.p, 0, c->mcap * sizeof(unsigned long long), s));
+  CG_CUDA(cudaMemsetAsync(c->mcounters.p, 0, 4 * sizeof(uint32_t), s));
   CG_CUDA(cudaMemsetAsync(dup_key, 0xFF, sizeof(unsigned long long), s));
   // every rank's owned layer is complete and its block count published (stream-ordered)
   if ((rc = barrier(ctx))) return rc;
-  const uint32_t cap_mask = static_cast<uint32_t>(c->mcap - 1);
+  const KeySet map{c->mkeys.as<unsigned long long>(), static_cast<uint32_t>(c->mcap - 1)};
   const dim3 per_rank(static_cast<unsigned>(ctx->num_sms), static_cast<unsigned>(c->nranks));
-  k_build_holders<<<per_rank, 256, 0, s>>>(c->owned.d_peers, c->mkeys, c->mmask, cap_mask,
-                                           c->mcounters, c->mplanes, dup_key, nullptr, 0);
+  k_build_holders<<<per_rank, 256, 0, s>>>(c->owned.d_peers, map, c->mmask.as<unsigned long long>(),
+                                           c->mcounters.as<uint32_t>(), c->mplanes.as<const float*>(),
+                                           dup_key, nullptr, 0);
   CG_CUDA(cudaGetLastError());
-  *out = ShardedBlocks{c->mkeys, c->mplanes, cap_mask};
+  *out = ShardedBlocks{KeyLookup{map.keys, map.mask}, c->mplanes.as<const float*>()};
   return CG_OK;
 }
 
@@ -647,46 +587,48 @@ int32_t sharded_mesh_close(cg_context* ctx) { return barrier(ctx); }
 static int32_t reset_holders(cg_context* ctx) {
   cg_comm* c = ctx->comm;
   cudaStream_t s = ctx->stream;
-  CG_CUDA(cudaMemsetAsync(c->hkeys, 0xFF, c->hcap * sizeof(unsigned long long), s));
-  CG_CUDA(cudaMemsetAsync(c->hmask, 0, c->hcap * sizeof(unsigned long long), s));
-  CG_CUDA(cudaMemsetAsync(c->counters, 0, 4 * sizeof(uint32_t), s));
+  CG_CUDA(cudaMemsetAsync(c->hkeys.p, 0xFF, c->hcap * sizeof(unsigned long long), s));
+  CG_CUDA(cudaMemsetAsync(c->hmask.p, 0, c->hcap * sizeof(unsigned long long), s));
+  CG_CUDA(cudaMemsetAsync(c->counters.p, 0, 4 * sizeof(uint32_t), s));
   CG_CUDA(cudaMemsetAsync(&ctx->d_counters->blocks_out, 0, sizeof(unsigned long long), s));
   return CG_OK;
 }
 static uint32_t fold_list_cap(const cg_comm* c) {
   return static_cast<uint32_t>(std::min<size_t>(c->list_cap, 0xFFFFFFF0u));
 }
-static void list_holders(cg_context* ctx, const unsigned long long* filter, uint32_t filter_mask) {
+static void list_holders(cg_context* ctx, KeyLookup filter) {
   cg_comm* c = ctx->comm;
   cudaStream_t s = ctx->stream;
-  const uint32_t hmask_cap = static_cast<uint32_t>(c->hcap - 1);
   const uint32_t list_cap = fold_list_cap(c);
+  const KeySet map{c->hkeys.as<unsigned long long>(), static_cast<uint32_t>(c->hcap - 1)};
+  unsigned long long* hmask = c->hmask.as<unsigned long long>();
+  uint32_t* hbase = c->hbase.as<uint32_t>();
+  uint32_t* counters = c->counters.as<uint32_t>();
   ctx->own_launches += 3;
   const dim3 per_rank(static_cast<unsigned>(ctx->num_sms), static_cast<unsigned>(c->nranks));
-  k_build_holders<<<per_rank, 256, 0, s>>>(c->partial.d_peers, c->hkeys, c->hmask, hmask_cap,
-                                           c->counters, nullptr, nullptr, filter, filter_mask);
-  k_list_owned<<<ctx->num_sms * 4, 256, 0, s>>>(c->hkeys, c->hmask, static_cast<uint32_t>(c->hcap),
-                                                c->rank, c->hbase, c->mine, list_cap, c->counters);
-  k_holder_slots<<<per_rank, 256, 0, s>>>(c->partial.d_peers, c->hkeys, c->hmask, c->hbase, hmask_cap,
-                                          c->rank, c->slots, list_cap, filter, filter_mask);
+  k_build_holders<<<per_rank, 256, 0, s>>>(c->partial.d_peers, map, hmask, counters, nullptr,
+                                           nullptr, filter.keys, filter.mask);
+  k_list_owned<<<ctx->num_sms * 4, 256, 0, s>>>(map.keys, hmask, static_cast<uint32_t>(c->hcap),
+                                                c->rank, hbase, c->mine.as<uint32_t>(), list_cap,
+                                                counters);
+  k_holder_slots<<<per_rank, 256, 0, s>>>(c->partial.d_peers, map.keys, hmask, hbase, map.mask,
+                                          c->rank, c->slots.as<uint32_t>(), list_cap, filter.keys,
+                                          filter.mask);
 }
 // every block the holder map gives this rank, folded into `owned` (blocks the layer holds are
 // read as they are: fresh, or reset by cg_reproject_submaps_sharded)
 static int32_t fold_owned(cg_context* ctx, cg_layer* owned) {
   cg_comm* c = ctx->comm;
   cudaStream_t s = ctx->stream;
-  const size_t smem = 3 * kVoxelsPerBlock * sizeof(uint32_t);
-  static bool attr_set[64] = {};
-  if (ctx->device < 0 || ctx->device >= 64 || !attr_set[ctx->device]) {
-    CG_CUDA(cudaFuncSetAttribute(k_fold_owned, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                 static_cast<int>(smem)));
-    if (ctx->device >= 0 && ctx->device < 64) attr_set[ctx->device] = true;
-  }
+  constexpr size_t smem = 3 * kVoxelsPerBlock * sizeof(uint32_t);
+  CG_CUDA(allow_dynamic_smem<k_fold_owned>(ctx->device, smem));
   ctx->own_launches += 2;
   k_fold_owned<<<ctx->num_sms * 4, kFoldThreads, smem, s>>>(
-      owned->v, c->partial.d_peers, c->hkeys, c->hmask, c->hbase, c->mine, c->slots, c->counters,
-      fold_list_cap(c), static_cast<int>(owned->num_blocks), &ctx->d_counters->blocks_out);
-  k_comm_overflow<<<1, 1, 0, s>>>(c->counters, owned->v.err);
+      owned->v, c->partial.d_peers, c->hkeys.as<unsigned long long>(),
+      c->hmask.as<unsigned long long>(), c->hbase.as<uint32_t>(), c->mine.as<uint32_t>(),
+      c->slots.as<uint32_t>(), c->counters.as<uint32_t>(), fold_list_cap(c),
+      static_cast<int>(owned->num_blocks), &ctx->d_counters->blocks_out);
+  k_comm_overflow<<<1, 1, 0, s>>>(c->counters.as<uint32_t>(), owned->v.err);
   CG_CUDA(cudaGetLastError());
   return CG_OK;
 }
@@ -800,7 +742,7 @@ int32_t cg_gather_global(const cg_layer* partial, cg_layer* owned, uint64_t* blo
   // every rank's partial layer is complete and its block count published (stream-ordered)
   if ((rc = barrier(ctx))) return rc;
   mark();
-  list_holders(ctx, nullptr, 0);
+  list_holders(ctx, KeyLookup{});
   mark();
   if ((rc = fold_owned(ctx, owned))) return rc;
   mark();
@@ -926,7 +868,7 @@ int32_t cg_reproject_submaps_sharded(const cg_layer* const* submaps, size_t n, s
   }
   // D: the union of every rank's published keys, identical on every rank
   const int R = c->nranks;
-  const size_t dcap = map_capacity(2 * partial->max_blocks, R);
+  const size_t dcap = key_set_capacity(2 * partial->max_blocks * static_cast<size_t>(R), 1024);
   uint32_t h[4] = {0, 0, 0, 0};
   rc = [&]() -> int32_t {
     CG_CUDA(c->dset.reserve(dcap * sizeof(unsigned long long)));
@@ -936,8 +878,8 @@ int32_t cg_reproject_submaps_sharded(const cg_layer* const* submaps, size_t n, s
     CG_CUDA(cudaMemsetAsync(c->dcounters, 0, 4 * sizeof(uint32_t), s));
     ctx->own_launches += 1;
     k_union_dirty<<<dim3(static_cast<unsigned>(ctx->num_sms), static_cast<unsigned>(R)), 256, 0, s>>>(
-        c->partial.d_peers, c->partial.dirty_cap, c->dset.as<unsigned long long>(),
-        static_cast<uint32_t>(dcap - 1), c->dcounters);
+        c->partial.d_peers, c->partial.dirty_cap,
+        KeySet{c->dset.as<unsigned long long>(), static_cast<uint32_t>(dcap - 1)}, c->dcounters);
     CG_CUDA(cudaMemcpyAsync(h, c->dcounters, sizeof(h), cudaMemcpyDeviceToHost, s));
     CG_CUDA(cudaStreamSynchronize(s));
     return CG_OK;
@@ -978,14 +920,13 @@ int32_t cg_reproject_submaps_sharded(const cg_layer* const* submaps, size_t n, s
   CG_CUDA(ctx->stage_b.reserve((static_cast<size_t>(owned->num_blocks) + 2) * sizeof(uint32_t)));
   uint32_t* counts = ctx->stage_b.as<uint32_t>();  // [0] blocks of D the owned layer holds
   uint32_t* slots = counts + 2;
-  const unsigned long long* dset = c->dset.as<unsigned long long>();
   rc = [&]() -> int32_t {
     if (h[0] == 0) return CG_OK;
-    int32_t r = reset_dirty_blocks(owned, reinterpret_cast<const uint64_t*>(dset),
-                                   static_cast<uint32_t>(dcap), slots, counts);
+    int32_t r = reset_dirty_blocks(owned, c->dset.as<uint64_t>(), static_cast<uint32_t>(dcap), slots,
+                                   counts);
     if (r) return r;
     if ((r = reset_holders(ctx))) return r;
-    list_holders(ctx, dset, static_cast<uint32_t>(dcap - 1));
+    list_holders(ctx, KeyLookup{c->dset.as<unsigned long long>(), static_cast<uint32_t>(dcap - 1)});
     return fold_owned(ctx, owned);
   }();
   // nobody clears or refills its partial layer while a peer still reads it

@@ -345,17 +345,6 @@ k_esdf_free(const uint64_t* __restrict__ keys, uint32_t n, const float* __restri
   }
 }
 
-__global__ void k_esdf_unpack_idx(const uint64_t* __restrict__ keys, uint32_t n,
-                                  int32_t* __restrict__ idx) {
-  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  int x, y, z;
-  unpack_block_key(keys[i], x, y, z);
-  idx[3 * i] = x;
-  idx[3 * i + 1] = y;
-  idx[3 * i + 2] = z;
-}
-
 // ------------------------------------------------------------------ incremental update
 // Counters of one update (uint32 words after the batch's counters): see cg_layer_esdf_update.
 enum UpdateCount { kUcSources = 0, kUcRemoved, kUcMoved, kUcChanged, kUcRegion, kUcWords = 8 };
@@ -666,8 +655,8 @@ int32_t cg_layer_esdf_batch(const cg_layer* L, const cg_esdf_config* cfg, cg_esd
                                             ctx->esdf_dist.as<float>(), ctx->esdf_fixed.as<uint32_t>(),
                                             ctx->esdf_slot_to_b.as<int32_t>(),
                                             ctx->esdf_dirty.as<uint8_t>(), counters);
-  k_esdf_unpack_idx<<<grid_for(n, 256), 256, 0, s>>>(keys, static_cast<uint32_t>(n),
-                                                     ctx->esdf_index.as<int32_t>());
+  k_unpack_idx<<<grid_for(n, 256), 256, 0, s>>>(keys, static_cast<uint32_t>(n),
+                                                ctx->esdf_index.as<int32_t>());
   uint64_t sweeps = 0, passes = 0;
   rc = run_sweeps(ctx, L, keys, n, P, nullptr, &sweeps, &passes, "cg_layer_esdf_batch");
   if (rc) return rc;
@@ -773,9 +762,9 @@ int32_t cg_layer_esdf_update(const cg_layer* L, const cg_esdf_config* cfg, cg_es
     CG_CUDA(ctx->esdf_index.reserve(n * 3 * sizeof(int32_t)));
     CG_CUDA(cudaMemcpyAsync(ctx->esdf_keys.p, keys, n * sizeof(uint64_t), cudaMemcpyDeviceToDevice, s));
     ctx->own_launches += 1;
-    k_esdf_unpack_idx<<<grid_for(n, 256), 256, 0, s>>>(ctx->esdf_keys.as<uint64_t>(),
-                                                       static_cast<uint32_t>(n),
-                                                       ctx->esdf_index.as<int32_t>());
+    k_unpack_idx<<<grid_for(n, 256), 256, 0, s>>>(ctx->esdf_keys.as<uint64_t>(),
+                                                  static_cast<uint32_t>(n),
+                                                  ctx->esdf_index.as<int32_t>());
   }
   // the sweeps read the layer's hash and these keys; the slots stay sort_blocks' (this call only)
   keys = ctx->esdf_keys.as<uint64_t>();

@@ -23,15 +23,11 @@ struct PackedHeader {
 static_assert(sizeof(PackedHeader) == 16, "record header");
 constexpr size_t kRecordWords = CG_PACKED_BLOCK_BYTES / 4;
 
-__host__ __device__ __forceinline__ uint32_t owner_of(uint64_t key, uint32_t nranks) {
-  return (hash_key(key ^ 0x9E3779B97F4A7C15ULL) >> 7) % nranks;
-}
-
 __global__ void k_owner_keys(const uint64_t* sorted_keys, int n, uint32_t nranks, uint32_t* owners,
                              unsigned long long* counts) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
-  const uint32_t o = owner_of(sorted_keys[i], nranks);
+  const uint32_t o = owner_pick(sorted_keys[i], nranks);
   owners[i] = o;
   atomicAdd(&counts[o], 1ull);
 }
@@ -109,11 +105,6 @@ __global__ void k_merge_records(LayerView B, const uint32_t* recs, const uint64_
   }
 }
 
-__global__ void k_iota32(uint32_t* v, int n) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n) v[i] = i;
-}
-
 }  // namespace cg
 
 using namespace cg;
@@ -122,7 +113,7 @@ extern "C" {
 
 int32_t cg_block_owner(int32_t bx, int32_t by, int32_t bz, int32_t nranks) {
   if (nranks <= 0) return -1;
-  return static_cast<int32_t>(owner_of(pack_block_key(bx, by, bz), static_cast<uint32_t>(nranks)));
+  return static_cast<int32_t>(owner_pick(pack_block_key(bx, by, bz), static_cast<uint32_t>(nranks)));
 }
 
 int32_t cg_layer_pack_by_owner(const cg_layer* L, int32_t nranks, void* d_packed, size_t capacity,
@@ -149,7 +140,7 @@ int32_t cg_layer_pack_by_owner(const cg_layer* L, int32_t nranks, void* d_packed
   CG_CUDA(ctx->stage_b.reserve(counts_off + nranks * sizeof(unsigned long long)));
   uint32_t* iota = ctx->val_a.as<uint32_t>();
   uint32_t* slots_sorted = ctx->val_b.as<uint32_t>();
-  k_iota32<<<grid_for(n, 256), 256, 0, s>>>(iota, n);
+  k_iota<<<grid_for(n, 256), 256, 0, s>>>(iota, n);
   size_t tmp1 = 0, tmp2 = 0;
   cub::DeviceRadixSort::SortPairs(nullptr, tmp1, L->v.block_keys, ctx->key_b.as<uint64_t>(), iota,
                                   slots_sorted, n, 0, 63, s);
@@ -168,7 +159,7 @@ int32_t cg_layer_pack_by_owner(const cg_layer* L, int32_t nranks, void* d_packed
   CG_CUDA(cudaMemsetAsync(d_counts, 0, nranks * sizeof(unsigned long long), s));
   k_owner_keys<<<grid_for(n, 256), 256, 0, s>>>(ctx->key_b.as<uint64_t>(), n,
                                                 static_cast<uint32_t>(nranks), owners, d_counts);
-  k_iota32<<<grid_for(n, 256), 256, 0, s>>>(pos_in, n);
+  k_iota<<<grid_for(n, 256), 256, 0, s>>>(pos_in, n);
   CG_CUDA(cub::DeviceRadixSort::SortPairs(ctx->cub_tmp.p, tmp2, owners, owners_sorted, pos_in,
                                           order, n, 0, 12, s));
   k_pack_records<<<n, 256, 0, s>>>(L->v, order, slots_sorted, n, static_cast<uint32_t*>(d_packed));

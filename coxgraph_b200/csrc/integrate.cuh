@@ -33,8 +33,7 @@ __device__ __forceinline__ int size_class(uint32_t n) {  // descending: class 0 
 // (frame, voxel relative to the frame's sensor voxel); the front half builds it (k_grazing_build),
 // the walk probes it.
 struct GrazingSet {
-  const unsigned long long* keys;      // open addressing, kEmptyKey = free
-  uint32_t mask;
+  KeyLookup set;
   const unsigned long long* ray_key;   // per ray (= bundle): its own packed bundle voxel
 };
 __device__ __forceinline__ unsigned long long grazing_key(uint32_t frame, int rx, int ry, int rz) {
@@ -42,15 +41,6 @@ __device__ __forceinline__ unsigned long long grazing_key(uint32_t frame, int rx
          (static_cast<unsigned long long>(rz & 0x3FFF) << 28) |
          (static_cast<unsigned long long>(ry & 0x3FFF) << 14) |
          static_cast<unsigned long long>(rx & 0x3FFF);
-}
-__device__ __forceinline__ bool grazing_contains(const GrazingSet& G, unsigned long long key) {
-  uint32_t h = hash_key(key) & G.mask;
-  for (;;) {
-    const unsigned long long k = G.keys[h];
-    if (k == key) return true;
-    if (k == kEmptyKey) return false;
-    h = (h + 1) & G.mask;
-  }
 }
 
 // ------------------------------------------------------------------ host

@@ -267,7 +267,7 @@ k_walk_segments(IntegratorParams P, const float* __restrict__ poses, const Ray* 
           bool skip = false;
           if (abs(rx) < 8192 && abs(ry) < 8192 && abs(rz) < 8192) {
             const unsigned long long gk = grazing_key(g_frame, rx, ry, rz);
-            skip = gk != own_key && grazing_contains(G, gk);
+            skip = gk != own_key && G.set.contains(gk);
           }
           if (skip) {
             // the reference "continue"s before it even looks the voxel up: no allocation, no
@@ -1119,7 +1119,7 @@ int32_t run_back_half(cg_context* ctx, const FrontBufs& fb, cg_layer* L, const I
     CG_CUDA(fill_bytes(ctx->d_walk_counters, 0, 2 * sizeof(uint32_t), s));
     {
       StageScope sc(ctx, kStageWalkSegments, 2);
-      const GrazingSet gz{fb.grazing_keys.as<unsigned long long>(), fb.grazing_mask,
+      const GrazingSet gz{KeyLookup{fb.grazing_set.keys, fb.grazing_set.mask},
                           fb.grazing_ray_key.as<unsigned long long>()};
       if (P.anti_grazing)
         k_walk_segments<true><<<walk_grid, kWalkThreads, 0, s>>>(

@@ -766,8 +766,7 @@ __global__ void k_grazing_build(KeyLayout kl, const uint64_t* __restrict__ keys,
                                 const uint32_t* __restrict__ heads,
                                 const uint32_t* __restrict__ num_heads,
                                 const uint32_t* __restrict__ ray_id,
-                                unsigned long long* set_keys, uint32_t set_mask,
-                                unsigned long long* __restrict__ ray_key) {
+                                KeySet set, unsigned long long* __restrict__ ray_key) {
   const uint32_t nb = *num_heads;
   for (uint32_t b = blockIdx.x * blockDim.x + threadIdx.x; b < nb; b += gridDim.x * blockDim.x) {
     const BundleInfo bi = bundle_info(keys, total, heads, nb, b);
@@ -776,16 +775,7 @@ __global__ void k_grazing_build(KeyLayout kl, const uint64_t* __restrict__ keys,
     const unsigned long long gk = grazing_key(kl.frame(bi.key), rx, ry, rz);
     ray_key[ray_id[b]] = gk;
     if (kl.clearing(bi.key)) continue;  // only non-clearing bundles are in the set
-    uint32_t h = hash_key(gk) & set_mask;
-    for (;;) {
-      const unsigned long long k = set_keys[h];
-      if (k == gk) break;
-      if (k == kEmptyKey) {
-        const unsigned long long old = atomicCAS(&set_keys[h], kEmptyKey, gk);
-        if (old == kEmptyKey || old == gk) break;
-      }
-      h = (h + 1) & set_mask;
-    }
+    set.insert(gk);
   }
 }
 
@@ -947,16 +937,14 @@ int32_t front_enqueue(cg_context* ctx, FrontBufs& fb, cudaStream_t s, int32_t* d
                                           fb.ray_count.as<unsigned long long>());
     }
     if (P.anti_grazing) {  // set of the scan's bundle voxels (at most one per point)
-      size_t gcap = 1024;
-      while (gcap < 2 * total) gcap <<= 1;
+      const size_t gcap = key_set_capacity(total, 1024);
       CG_CUDA(fb.grazing_keys.reserve(gcap * sizeof(unsigned long long)));
       CG_CUDA(fb.grazing_ray_key.reserve(upper * sizeof(unsigned long long)));
-      fb.grazing_mask = static_cast<uint32_t>(gcap - 1);
+      fb.grazing_set = KeySet{fb.grazing_keys.as<unsigned long long>(), static_cast<uint32_t>(gcap - 1)};
       CG_CUDA(fill_bytes(fb.grazing_keys.p, 0xFF, gcap * sizeof(unsigned long long), s));
       k_grazing_build<<<bgrid, 256, 0, s>>>(kl, dk.Current(), static_cast<uint32_t>(total),
                                             fb.scan.as<uint32_t>(), d_num, fb.ray_id.as<uint32_t>(),
-                                            fb.grazing_keys.as<unsigned long long>(),
-                                            fb.grazing_mask,
+                                            fb.grazing_set,
                                             fb.grazing_ray_key.as<unsigned long long>());
     }
   } else {

@@ -232,14 +232,15 @@ __global__ void k_probe_lengths(LayerView L, int n, unsigned long long* out) {
   }
 }
 
-__global__ void k_unpack_idx(const uint64_t* sorted_keys, int n, int32_t* out_idx) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+__global__ void k_unpack_idx(const uint64_t* __restrict__ keys, uint32_t n,
+                             int32_t* __restrict__ idx) {
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   int x, y, z;
-  unpack_block_key(sorted_keys[i], x, y, z);
-  out_idx[3 * i] = x;
-  out_idx[3 * i + 1] = y;
-  out_idx[3 * i + 2] = z;
+  unpack_block_key(keys[i], x, y, z);
+  idx[3 * i] = x;
+  idx[3 * i + 1] = y;
+  idx[3 * i + 2] = z;
 }
 
 __global__ void k_upload_insert(LayerView L, const int32_t* idx, int n, int32_t* entries) {
@@ -770,7 +771,7 @@ int32_t cg_layer_block_indices(const cg_layer* L, size_t capacity, int32_t* idx,
   int32_t rc = sort_blocks(L, &keys, &slots);
   if (rc) return rc;
   CG_CUDA(ctx->stage_b.reserve(n * 3 * sizeof(int32_t)));
-  k_unpack_idx<<<grid_for(n, 256), 256, 0, ctx->stream>>>(keys, static_cast<int>(n),
+  k_unpack_idx<<<grid_for(n, 256), 256, 0, ctx->stream>>>(keys, static_cast<uint32_t>(n),
                                                           ctx->stage_b.as<int32_t>());
   CG_CUDA(cudaMemcpyAsync(idx, ctx->stage_b.p, n * 3 * sizeof(int32_t), cudaMemcpyDeviceToHost,
                           ctx->stream));

@@ -27,18 +27,20 @@ namespace cg {
 
 constexpr int kTab = 4;  // cached neighbourhood of source block slots: kTab^3
 
-__global__ void k_mark_candidates(LayerView A, int num_a, Xform T_B_A, float block_size_out,
-                                  uint64_t* set_keys, uint32_t set_mask, uint64_t* list,
-                                  CallCounters* counters, int32_t* err) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= num_a) return;
+// transformLayer's forward pass for one source block (`key`, blocks of block_size_in): visit(k)
+// for every destination block k (blocks of block_size_out) the block's bounding sphere can reach
+// under T_B_A, one grid sample at a time (a block may come more than once); a sample outside the
+// key range raises kErrOutOfRange instead
+template <class Visit>
+__device__ __forceinline__ void forward_pass(uint64_t key, float block_size_in, const Xform& T_B_A,
+                                             float block_size_out, int32_t* err, Visit visit) {
   int bx, by, bz;
-  unpack_block_key(A.block_keys[i], bx, by, bz);
-  const V3 c_in = V3{center_coord(bx, A.block_size), center_coord(by, A.block_size),
-                     center_coord(bz, A.block_size)};
+  unpack_block_key(key, bx, by, bz);
+  const V3 c_in = V3{center_coord(bx, block_size_in), center_coord(by, block_size_in),
+                     center_coord(bz, block_size_in)};
   const V3 c = apply(T_B_A, c_in);
   const float kDiag = 1.7320508075688772f;  // kUnitCubeDiagonalLength
-  const float offset = kDiag * A.block_size * 0.5f;
+  const float offset = kDiag * block_size_in * 0.5f;
   const float inv_out = 1.0f / block_size_out;
   constexpr int lim = kVoxIdxOffset / kVps;
   for (float x = c.x - offset; x < c.x + offset; x += block_size_out)
@@ -50,24 +52,19 @@ __global__ void k_mark_candidates(LayerView A, int num_a, Xform T_B_A, float blo
           atomicOr(err, kErrOutOfRange);
           continue;
         }
-        const uint64_t key = pack_block_key(ix, iy, iz);
-        uint32_t h = hash_key(key) & set_mask;
-        for (;;) {
-          const uint64_t k = set_keys[h];
-          if (k == key) break;
-          if (k == kEmptyKey) {
-            const unsigned long long old = atomicCAS(
-                reinterpret_cast<unsigned long long*>(&set_keys[h]), kEmptyKey, key);
-            if (old == kEmptyKey) {
-              const unsigned long long pos = atomicAdd(&counters->candidates, 1ull);
-              list[pos] = key;
-              break;
-            }
-            if (old == key) break;
-          }
-          h = (h + 1) & set_mask;
-        }
+        visit(pack_block_key(ix, iy, iz));
       }
+}
+
+__global__ void k_mark_candidates(LayerView A, int num_a, Xform T_B_A, float block_size_out,
+                                  KeySet set, uint64_t* list, CallCounters* counters, int32_t* err) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= num_a) return;
+  forward_pass(A.block_keys[i], A.block_size, T_B_A, block_size_out, err, [&](uint64_t key) {
+    bool inserted;
+    set.insert(key, &inserted);
+    if (inserted) list[atomicAdd(&counters->candidates, 1ull)] = key;
+  });
 }
 
 struct SlotTable {
@@ -265,55 +262,70 @@ __device__ __forceinline__ bool resample_voxel(const LayerView& A, const SlotTab
 constexpr int kMergeThreads = 512;
 constexpr int kVoxPerThread = kVoxelsPerBlock / kMergeThreads;
 
+// dynamic shared memory of k_resample_merge / k_project_batch: one resampled block, planar
+struct ResampleTile {
+  float d[kVoxelsPerBlock];
+  float w[kVoxelsPerBlock];
+  uint32_t c[kVoxelsPerBlock];
+  SlotTable tab;
+};
+
+// Resamples destination block `key` of B from A (R8 / R9; T_A_B: B's frame -> A's) into t; every
+// thread of the CTA calls it after a barrier that ends the previous use of t.  Returns, on every
+// thread, whether any voxel carried data (transformLayer keeps only such blocks).
+__device__ __forceinline__ bool resample_block(const LayerView& A, const LayerView& B,
+                                               const Xform& T_A_B, uint64_t key, ResampleTile& t) {
+  int bx, by, bz;
+  unpack_block_key(key, bx, by, bz);
+  const V3 org_out = V3{static_cast<float>(bx) * B.block_size, static_cast<float>(by) * B.block_size,
+                        static_cast<float>(bz) * B.block_size};
+  // the source blocks around the destination block's reach
+  if (threadIdx.x < kTab * kTab * kTab) {
+    const V3 ctr = V3{center_coord(bx, B.block_size), center_coord(by, B.block_size),
+                      center_coord(bz, B.block_size)};
+    const V3 pc = apply(T_A_B, ctr);
+    const float reach = 0.8660254f * B.block_size + A.voxel_size;
+    const int ax = __float2int_rd((pc.x - reach) * A.block_size_inv);
+    const int ay = __float2int_rd((pc.y - reach) * A.block_size_inv);
+    const int az = __float2int_rd((pc.z - reach) * A.block_size_inv);
+    const int i = threadIdx.x;
+    const int dx = i % kTab, dy = (i / kTab) % kTab, dz = i / (kTab * kTab);
+    t.tab.slot[i] = A.find_slot(pack_block_key(ax + dx, ay + dy, az + dz));
+    if (i == 0) {
+      t.tab.ax = ax;
+      t.tab.ay = ay;
+      t.tab.az = az;
+    }
+  }
+  __syncthreads();
+  bool any = false;
+#pragma unroll 1
+  for (int j = 0; j < kVoxPerThread; ++j) {
+    const int lin = threadIdx.x + j * kMergeThreads;
+    const int vx = lin & 15, vy = (lin >> 4) & 15, vz = lin >> 8;
+    const V3 center_out =
+        org_out + V3{center_coord(vx, B.voxel_size), center_coord(vy, B.voxel_size),
+                     center_coord(vz, B.voxel_size)};
+    const V3 p = apply(T_A_B, center_out);
+    VoxelState v;
+    any |= resample_voxel(A, t.tab, p, v);
+    t.d[lin] = v.d;
+    t.w[lin] = v.w;
+    t.c[lin] = v.c;
+  }
+  return __syncthreads_or(any ? 1 : 0) != 0;
+}
+
 __global__ void __launch_bounds__(kMergeThreads)
 k_resample_merge(LayerView A, LayerView B, Xform T_A_B, const uint64_t* __restrict__ cand,
                  CallCounters* counters) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
-  float* s_d = reinterpret_cast<float*>(smem_raw);                 // resampled block, planar
-  float* s_w = s_d + kVoxelsPerBlock;
-  uint32_t* s_c = reinterpret_cast<uint32_t*>(s_w + kVoxelsPerBlock);
-  SlotTable& tab = *reinterpret_cast<SlotTable*>(s_c + kVoxelsPerBlock);
+  ResampleTile& t = *reinterpret_cast<ResampleTile*>(smem_raw);
   __shared__ int s_slot;
   const unsigned long long num_cand = counters->candidates;
   for (unsigned long long c = blockIdx.x; c < num_cand; c += gridDim.x) {
-    int bx, by, bz;
-    unpack_block_key(cand[c], bx, by, bz);
-    const V3 org_out = V3{static_cast<float>(bx) * B.block_size, static_cast<float>(by) * B.block_size,
-                          static_cast<float>(bz) * B.block_size};
-    __syncthreads();  // previous iteration done with tab / s_slot
-    if (threadIdx.x == 0) {
-      const V3 ctr = V3{center_coord(bx, B.block_size), center_coord(by, B.block_size),
-                        center_coord(bz, B.block_size)};
-      const V3 pc = apply(T_A_B, ctr);
-      const float reach = 0.8660254f * B.block_size + A.voxel_size;
-      tab.ax = __float2int_rd((pc.x - reach) * A.block_size_inv);
-      tab.ay = __float2int_rd((pc.y - reach) * A.block_size_inv);
-      tab.az = __float2int_rd((pc.z - reach) * A.block_size_inv);
-    }
-    __syncthreads();
-    if (threadIdx.x < kTab * kTab * kTab) {
-      const int t = threadIdx.x;
-      const int dx = t % kTab, dy = (t / kTab) % kTab, dz = t / (kTab * kTab);
-      tab.slot[t] = A.find_slot(pack_block_key(tab.ax + dx, tab.ay + dy, tab.az + dz));
-    }
-    __syncthreads();
-    bool any = false;
-#pragma unroll 1
-    for (int j = 0; j < kVoxPerThread; ++j) {
-      const int lin = threadIdx.x + j * kMergeThreads;
-      const int vx = lin & 15, vy = (lin >> 4) & 15, vz = lin >> 8;
-      const V3 center_out =
-          org_out + V3{center_coord(vx, B.voxel_size), center_coord(vy, B.voxel_size),
-                       center_coord(vz, B.voxel_size)};
-      const V3 p = apply(T_A_B, center_out);
-      VoxelState t;
-      any |= resample_voxel(A, tab, p, t);
-      s_d[lin] = t.d;
-      s_w[lin] = t.w;
-      s_c[lin] = t.c;
-    }
-    const int has_data = __syncthreads_or(any ? 1 : 0);
-    if (!has_data) continue;  // block dropped from the transformed layer: nothing merged
+    __syncthreads();  // previous iteration done with t / s_slot
+    if (!resample_block(A, B, T_A_B, cand[c], t)) continue;  // dropped: nothing merged
     if (threadIdx.x == 0) {
       const int e = B.insert_entry(cand[c]);
       s_slot = B.hash_vals[e];  // written by this thread or by an earlier kernel
@@ -333,7 +345,7 @@ k_resample_merge(LayerView A, LayerView B, Xform T_A_B, const uint64_t* __restri
     for (int j = 0; j < kVoxPerThread; ++j) {
       const int lin = threadIdx.x + j * kMergeThreads;
       VoxelState b{dp[lin], wp[lin], cp[lin]};
-      merge_voxel(s_d[lin], s_w[lin], s_c[lin], b);
+      merge_voxel(t.d[lin], t.w[lin], t.c[lin], b);
       dp[lin] = b.d;
       wp[lin] = b.w;
       cp[lin] = b.c;
@@ -362,8 +374,7 @@ static int32_t enqueue_merge(const cg_layer* A, const float T_B_A[7], cg_layer* 
   // candidate set / list sized from the forward pass's own bound (a coarse source layer merged
   // into a fine one marks more than 27 destination blocks per source block)
   const size_t cand_bound = mark_bound(A, B, nA);
-  size_t cap = 1024;
-  while (cap < 2 * cand_bound) cap <<= 1;
+  const size_t cap = key_set_capacity(cand_bound, 1024);
   CG_CUDA(ctx->cand_keys.reserve(cap * sizeof(uint64_t)));
   CG_CUDA(ctx->cand_list.reserve(cand_bound * sizeof(uint64_t)));
   const Xform T = make_xform(T_B_A);
@@ -372,20 +383,15 @@ static int32_t enqueue_merge(const cg_layer* A, const float T_B_A[7], cg_layer* 
     CG_CUDA(cudaMemsetAsync(ctx->cand_keys.p, 0xFF, cap * sizeof(uint64_t), s));
     k_reset_merge_counters<<<1, 1, 0, s>>>(ctx->d_counters);
     k_mark_candidates<<<grid_for(nA, 128), 128, 0, s>>>(
-        A->v, static_cast<int>(nA), T, B->v.block_size, ctx->cand_keys.as<uint64_t>(),
-        static_cast<uint32_t>(cap - 1), ctx->cand_list.as<uint64_t>(), ctx->d_counters, B->v.err);
+        A->v, static_cast<int>(nA), T, B->v.block_size,
+        KeySet{ctx->cand_keys.as<unsigned long long>(), static_cast<uint32_t>(cap - 1)},
+        ctx->cand_list.as<uint64_t>(), ctx->d_counters, B->v.err);
   }
   const Xform Ti = inverse_xform_host(T);
   const unsigned grid = static_cast<unsigned>(
       std::min<size_t>(cand_bound, static_cast<size_t>(ctx->num_sms) * 4));
-  const size_t smem = 3 * kVoxelsPerBlock * sizeof(float) + sizeof(SlotTable);
-  // per device (a process may hold contexts on several GPUs): one flag per device ordinal
-  static bool attr_set[64] = {};
-  if (ctx->device < 0 || ctx->device >= 64 || !attr_set[ctx->device]) {
-    CG_CUDA(cudaFuncSetAttribute(k_resample_merge, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                 static_cast<int>(smem)));
-    if (ctx->device >= 0 && ctx->device < 64) attr_set[ctx->device] = true;
-  }
+  constexpr size_t smem = sizeof(ResampleTile);
+  CG_CUDA(allow_dynamic_smem<k_resample_merge>(ctx->device, smem));
   {
     StageScope sc(ctx, kStageMergeResample, 1);
     k_resample_merge<<<grid, kMergeThreads, smem, s>>>(A->v, B->v, Ti,
@@ -418,21 +424,13 @@ struct BatchSubmap {
 };
 constexpr int kBatchMax = 64;
 
-// `filter_keys` (optional): a hash set of destination blocks; blocks outside it are not marked
-// (incremental re-projection).  `map_mask` may be null: plain set insertion.
-__device__ __forceinline__ bool key_set_contains(const uint64_t* keys, uint32_t mask, uint64_t key) {
-  uint32_t h = hash_key(key) & mask;
-  for (;;) {
-    const uint64_t k = keys[h];
-    if (k == key) return true;
-    if (k == kEmptyKey) return false;
-    h = (h + 1) & mask;
-  }
-}
+// `filter_keys` (optional): a key set of filter_mask + 1 entries; the destination blocks outside it
+// are not marked (incremental re-projection).  `map_mask` may be null: plain set insertion.
 __global__ void k_mark_batch(const BatchSubmap* __restrict__ desc, int n, uint32_t total_blocks,
-                             float block_size_out, uint64_t* map_keys, unsigned long long* map_mask,
-                             uint32_t map_cap_mask, int32_t* err,
-                             const uint64_t* __restrict__ filter_keys, uint32_t filter_mask) {
+                             float block_size_out, KeySet map, unsigned long long* map_mask,
+                             int32_t* err, const unsigned long long* __restrict__ filter_keys,
+                             uint32_t filter_mask) {
+  const KeyLookup filter{filter_keys, filter_mask};
   const uint32_t g = blockIdx.x * blockDim.x + threadIdx.x;
   if (g >= total_blocks) return;
   int lo = 0, hi = n;  // desc[lo].first_block <= g
@@ -441,39 +439,12 @@ __global__ void k_mark_batch(const BatchSubmap* __restrict__ desc, int n, uint32
     if (desc[mid].first_block <= g) lo = mid; else hi = mid;
   }
   const BatchSubmap& d = desc[lo];
-  int bx, by, bz;
-  unpack_block_key(d.A.block_keys[g - d.first_block], bx, by, bz);
-  const V3 c_in = V3{center_coord(bx, d.A.block_size), center_coord(by, d.A.block_size),
-                     center_coord(bz, d.A.block_size)};
-  const V3 c = apply(d.T_B_A, c_in);
-  const float kDiag = 1.7320508075688772f;  // kUnitCubeDiagonalLength
-  const float offset = kDiag * d.A.block_size * 0.5f;
-  const float inv_out = 1.0f / block_size_out;
-  constexpr int lim = kVoxIdxOffset / kVps;
-  for (float x = c.x - offset; x < c.x + offset; x += block_size_out)
-    for (float y = c.y - offset; y < c.y + offset; y += block_size_out)
-      for (float z = c.z - offset; z < c.z + offset; z += block_size_out) {
-        const int ix = grid_index(x, inv_out), iy = grid_index(y, inv_out),
-                  iz = grid_index(z, inv_out);
-        if (ix < -lim || ix >= lim || iy < -lim || iy >= lim || iz < -lim || iz >= lim) {
-          atomicOr(err, kErrOutOfRange);
-          continue;
-        }
-        const uint64_t key = pack_block_key(ix, iy, iz);
-        if (filter_keys && !key_set_contains(filter_keys, filter_mask, key)) continue;
-        uint32_t h = hash_key(key) & map_cap_mask;
-        for (;;) {
-          const uint64_t k = map_keys[h];
-          if (k == key) break;
-          if (k == kEmptyKey) {
-            const unsigned long long old = atomicCAS(
-                reinterpret_cast<unsigned long long*>(&map_keys[h]), kEmptyKey, key);
-            if (old == kEmptyKey || old == key) break;
-          }
-          h = (h + 1) & map_cap_mask;
-        }
-        if (map_mask) atomicOr(&map_mask[h], 1ull << lo);
-      }
+  forward_pass(d.A.block_keys[g - d.first_block], d.A.block_size, d.T_B_A, block_size_out, err,
+               [&](uint64_t key) {
+                 if (filter.keys && !filter.contains(key)) return;
+                 const int e = map.insert(key);
+                 if (map_mask && e >= 0) atomicOr(&map_mask[e], 1ull << lo);
+               });
 }
 
 // Candidates are listed rank-major: first the lowest-numbered submap of every destination block,
@@ -538,14 +509,11 @@ __global__ void k_list_candidates(const unsigned long long* __restrict__ map_mas
 // unfinished candidate never waits: no deadlock whatever the grid size or residency.
 __global__ void __launch_bounds__(kMergeThreads)
 k_project_batch(const BatchSubmap* __restrict__ desc, LayerView B,
-                const uint64_t* __restrict__ map_keys, const BatchCand* __restrict__ list,
+                const unsigned long long* __restrict__ map_keys, const BatchCand* __restrict__ list,
                 const RankTable* __restrict__ table, unsigned long long* done,
                 uint32_t* work_counter, CallCounters* counters) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
-  float* s_d = reinterpret_cast<float*>(smem_raw);  // resampled block, planar
-  float* s_w = s_d + kVoxelsPerBlock;
-  uint32_t* s_c = reinterpret_cast<uint32_t*>(s_w + kVoxelsPerBlock);
-  SlotTable& tab = *reinterpret_cast<SlotTable*>(s_c + kVoxelsPerBlock);
+  ResampleTile& t = *reinterpret_cast<ResampleTile*>(smem_raw);
   __shared__ uint32_t s_cand;
   __shared__ int s_slot;
   const uint32_t num_cand = table->total;
@@ -558,46 +526,8 @@ k_project_batch(const BatchSubmap* __restrict__ desc, LayerView B,
     const BatchCand cd = list[c];
     const uint32_t rank = cd.sub_rank >> 8;
     const BatchSubmap& d = desc[cd.sub_rank & 0xFFu];
-    const LayerView& A = d.A;
-    const uint64_t key = map_keys[cd.entry];
-    int bx, by, bz;
-    unpack_block_key(key, bx, by, bz);
-    const V3 org_out = V3{static_cast<float>(bx) * B.block_size, static_cast<float>(by) * B.block_size,
-                          static_cast<float>(bz) * B.block_size};
-    if (threadIdx.x < kTab * kTab * kTab) {
-      const V3 ctr = V3{center_coord(bx, B.block_size), center_coord(by, B.block_size),
-                        center_coord(bz, B.block_size)};
-      const V3 pc = apply(d.T_A_B, ctr);
-      const float reach = 0.8660254f * B.block_size + A.voxel_size;
-      const int ax = __float2int_rd((pc.x - reach) * A.block_size_inv);
-      const int ay = __float2int_rd((pc.y - reach) * A.block_size_inv);
-      const int az = __float2int_rd((pc.z - reach) * A.block_size_inv);
-      const int t = threadIdx.x;
-      const int dx = t % kTab, dy = (t / kTab) % kTab, dz = t / (kTab * kTab);
-      tab.slot[t] = A.find_slot(pack_block_key(ax + dx, ay + dy, az + dz));
-      if (t == 0) {
-        tab.ax = ax;
-        tab.ay = ay;
-        tab.az = az;
-      }
-    }
-    __syncthreads();
-    bool any = false;
-#pragma unroll 1
-    for (int j = 0; j < kVoxPerThread; ++j) {
-      const int lin = threadIdx.x + j * kMergeThreads;
-      const int vx = lin & 15, vy = (lin >> 4) & 15, vz = lin >> 8;
-      const V3 center_out =
-          org_out + V3{center_coord(vx, B.voxel_size), center_coord(vy, B.voxel_size),
-                       center_coord(vz, B.voxel_size)};
-      const V3 p = apply(d.T_A_B, center_out);
-      VoxelState t;
-      any |= resample_voxel(A, tab, p, t);
-      s_d[lin] = t.d;
-      s_w[lin] = t.w;
-      s_c[lin] = t.c;
-    }
-    const int has_data = __syncthreads_or(any ? 1 : 0);
+    const unsigned long long key = map_keys[cd.entry];
+    const bool has_data = resample_block(d.A, B, d.T_A_B, key, t);
     unsigned long long* turn = done + cd.entry;
     if (!has_data) {  // dropped from its transformed layer: nothing merged, nobody waits for it
       if (threadIdx.x == 0) atomicOr(turn, 1ull << rank);
@@ -632,7 +562,7 @@ k_project_batch(const BatchSubmap* __restrict__ desc, LayerView B,
 #pragma unroll
       for (int j = 0; j < kVoxPerThread; ++j) {
         const int lin = threadIdx.x + j * kMergeThreads;
-        merge_voxel(s_d[lin], s_w[lin], s_c[lin], st[j]);
+        merge_voxel(t.d[lin], t.w[lin], t.c[lin], st[j]);
         __stcg(dp + lin, st[j].d);
         __stcg(wp + lin, st[j].w);
         __stcg(cp + lin, st[j].c);
@@ -653,7 +583,7 @@ __global__ void k_copy_desc(uint32_t* __restrict__ dst, const uint32_t* __restri
 // context's stream, nothing is read back
 static int32_t project_batch(const cg_layer* const* submaps, const BatchSubmap* h_desc,
                              const BatchSubmap* d_desc, size_t i0, size_t i1, cg_layer* G,
-                             const uint64_t* filter_keys = nullptr, uint32_t filter_mask = 0) {
+                             KeyLookup filter = KeyLookup{}) {
   cg_context* ctx = G->ctx;
   cudaStream_t s = ctx->stream;
   const int n = static_cast<int>(i1 - i0);
@@ -665,8 +595,7 @@ static int32_t project_batch(const cg_layer* const* submaps, const BatchSubmap* 
     cand_bound += mark_bound(A, G, h_desc[i0 + k].num_blocks);
   }
   if (total == 0) return CG_OK;
-  size_t cap = 4096;
-  while (cap < 2 * cand_bound) cap <<= 1;
+  const size_t cap = key_set_capacity(cand_bound, 4096);
   CG_CUDA(ctx->cand_keys.reserve(cap * sizeof(uint64_t)));
   // masks, then the per-entry "done" masks of the fused fold, then the rank table (one memset
   // clears all)
@@ -682,26 +611,22 @@ static int32_t project_batch(const cg_layer* const* submaps, const BatchSubmap* 
     CG_CUDA(cudaMemsetAsync(masks, 0, scratch_bytes, s));
     CG_CUDA(cudaMemsetAsync(ctx->d_work_counter, 0, sizeof(uint32_t), s));
     k_mark_batch<<<grid_for(total, 128), 128, 0, s>>>(
-        d_desc + i0, n, total, G->v.block_size, ctx->cand_keys.as<uint64_t>(), masks,
-        static_cast<uint32_t>(cap - 1), G->v.err, filter_keys, filter_mask);
+        d_desc + i0, n, total, G->v.block_size,
+        KeySet{ctx->cand_keys.as<unsigned long long>(), static_cast<uint32_t>(cap - 1)}, masks,
+        G->v.err, filter.keys, filter.mask);
     k_rank_hist<<<grid_for(cap, 256), 256, 0, s>>>(masks, static_cast<uint32_t>(cap), table);
     k_list_candidates<<<grid_for(cap, 256), 256, 0, s>>>(masks, static_cast<uint32_t>(cap), table,
                                                          ctx->merge_cands.as<BatchCand>(),
                                                          ctx->d_counters);
   }
-  const size_t smem = 3 * kVoxelsPerBlock * sizeof(float) + sizeof(SlotTable);
-  static bool attr_set[64] = {};  // per device ordinal
-  if (ctx->device < 0 || ctx->device >= 64 || !attr_set[ctx->device]) {
-    CG_CUDA(cudaFuncSetAttribute(k_project_batch, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                 static_cast<int>(smem)));
-    if (ctx->device >= 0 && ctx->device < 64) attr_set[ctx->device] = true;
-  }
+  constexpr size_t smem = sizeof(ResampleTile);
+  CG_CUDA(allow_dynamic_smem<k_project_batch>(ctx->device, smem));
   {
     StageScope sc(ctx, kStageMergeResample, 1);
     const unsigned grid = static_cast<unsigned>(
         std::min<size_t>(cand_bound, static_cast<size_t>(ctx->num_sms) * 2));
     k_project_batch<<<grid, kMergeThreads, smem, s>>>(
-        d_desc + i0, G->v, ctx->cand_keys.as<uint64_t>(), ctx->merge_cands.as<BatchCand>(), table,
+        d_desc + i0, G->v, ctx->cand_keys.as<unsigned long long>(), ctx->merge_cands.as<BatchCand>(), table,
         done, ctx->d_work_counter, ctx->d_counters);
   }
   CG_CUDA(cudaGetLastError());
@@ -907,13 +832,13 @@ int32_t reproject_local(const cg_layer* const* submaps, size_t n, size_t num_kno
   uint64_t removed = 0;
   if (dirty_src > 0) {
     // the dirty set: destination blocks a moved submap marks under either pose, or a new one marks
-    size_t cap = 4096;
-    while (cap < 2 * dirty_bound) cap <<= 1;
+    const size_t cap = key_set_capacity(dirty_bound, 4096);
     const size_t g_blocks = static_cast<size_t>(G->num_blocks);
     CG_CUDA(ctx->stage_a.reserve(cap * sizeof(uint64_t)));
     CG_CUDA(ctx->stage_b.reserve((g_blocks + 2) * sizeof(uint32_t)));
     uint32_t* counts = ctx->stage_b.as<uint32_t>();  // [0] dirty blocks present in G, [1] dirty blocks
     uint32_t* slots = counts + 2;
+    const KeySet dirty_set{ctx->stage_a.as<unsigned long long>(), static_cast<uint32_t>(cap - 1)};
     const uint64_t* dirty_keys = ctx->stage_a.as<uint64_t>();
     {
       StageScope sc(ctx, kStageMergeMark, 3);
@@ -921,7 +846,7 @@ int32_t reproject_local(const cg_layer* const* submaps, size_t n, size_t num_kno
       CG_CUDA(cudaMemsetAsync(counts, 0, 2 * sizeof(uint32_t), s));
       k_mark_batch<<<grid_for(dirty_src, 128), 128, 0, s>>>(
           d_desc + n, static_cast<int>(2 * moved.size() + num_new), dirty_src, G->v.block_size,
-          ctx->stage_a.as<uint64_t>(), nullptr, static_cast<uint32_t>(cap - 1), G->v.err, nullptr, 0);
+          dirty_set, nullptr, G->v.err, nullptr, 0);
       k_dirty_slots<<<grid_for(cap, 256), 256, 0, s>>>(
           G->v, dirty_keys, static_cast<uint32_t>(cap), slots, counts,
           dirty ? dirty->keys : nullptr, dirty ? dirty->count : nullptr, dirty ? dirty->cap : 0);
@@ -974,7 +899,7 @@ int32_t reproject_local(const cg_layer* const* submaps, size_t n, size_t num_kno
     for (size_t i0 = 0; i0 < num_known; i0 += kBatchMax) {
       int32_t rc = project_batch(submaps, h.data(), d_desc, i0,
                                  std::min(num_known, i0 + static_cast<size_t>(kBatchMax)), G,
-                                 dirty_keys, static_cast<uint32_t>(cap - 1));
+                                 KeyLookup{dirty_set.keys, dirty_set.mask});
       if (rc) return rc;
     }
     for (size_t i0 = num_known; i0 < n; i0 += kBatchMax) {

@@ -511,17 +511,6 @@ k_mesh_blocks(LayerView L, Blocks blocks, const uint64_t* __restrict__ sorted_ke
   }
 }
 
-__global__ void k_mesh_unpack_idx(const uint64_t* __restrict__ keys, uint32_t n,
-                                  int32_t* __restrict__ idx) {
-  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  int x, y, z;
-  unpack_block_key(keys[i], x, y, z);
-  idx[3 * i] = x;
-  idx[3 * i + 1] = y;
-  idx[3 * i + 2] = z;
-}
-
 }  // namespace cg
 
 using namespace cg;
@@ -580,7 +569,7 @@ static int32_t mesh_to_device(const cg_layer* L, float min_weight, int32_t use_c
       else
         launch_mesh<false>(grid, s, L, LocalBlocks{}, keys, slots, nb, min_weight, use_color,
                            only_updated, counts, nullptr, nullptr, nullptr, nullptr);
-      k_mesh_unpack_idx<<<grid_for(n, 256), 256, 0, s>>>(keys, nb, ctx->mc_index.as<int32_t>());
+      k_unpack_idx<<<grid_for(n, 256), 256, 0, s>>>(keys, nb, ctx->mc_index.as<int32_t>());
     }
     CG_CUDA(cub::DeviceScan::ExclusiveSum(ctx->cub_tmp.p, tmp, counts, begin, static_cast<int>(n + 1), s));
     uint32_t back[3] = {0u, 0u, 0u};  // total, duplicate key (low, high word)
