@@ -18,8 +18,9 @@ OBJS = $(OBJ)/layer.o $(OBJ)/integrate.o $(OBJ)/integrate_front.o $(OBJ)/integra
 HOSTCHK = build/host_api_check
 DEPTHCHK = build/depth_api_check
 ESDFCHK = build/esdf_update_check
+GATHERCHK = build/mesh_gather_check
 
-all: $(LIB) oracle $(HOSTCHK) $(DEPTHCHK) $(ESDFCHK)
+all: $(LIB) oracle $(HOSTCHK) $(DEPTHCHK) $(ESDFCHK) $(GATHERCHK)
 
 $(OBJ)/%.o: $(SRC)/%.cu $(HDRS)
 	@mkdir -p $(OBJ)
@@ -45,6 +46,11 @@ $(DEPTHCHK): tests/host/depth_api_check.cc coxgraph_b200/host/coxgraph_b200.hpp 
 # C++ incremental-ESDF driver (tests/test_host_esdf_update.py)
 $(ESDFCHK): tests/host/esdf_update_check.cc coxgraph_b200/host/coxgraph_b200.hpp include/coxgraph_b200.h $(LIB)
 	g++ -std=c++17 -O1 -Wall -Wextra tests/host/esdf_update_check.cc -o $@ -Lcoxgraph_b200/lib \
+	    -lcoxgraph_b200 -Wl,-rpath,'$$ORIGIN/../coxgraph_b200/lib'
+
+# C++ sharded-mesh gather driver (tests/test_host_mesh_gather.py)
+$(GATHERCHK): tests/host/mesh_gather_check.cc coxgraph_b200/host/coxgraph_b200.hpp include/coxgraph_b200.h $(LIB)
+	g++ -std=c++17 -O1 -Wall -Wextra tests/host/mesh_gather_check.cc -o $@ -Lcoxgraph_b200/lib \
 	    -lcoxgraph_b200 -Wl,-rpath,'$$ORIGIN/../coxgraph_b200/lib'
 
 clean:

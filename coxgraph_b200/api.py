@@ -60,6 +60,7 @@ class Context:
                                                  C.byref(self._h)))
         self.device = int(device)
         self.has_comm = False   # commInit done (multi-GPU merge through the C ABI)
+        self.comm_rank = None   # this context's rank in its communicator
 
     def synchronize(self):
         capi.check(capi.load().cg_context_synchronize(self._h))
@@ -319,13 +320,18 @@ def _mesh(entry, layer, min_weight, use_color, only_updated, fetch):
     B, V = nb.value, nv.value
     if not fetch:  # the mesh stays on the device (cg_mesh_fetch copies it out later)
         return B, V
+    return _fetch_mesh(layer.ctx, B, V)
+
+
+def _fetch_mesh(ctx, B, V):
+    """cg_mesh_fetch of the B blocks / V vertices retained in `ctx` -> generateMesh's tuple."""
     idx = np.zeros((B, 3), np.int32)
     begin = np.zeros(B + 1, np.uint32)
     v = np.zeros((V, 3), np.float32)
     n = np.zeros((V, 3), np.float32)
     c = np.zeros((V, 4), np.uint8)
     if B:
-        capi.check(capi.load().cg_mesh_fetch(layer.ctx._h, B, V, _ptr(idx), _ptr(begin),
+        capi.check(capi.load().cg_mesh_fetch(ctx._h, B, V, _ptr(idx), _ptr(begin),
                                              _ptr(v) if V else None, _ptr(n) if V else None,
                                              _ptr(c) if V else None))
     return idx, begin, v, n, c
@@ -632,6 +638,7 @@ def commInit(ctx, unique_id, rank, nranks):
     buf = (C.c_uint8 * 128).from_buffer_copy(unique_id)
     capi.check(capi.load().cg_comm_init(ctx._h, buf, int(rank), int(nranks)))
     ctx.has_comm = True
+    ctx.comm_rank = int(rank)
 
 
 def gatherGlobal(partial_layer, owned_layer):
@@ -680,6 +687,20 @@ def generateMeshSharded(owned_layer, min_weight=1e-4, use_color=True, only_updat
     peers).  Same tuple as Layer.generateMesh."""
     return _mesh(capi.load().cg_layer_mesh_sharded, owned_layer, min_weight, use_color,
                  only_updated, fetch)
+
+
+def gatherMeshSharded(ctx, root=0, fetch=True):
+    """Collective, right after generateMeshSharded on every rank: the ranks' block meshes are
+    gathered onto rank `root`, which then holds exactly what generateMesh leaves for one layer
+    holding every rank's owned blocks (so getConnectedMesh there is the combined map's PLY mesh).
+    Returns Layer.generateMesh's tuple on the root (with fetch=False only the global (B, V)) and
+    the global (B, V) on the other ranks, whose own share stays retained."""
+    nb, nv = C.c_size_t(0), C.c_size_t(0)
+    capi.check(capi.load().cg_mesh_gather_sharded(ctx._h, int(root), C.byref(nb), C.byref(nv)))
+    B, V = nb.value, nv.value
+    if not fetch or ctx.comm_rank != int(root):
+        return B, V
+    return _fetch_mesh(ctx, B, V)
 
 
 def commPeerMappings(ctx):

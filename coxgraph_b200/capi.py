@@ -240,6 +240,8 @@ SYMBOLS = {
     "cg_layer_mesh_sharded": (C.c_int32, [_P, C.c_float, C.c_int32, C.c_int32, C.c_size_t, C.c_size_t,
                                           _P, _P, _P, _P, _P, C.POINTER(C.c_size_t),
                                           C.POINTER(C.c_size_t)]),
+    "cg_mesh_gather_sharded": (C.c_int32, [_P, C.c_int32, C.POINTER(C.c_size_t),
+                                           C.POINTER(C.c_size_t)]),
     "cg_comm_peer_mappings": (C.c_int32, [_P, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
     "cg_debug_selftest": (C.c_int32, [_P, C.c_int32, C.c_uint64, C.POINTER(C.c_uint64)]),
 }

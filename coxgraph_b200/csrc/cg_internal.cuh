@@ -31,6 +31,10 @@ constexpr uint64_t kInvalidPointKey = ~0ull;         // sorts behind every valid
 constexpr int kClearingBit = 60;
 
 enum ErrBits { kErrPoolFull = 1, kErrOutOfRange = 2, kErrTouchFull = 4, kErrSegmentFull = 8, kErrKeyRange = 16 };
+// cg_context::mc_kind: nothing retained (none yet, or the last mesh call failed), the result of
+// cg_layer_mesh, of cg_layer_mesh_sharded, a sharded result already gathered (on the root: the
+// gathered mesh), or buffers that cg_esdf_free_points has reused
+enum MeshKind { kMeshNone = 0, kMeshLocal, kMeshSharded, kMeshGathered, kMeshReused };
 
 // ------------------------------------------------------------------ key packing
 __host__ __device__ __forceinline__ uint64_t pack_block_key(int x, int y, int z) {
@@ -389,6 +393,14 @@ struct cg_context : cg::FrontBufs {
   // marching cubes (mesh.cu)
   cg::DevBuf mc_counts, mc_index, mc_vertices, mc_normals, mc_colors;
   size_t mc_blocks = 0, mc_total = 0;  // size of the retained result (cg_mesh_fetch)
+  // what the retained result is (cg::MeshKind), and the cg_layer_mesh_sharded calls made on this
+  // context: cg_mesh_gather_sharded gathers only the result of every rank's latest sharded call
+  int mc_kind = 0;
+  uint64_t mc_sharded_calls = 0;
+  // cg_mesh_gather_sharded on the root: the peers' block meshes as received, the sort of every
+  // rank's block keys, the per-rank source table, and the buffers the gathered mesh is placed in
+  // (swapped with mc_* once placed)
+  cg::DevBuf mg_in, mg_sort, mg_src, mg_counts, mg_index, mg_vertices, mg_normals, mg_colors;
   cg::DevBuf weld_keys, weld_words, weld_out;  // vertex welding (mesh_connect.cu)
   // ESDF of a layer (esdf.cu): working / result planes in (z, y, x) block order, retained until
   // the next cg_layer_esdf_batch / cg_layer_esdf_update on this context

@@ -14,12 +14,13 @@
 //                    mergeVoxelAIntoVoxelB, R10; reference call site of that overload:
 //                    coxgraph/src/server/submap_collection.cpp:31-33); the block is written once
 // — gather and fold are ONE kernel, there is no packing pass, no staging copy and no host
-// synchronisation between listing, exchange and fold.  NCCL (loaded at run time from
-// libnccl.so.2, the one torch has loaded if there is one) is the bootstrap and the barrier only:
-// unique id -> communicator, one all-gather of the IPC handles when a partial layer is bound, and a
-// one-word all-reduce on the stream before and after the kernels (all partial layers complete /
-// all peers done reading).  The fold order is fixed, so the result is deterministic and equal to
-// the packed exchange of exchange.cu (hash owner, NCCL all-to-all) block for block.
+// synchronisation between listing, exchange and fold.  For the gather and the sharded mesh, NCCL
+// (loaded at run time from libnccl.so.2, the one torch has loaded if there is one) is the bootstrap
+// and the barrier only: unique id -> communicator, one all-gather of the IPC handles when a layer
+// is bound, and a one-word all-reduce on the stream before and after the kernels (all partial
+// layers complete / all peers done reading).  The fold order is fixed, so the result is
+// deterministic and equal to the packed exchange of exchange.cu (hash owner, NCCL all-to-all)
+// block for block.
 //
 // cg_layer_mesh_sharded (mesh.cu) meshes the owned layers where they lie.  Its collective half is
 // here: the owned layer is bound like the partial one (its own binding, so alternating gather and
@@ -27,6 +28,17 @@
 // records where each block's planes are.  The mesh kernel resolves the one-block halo (the +x/+y/+z
 // neighbours and a vertex's colour block) through that map and reads the peer's planes over
 // NVLink; a key two ranks hold is found while the map is built.
+//
+// cg_mesh_gather_sharded moves those block meshes to one root rank, where they become the mesh
+// cg_layer_mesh leaves for the union of the owned layers.  The mesh buffers are per-call scratch
+// that grows, so they are not mapped over IPC: one all-gather of a few words per rank (block and
+// vertex counts, what the rank retains, the root) sizes the root's buffers, one all-reduce is the
+// go/no-go, and NCCL point-to-point sends move each peer's block indices, vertex ranges, vertices,
+// normals and colours into the root's staging buffer.  On the root, k_gather_keys + a radix sort
+// put every rank's blocks in the packed-key order of sort_blocks, a scan of the per-block vertex
+// counts gives vertex_begin, and k_place_blocks copies each block's range into fresh buffers that
+// then replace the root's own share.
+#include <cub/cub.cuh>
 #include <dlfcn.h>
 #include <string.h>
 
@@ -49,6 +61,10 @@ struct Nccl {
   int (*CommDestroy)(ncclComm_t) = nullptr;
   int (*AllReduce)(const void*, void*, size_t, int, int, ncclComm_t, cudaStream_t) = nullptr;
   int (*AllGather)(const void*, void*, size_t, int, ncclComm_t, cudaStream_t) = nullptr;
+  int (*Send)(const void*, size_t, int, int, ncclComm_t, cudaStream_t) = nullptr;
+  int (*Recv)(void*, size_t, int, int, ncclComm_t, cudaStream_t) = nullptr;
+  int (*GroupStart)() = nullptr;
+  int (*GroupEnd)() = nullptr;
   const char* (*GetErrorString)(int) = nullptr;
 };
 static Nccl g_nccl;
@@ -68,9 +84,13 @@ static int32_t load_nccl() {
   n.CommDestroy = reinterpret_cast<decltype(n.CommDestroy)>(dlsym(h, "ncclCommDestroy"));
   n.AllReduce = reinterpret_cast<decltype(n.AllReduce)>(dlsym(h, "ncclAllReduce"));
   n.AllGather = reinterpret_cast<decltype(n.AllGather)>(dlsym(h, "ncclAllGather"));
+  n.Send = reinterpret_cast<decltype(n.Send)>(dlsym(h, "ncclSend"));
+  n.Recv = reinterpret_cast<decltype(n.Recv)>(dlsym(h, "ncclRecv"));
+  n.GroupStart = reinterpret_cast<decltype(n.GroupStart)>(dlsym(h, "ncclGroupStart"));
+  n.GroupEnd = reinterpret_cast<decltype(n.GroupEnd)>(dlsym(h, "ncclGroupEnd"));
   n.GetErrorString = reinterpret_cast<decltype(n.GetErrorString)>(dlsym(h, "ncclGetErrorString"));
   if (!n.GetUniqueId || !n.CommInitRank || !n.CommDestroy || !n.AllReduce || !n.AllGather ||
-      !n.GetErrorString) {
+      !n.Send || !n.Recv || !n.GroupStart || !n.GroupEnd || !n.GetErrorString) {
     set_error("libnccl.so.2 lacks an expected symbol");
     return CG_ERR_UNSUPPORTED;
   }
@@ -155,6 +175,7 @@ struct cg_comm {
   cg::DevBuf mplanes;                 // the block's distance plane in its holder's pool
   cg::DevBuf mcounters;               // k_build_holders' words ([2] overflow: cannot happen)
   size_t mcap = 0;
+  cg::DevBuf gwords;                  // cg_mesh_gather_sharded: every rank's GatherWords
 };
 
 namespace cg {
@@ -424,7 +445,7 @@ static void unbind(cg_comm* c) {
   if (c->dcounters) cudaFree(c->dcounters);
   c->dcounters = nullptr;
   for (DevBuf* d : {&c->hkeys, &c->hmask, &c->hbase, &c->mine, &c->slots, &c->counters, &c->mkeys,
-                    &c->mmask, &c->mplanes, &c->mcounters})
+                    &c->mmask, &c->mplanes, &c->mcounters, &c->gwords})
     d->release();
   c->hcap = c->list_cap = c->mcap = 0;
 }
@@ -633,6 +654,88 @@ static int32_t fold_owned(cg_context* ctx, cg_layer* owned) {
   return CG_OK;
 }
 
+// ---- cg_mesh_gather_sharded
+// What every rank tells the others in the opening all-gather.
+struct GatherWords {
+  unsigned long long blocks, vertices;  // the retained mesh
+  unsigned long long kind, calls;       // cg_context::mc_kind, mc_sharded_calls
+  long long root;
+};
+// One rank's block meshes as the root reads them: its own retained buffers, or the regions of
+// mg_in a peer's sends landed in.  Block b of the rank is block first + b of the concatenation.
+struct MeshSource {
+  const int32_t* idx;     // [3 blocks] block indices, (z, y, x) order
+  const uint32_t* begin;  // [blocks + 1] vertex ranges
+  const uint32_t* vertices;
+  const uint32_t* normals;
+  const uint32_t* colors;
+  uint32_t blocks, first;
+};
+// every rank's block keys, with (rank << 32 | block) as payload.  Grid y = rank.
+__global__ void k_gather_keys(const MeshSource* __restrict__ src, unsigned long long* __restrict__ keys,
+                              unsigned long long* __restrict__ vals) {
+  const int r = blockIdx.y;
+  const MeshSource S = src[r];
+  for (uint32_t b = blockIdx.x * blockDim.x + threadIdx.x; b < S.blocks; b += gridDim.x * blockDim.x) {
+    keys[S.first + b] = pack_block_key(S.idx[3 * b], S.idx[3 * b + 1], S.idx[3 * b + 2]);
+    vals[S.first + b] = (static_cast<unsigned long long>(r) << 32) | b;
+  }
+}
+// vertex count of every block in sorted order, and a 0 behind the last (for the exclusive scan)
+__global__ void k_gather_counts(const MeshSource* __restrict__ src,
+                                const unsigned long long* __restrict__ vals, uint32_t n,
+                                uint32_t* __restrict__ counts) {
+  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i <= n; i += gridDim.x * blockDim.x) {
+    uint32_t k = 0;
+    if (i < n) {
+      const unsigned long long p = vals[i];
+      const uint32_t* begin = src[p >> 32].begin;
+      const uint32_t b = static_cast<uint32_t>(p);
+      k = begin[b + 1] - begin[b];
+    }
+    counts[i] = k;
+  }
+}
+// n words, one warp: 16-byte accesses when source and destination share their alignment
+__device__ __forceinline__ void warp_copy(uint32_t* __restrict__ d, const uint32_t* __restrict__ s,
+                                          uint32_t n, int lane) {
+  if (((reinterpret_cast<uintptr_t>(d) ^ reinterpret_cast<uintptr_t>(s)) & 15u) == 0) {
+    const uint32_t head = min(n, static_cast<uint32_t>(((16u - (reinterpret_cast<uintptr_t>(d) & 15u)) & 15u) >> 2));
+    if (lane < static_cast<int>(head)) d[lane] = s[lane];
+    d += head;
+    s += head;
+    n -= head;
+    const uint32_t quads = n >> 2;
+    for (uint32_t q = lane; q < quads; q += 32)
+      reinterpret_cast<uint4*>(d)[q] = reinterpret_cast<const uint4*>(s)[q];
+    const uint32_t tail = n & 3u;
+    if (lane < static_cast<int>(tail)) d[4 * quads + lane] = s[4 * quads + lane];
+  } else {
+    for (uint32_t k = lane; k < n; k += 32) d[k] = s[k];
+  }
+}
+// one warp per block in sorted order: its index and its vertex range (vertices, normals, colours)
+// go to their place in the gathered mesh
+constexpr int kPlaceThreads = 256;
+__global__ void __launch_bounds__(kPlaceThreads)
+k_place_blocks(const MeshSource* __restrict__ src, const unsigned long long* __restrict__ vals,
+               const uint32_t* __restrict__ begin, uint32_t n, int32_t* __restrict__ idx,
+               uint32_t* __restrict__ vertices, uint32_t* __restrict__ normals,
+               uint32_t* __restrict__ colors) {
+  const int lane = threadIdx.x & 31;
+  const uint32_t warps = gridDim.x * (kPlaceThreads / 32);
+  for (uint32_t i = blockIdx.x * (kPlaceThreads / 32) + (threadIdx.x >> 5); i < n; i += warps) {
+    const unsigned long long p = vals[i];
+    const MeshSource& S = src[p >> 32];
+    const uint32_t b = static_cast<uint32_t>(p);
+    const uint32_t lo = S.begin[b], k = S.begin[b + 1] - lo, at = begin[i];
+    if (lane < 3) idx[3 * static_cast<size_t>(i) + lane] = S.idx[3 * static_cast<size_t>(b) + lane];
+    warp_copy(vertices + 3 * static_cast<size_t>(at), S.vertices + 3 * static_cast<size_t>(lo), 3 * k, lane);
+    warp_copy(normals + 3 * static_cast<size_t>(at), S.normals + 3 * static_cast<size_t>(lo), 3 * k, lane);
+    warp_copy(colors + at, S.colors + lo, k, lane);
+  }
+}
+
 }  // namespace cg
 
 using namespace cg;
@@ -793,6 +896,20 @@ static int32_t status_of(uint32_t word) {  // the most severe failure a rank rep
     if ((word >> (8 * f)) & 0xFFu) return kinds[f];
   return CG_OK;
 }
+// A barrier that carries every rank's status_bits(local), summed into *word (one host
+// synchronisation).
+static int32_t status_barrier(cg_context* ctx, int32_t local, uint32_t* word) {
+  cg_comm* c = ctx->comm;
+  cudaStream_t s = ctx->stream;
+  *word = status_bits(local);
+  CG_CUDA(cudaMemcpyAsync(c->d_token, word, sizeof(*word), cudaMemcpyHostToDevice, s));
+  int32_t rc;
+  if ((rc = barrier(ctx))) return rc;
+  CG_CUDA(cudaMemcpyAsync(word, c->d_token, sizeof(*word), cudaMemcpyDeviceToHost, s));
+  CG_CUDA(cudaMemsetAsync(c->d_token, 0, sizeof(int), s));
+  CG_CUDA(cudaStreamSynchronize(s));
+  return CG_OK;
+}
 
 int32_t cg_reproject_submaps_sharded(const cg_layer* const* submaps, size_t n, size_t num_known,
                                      const float* poses_old, const float* poses_new,
@@ -852,14 +969,10 @@ int32_t cg_reproject_submaps_sharded(const cg_layer* const* submaps, size_t n, s
     k_publish_words<<<1, 1, 0, s>>>(c->partial.shared, static_cast<uint32_t>(partial->num_blocks),
                                     static_cast<uint32_t>(owned->num_blocks), fbits);
   }
-  uint32_t word = status_bits(local);
-  CG_CUDA(cudaMemcpyAsync(c->d_token, &word, sizeof(word), cudaMemcpyHostToDevice, s));
+  uint32_t word = 0;
   int32_t rc;
   // every rank's partial layer, dirty keys and counts are complete (stream-ordered)
-  if ((rc = barrier(ctx))) return rc;
-  CG_CUDA(cudaMemcpyAsync(&word, c->d_token, sizeof(word), cudaMemcpyDeviceToHost, s));
-  CG_CUDA(cudaMemsetAsync(c->d_token, 0, sizeof(int), s));
-  CG_CUDA(cudaStreamSynchronize(s));
+  if ((rc = status_barrier(ctx, local, &word))) return rc;
   if (local) return local;
   if (word) {
     set_error("%s: another rank's local step failed (status %d); no owned layer was changed", who,
@@ -945,6 +1058,286 @@ int32_t cg_reproject_submaps_sharded(const cg_layer* const* submaps, size_t n, s
     stats->blocks_folded = static_cast<uint64_t>(owned->num_blocks - (owned_before - listed));
     stats->blocks_removed = removed;
   }
+  return CG_OK;
+}
+
+// ---- cg_mesh_gather_sharded (DESIGN.md §5): every rank's block meshes -> the root, in the block
+// order cg_layer_mesh gives the union of the owned layers.
+static const char* kGatherWho = "cg_mesh_gather_sharded";
+
+// The same verdict on every rank: it judges the all-gathered words only.
+static int32_t gather_verdict(const std::vector<GatherWords>& all) {
+  const char* who = kGatherWho;
+  const int R = static_cast<int>(all.size());
+  for (int r = 0; r < R; ++r) {
+    if (all[r].root < 0 || all[r].root >= R) {
+      set_error("%s: rank %d passed root %lld, outside [0, %d)", who, r, all[r].root, R);
+      return CG_ERR_INVALID_ARG;
+    }
+  }
+  for (int r = 1; r < R; ++r) {
+    if (all[r].root != all[0].root) {
+      set_error("%s: the ranks passed different roots (rank 0: %lld, rank %d: %lld)", who,
+                all[0].root, r, all[r].root);
+      return CG_ERR_INVALID_ARG;
+    }
+  }
+  for (int r = 0; r < R; ++r) {
+    const char* why = nullptr;
+    switch (static_cast<int>(all[r].kind)) {
+      case kMeshSharded: break;
+      case kMeshLocal: why = "is from cg_layer_mesh, not cg_layer_mesh_sharded"; break;
+      case kMeshGathered: why = "has been gathered already (call cg_layer_mesh_sharded again)"; break;
+      case kMeshReused: why = "is gone: cg_esdf_free_points reused its buffers"; break;
+      default: why = "does not exist (no mesh call yet, or the last one failed)"; break;
+    }
+    if (why) {
+      set_error("%s: rank %d's retained mesh %s", who, r, why);
+      return CG_ERR_INVALID_ARG;
+    }
+    if (all[r].calls != all[0].calls) {
+      set_error("%s: rank %d's mesh is from its cg_layer_mesh_sharded call %llu, rank 0's from call %llu",
+                who, r, all[r].calls, all[0].calls);
+      return CG_ERR_INVALID_ARG;
+    }
+  }
+  unsigned long long blocks = 0, vertices = 0;
+  for (const GatherWords& w : all) {
+    blocks += w.blocks;
+    vertices += w.vertices;
+  }
+  if (vertices > 0xFFFFFFFFull || blocks > 0x7FFFFFF0ull) {
+    set_error("%s: the gathered mesh would hold %llu blocks and %llu vertices; vertex_begin (uint32) "
+              "indexes at most 4294967295 vertices", who, blocks, vertices);
+    return CG_ERR_INVALID_ARG;
+  }
+  return CG_OK;
+}
+
+// Where a peer's sends land in the root's mg_in (byte offsets, 256-byte aligned).
+struct PeerRegions {
+  size_t idx, begin, vertices, normals, colors;
+};
+
+// Every buffer the root needs, reserved before the first byte moves.
+static int32_t gather_reserve(cg_context* ctx, const std::vector<GatherWords>& all, int root,
+                              std::vector<PeerRegions>* regions) {
+  const size_t R = all.size();
+  size_t N = 0, V = 0, in_bytes = 0;
+  auto take = [&](size_t bytes) {
+    const size_t at = in_bytes;
+    in_bytes += (bytes + 255) & ~static_cast<size_t>(255);
+    return at;
+  };
+  regions->assign(R, PeerRegions{0, 0, 0, 0, 0});
+  for (size_t r = 0; r < R; ++r) {
+    const size_t n = all[r].blocks, v = all[r].vertices;
+    N += n;
+    V += v;
+    if (static_cast<int>(r) == root || n == 0) continue;
+    PeerRegions& g = (*regions)[r];
+    g.idx = take(3 * n * sizeof(int32_t));
+    g.begin = take((n + 1) * sizeof(uint32_t));
+    g.vertices = take(3 * v * sizeof(float));
+    g.normals = take(3 * v * sizeof(float));
+    g.colors = take(v * sizeof(uint32_t));
+  }
+  if (N == 0) return CG_OK;
+  CG_CUDA(ctx->mg_in.reserve(in_bytes));
+  CG_CUDA(ctx->mg_sort.reserve(4 * N * sizeof(unsigned long long)));
+  CG_CUDA(ctx->mg_src.reserve(R * sizeof(MeshSource)));
+  CG_CUDA(ctx->mg_counts.reserve((2 * (N + 1) + 2) * sizeof(uint32_t)));
+  CG_CUDA(ctx->mg_index.reserve(3 * N * sizeof(int32_t)));
+  CG_CUDA(ctx->mg_vertices.reserve(3 * V * sizeof(float)));
+  CG_CUDA(ctx->mg_normals.reserve(3 * V * sizeof(float)));
+  CG_CUDA(ctx->mg_colors.reserve(V * sizeof(uint32_t)));
+  size_t sort_tmp = 0, scan_tmp = 0;
+  CG_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, sort_tmp, static_cast<const unsigned long long*>(nullptr),
+                                          static_cast<unsigned long long*>(nullptr),
+                                          static_cast<const unsigned long long*>(nullptr),
+                                          static_cast<unsigned long long*>(nullptr),
+                                          static_cast<int>(N), 0, 63, ctx->stream));
+  CG_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, scan_tmp, static_cast<const uint32_t*>(nullptr),
+                                        static_cast<uint32_t*>(nullptr), static_cast<int>(N + 1),
+                                        ctx->stream));
+  CG_CUDA(ctx->cub_tmp.reserve(std::max(sort_tmp, scan_tmp)));
+  return CG_OK;
+}
+
+// Each peer's block meshes to the root (NCCL point-to-point, one group); a rank without blocks
+// sends nothing, and the root posts exactly the receives that match.
+static int32_t gather_transfer(cg_context* ctx, const std::vector<GatherWords>& all, int root,
+                               const std::vector<PeerRegions>& regions) {
+  cg_comm* c = ctx->comm;
+  cudaStream_t s = ctx->stream;
+  int e = g_nccl.GroupStart();
+  if (e != ncclSuccess) {
+    set_error("%s: ncclGroupStart failed: %s", kGatherWho, g_nccl.GetErrorString(e));
+    return CG_ERR_CUDA;
+  }
+  auto send = [&](const void* p, size_t bytes) {
+    if (e == ncclSuccess && bytes) e = g_nccl.Send(p, bytes, ncclInt8, root, c->comm, s);
+  };
+  auto recv = [&](size_t at, size_t bytes, int peer) {
+    if (e == ncclSuccess && bytes)
+      e = g_nccl.Recv(ctx->mg_in.as<char>() + at, bytes, ncclInt8, peer, c->comm, s);
+  };
+  if (c->rank != root) {
+    const size_t n = ctx->mc_blocks, v = ctx->mc_total;
+    if (n > 0) {
+      send(ctx->mc_index.p, 3 * n * sizeof(int32_t));
+      send(ctx->mc_counts.as<uint32_t>() + (n + 1), (n + 1) * sizeof(uint32_t));
+      send(ctx->mc_vertices.p, 3 * v * sizeof(float));
+      send(ctx->mc_normals.p, 3 * v * sizeof(float));
+      send(ctx->mc_colors.p, v * sizeof(uint32_t));
+    }
+  } else {
+    for (int r = 0; r < c->nranks; ++r) {
+      const size_t n = all[r].blocks, v = all[r].vertices;
+      if (r == root || n == 0) continue;
+      const PeerRegions& g = regions[r];
+      recv(g.idx, 3 * n * sizeof(int32_t), r);
+      recv(g.begin, (n + 1) * sizeof(uint32_t), r);
+      recv(g.vertices, 3 * v * sizeof(float), r);
+      recv(g.normals, 3 * v * sizeof(float), r);
+      recv(g.colors, v * sizeof(uint32_t), r);
+    }
+  }
+  const int end = g_nccl.GroupEnd();
+  if (e == ncclSuccess) e = end;
+  if (e != ncclSuccess) {
+    set_error("%s: NCCL error %d (%s) in the transfer to rank %d", kGatherWho, e,
+              g_nccl.GetErrorString(e), root);
+    return CG_ERR_CUDA;
+  }
+  return CG_OK;
+}
+
+// On the root: every rank's blocks sorted by packed key, vertex_begin by a scan of their vertex
+// counts, each block placed into the mg_* buffers, which then become the retained mesh.
+static int32_t gather_place(cg_context* ctx, const std::vector<GatherWords>& all, int root,
+                            const std::vector<PeerRegions>& regions) {
+  cudaStream_t s = ctx->stream;
+  const int R = static_cast<int>(all.size());
+  size_t N = 0;
+  for (const GatherWords& w : all) N += w.blocks;
+  if (N == 0) return CG_OK;
+  std::vector<MeshSource> src(R);
+  uint32_t first = 0;
+  uint32_t most = 0;
+  for (int r = 0; r < R; ++r) {
+    const uint32_t n = static_cast<uint32_t>(all[r].blocks);
+    MeshSource& S = src[r];
+    if (r == root) {
+      S = MeshSource{ctx->mc_index.as<int32_t>(), ctx->mc_counts.as<uint32_t>() + (n + 1),
+                     ctx->mc_vertices.as<uint32_t>(), ctx->mc_normals.as<uint32_t>(),
+                     ctx->mc_colors.as<uint32_t>(), n, first};
+    } else {
+      const char* in = ctx->mg_in.as<char>();
+      const PeerRegions& g = regions[r];
+      S = MeshSource{reinterpret_cast<const int32_t*>(in + g.idx),
+                     reinterpret_cast<const uint32_t*>(in + g.begin),
+                     reinterpret_cast<const uint32_t*>(in + g.vertices),
+                     reinterpret_cast<const uint32_t*>(in + g.normals),
+                     reinterpret_cast<const uint32_t*>(in + g.colors), n, first};
+    }
+    first += n;
+    most = std::max(most, n);
+  }
+  CG_CUDA(cudaMemcpyAsync(ctx->mg_src.p, src.data(), R * sizeof(MeshSource), cudaMemcpyHostToDevice, s));
+  const MeshSource* d_src = ctx->mg_src.as<MeshSource>();
+  unsigned long long* keys_in = ctx->mg_sort.as<unsigned long long>();
+  unsigned long long *keys_out = keys_in + N, *vals_in = keys_out + N, *vals_out = vals_in + N;
+  uint32_t* counts = ctx->mg_counts.as<uint32_t>();
+  uint32_t* begin = counts + (N + 1);
+  const uint32_t n = static_cast<uint32_t>(N);
+  ctx->own_launches += 3;
+  const unsigned per_rank = static_cast<unsigned>(std::min<size_t>(grid_for(most, 256), ctx->num_sms * 4));
+  k_gather_keys<<<dim3(per_rank, static_cast<unsigned>(R)), 256, 0, s>>>(d_src, keys_in, vals_in);
+  size_t tmp = ctx->cub_tmp.cap;
+  CG_CUDA(cub::DeviceRadixSort::SortPairs(ctx->cub_tmp.p, tmp, keys_in, keys_out, vals_in, vals_out,
+                                          static_cast<int>(n), 0, 63, s));
+  k_gather_counts<<<std::min<unsigned>(grid_for(N + 1, 256), ctx->num_sms * 4), 256, 0, s>>>(
+      d_src, vals_out, n, counts);
+  tmp = ctx->cub_tmp.cap;
+  CG_CUDA(cub::DeviceScan::ExclusiveSum(ctx->cub_tmp.p, tmp, counts, begin, static_cast<int>(n + 1), s));
+  k_place_blocks<<<std::min<unsigned>(grid_for(N, kPlaceThreads / 32), ctx->num_sms * 16),
+                   kPlaceThreads, 0, s>>>(d_src, vals_out, begin, n, ctx->mg_index.as<int32_t>(),
+                                          ctx->mg_vertices.as<uint32_t>(), ctx->mg_normals.as<uint32_t>(),
+                                          ctx->mg_colors.as<uint32_t>());
+  CG_CUDA(cudaGetLastError());
+  // the root's own share was a source: the placed buffers replace it, the old ones are the next
+  // gather's scratch
+  std::swap(ctx->mc_counts, ctx->mg_counts);
+  std::swap(ctx->mc_index, ctx->mg_index);
+  std::swap(ctx->mc_vertices, ctx->mg_vertices);
+  std::swap(ctx->mc_normals, ctx->mg_normals);
+  std::swap(ctx->mc_colors, ctx->mg_colors);
+  return CG_OK;
+}
+
+int32_t cg_mesh_gather_sharded(cg_context* ctx, int32_t root, size_t* num_blocks_out,
+                               size_t* num_vertices_out) {
+  const char* who = kGatherWho;
+  if (num_blocks_out) *num_blocks_out = 0;
+  if (num_vertices_out) *num_vertices_out = 0;
+  if (!ctx) {
+    set_error("%s: null context", who);
+    return CG_ERR_INVALID_ARG;
+  }
+  cg_comm* c = ctx->comm;
+  if (!c) {
+    set_error("%s: call cg_comm_init first", who);
+    return CG_ERR_INVALID_ARG;
+  }
+  CG_CUDA(cudaSetDevice(ctx->device));
+  cudaStream_t s = ctx->stream;
+  const int R = c->nranks;
+  // the opening: one all-gather of every rank's words (the retained mesh, its kind, the root)
+  const GatherWords mine{ctx->mc_blocks, ctx->mc_total, static_cast<unsigned long long>(ctx->mc_kind),
+                         ctx->mc_sharded_calls, root};
+  CG_CUDA(c->gwords.reserve(R * sizeof(GatherWords)));
+  char* d_all = c->gwords.as<char>();
+  CG_CUDA(cudaMemcpyAsync(d_all + c->rank * sizeof(GatherWords), &mine, sizeof(GatherWords),
+                          cudaMemcpyHostToDevice, s));
+  CG_NCCL(g_nccl.AllGather(d_all + c->rank * sizeof(GatherWords), d_all, sizeof(GatherWords),
+                           ncclInt8, c->comm, s));
+  std::vector<GatherWords> all(R);
+  CG_CUDA(cudaMemcpyAsync(all.data(), d_all, R * sizeof(GatherWords), cudaMemcpyDeviceToHost, s));
+  CG_CUDA(cudaStreamSynchronize(s));
+  // every check, and every reservation on the root, before the go/no-go
+  int32_t local = gather_verdict(all);
+  const int rt = static_cast<int>(all[0].root);
+  std::vector<PeerRegions> regions;
+  if (local == CG_OK && c->rank == rt) local = gather_reserve(ctx, all, rt, &regions);
+  uint32_t word = 0;
+  int32_t rc = status_barrier(ctx, local, &word);
+  if (rc) return rc;
+  if (word) {
+    if (local == CG_OK)
+      set_error("%s: rank %d (the root) could not reserve its buffers (status %d); nothing was moved",
+                who, rt, status_of(word));
+    const int32_t rb = barrier(ctx);
+    return rb ? rb : status_of(word);
+  }
+  rc = gather_transfer(ctx, all, rt, regions);
+  if (rc == CG_OK && c->rank == rt) rc = gather_place(ctx, all, rt, regions);
+  // a rank re-meshes or clears its owned layer only after the root has everything
+  const int32_t rb = barrier(ctx);
+  if (rc) return rc;
+  if (rb) return rb;
+  size_t N = 0, V = 0;
+  for (const GatherWords& w : all) {
+    N += w.blocks;
+    V += w.vertices;
+  }
+  if (c->rank == rt) {
+    ctx->mc_blocks = N;
+    ctx->mc_total = V;
+  }
+  ctx->mc_kind = kMeshGathered;
+  if (num_blocks_out) *num_blocks_out = N;
+  if (num_vertices_out) *num_vertices_out = V;
   return CG_OK;
 }
 

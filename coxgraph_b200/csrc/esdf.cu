@@ -837,6 +837,7 @@ int32_t cg_esdf_free_points(cg_context* ctx, float min_distance, size_t capacity
     return CG_ERR_UNSUPPORTED;
   }
   cudaStream_t s = ctx->stream;
+  ctx->mc_kind = kMeshReused;
   CG_CUDA(ctx->mc_counts.reserve(2 * (n + 1) * sizeof(uint32_t)));
   uint32_t* counts = ctx->mc_counts.as<uint32_t>();
   uint32_t* begin = counts + (n + 1);

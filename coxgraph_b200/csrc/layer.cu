@@ -563,7 +563,9 @@ int32_t cg_context_destroy(cg_context* ctx) {
                     &ctx->esdf_slot_to_b, &ctx->esdf_dirty, &ctx->esdf_list, &ctx->esdf_index,
                     &ctx->esdf_counters, &ctx->esdf_dist_next, &ctx->esdf_packed_next,
                     &ctx->esdf_old_b, &ctx->esdf_sources, &ctx->esdf_region,
-                    &ctx->esdf_region_list, &ctx->weld_keys, &ctx->weld_words, &ctx->weld_out};
+                    &ctx->esdf_region_list, &ctx->weld_keys, &ctx->weld_words, &ctx->weld_out,
+                    &ctx->mg_in, &ctx->mg_sort, &ctx->mg_src, &ctx->mg_counts, &ctx->mg_index,
+                    &ctx->mg_vertices, &ctx->mg_normals, &ctx->mg_colors};
   for (DevBuf* b : bufs) b->release();
   drain_events(ctx);
   for (cudaEvent_t e : ctx->event_pool) cudaEventDestroy(e);

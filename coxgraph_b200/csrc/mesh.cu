@@ -540,7 +540,11 @@ static int32_t mesh_to_device(const cg_layer* L, float min_weight, int32_t use_c
   *n_vertices = 0;
   ctx->mc_blocks = 0;
   ctx->mc_total = 0;
-  if (n == 0 && !sharded) return CG_OK;  // a rank without blocks still takes part in the exchange
+  ctx->mc_kind = kMeshNone;
+  if (n == 0 && !sharded) {  // a rank without blocks still takes part in the exchange
+    ctx->mc_kind = kMeshLocal;
+    return CG_OK;
+  }
   const uint64_t* keys = nullptr;
   const uint32_t* slots = nullptr;
   int32_t rc;
@@ -610,6 +614,7 @@ static int32_t mesh_to_device(const cg_layer* L, float min_weight, int32_t use_c
     const int32_t rb = sharded_mesh_close(ctx);
     if (rc == CG_OK) rc = rb;
   }
+  if (rc == CG_OK) ctx->mc_kind = sharded ? kMeshSharded : kMeshLocal;
   return rc;
 }
 
@@ -677,6 +682,7 @@ int32_t cg_layer_mesh_sharded(const cg_layer* owned, float min_weight, int32_t u
     return CG_ERR_INVALID_ARG;
   }
   CG_CUDA(cudaSetDevice(owned->ctx->device));
+  ++owned->ctx->mc_sharded_calls;
   size_t nb = 0, nv = 0;
   int32_t rc = mesh_to_device(owned, min_weight, use_color, only_updated, true, &nb, &nv);
   if (num_blocks_out) *num_blocks_out = nb;

@@ -28,6 +28,7 @@
 #include <memory>
 #include <stdexcept>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include "../../include/coxgraph_b200.h"
@@ -91,6 +92,7 @@ class Context {
   Context(const Context&) = delete;
   Context& operator=(const Context&) = delete;
   cg_context* handle() const { return ctx_; }
+  int commRank() const { return comm_rank_; }  // -1 until commInit
   void synchronize() const { check(cg_context_synchronize(ctx_)); }
   uint64_t kernelLaunches() const { return cg_context_kernel_launches(ctx_); }
   // queue the host->device copy of a LATER job's clouds into staging slot 0 / 1 and return at
@@ -103,7 +105,9 @@ class Context {
   }
 
  private:
+  friend inline void commInit(const Context& ctx, const std::vector<uint8_t>& id, int rank, int nranks);
   cg_context* ctx_ = nullptr;
+  mutable int comm_rank_ = -1;
 };
 
 // ---- voxblox::Block<TsdfVoxel> as handed across the boundary ---------------------------
@@ -412,6 +416,7 @@ inline std::vector<uint8_t> commUniqueId() {
 inline void commInit(const Context& ctx, const std::vector<uint8_t>& id, int rank, int nranks) {
   if (id.size() != CG_COMM_ID_BYTES) fatal_handler()(CG_ERR_INVALID_ARG, "commInit: 128-byte id expected");
   check(cg_comm_init(ctx.handle(), id.data(), rank, nranks));
+  ctx.comm_rank_ = rank;
 }
 inline void getProjectedMapSharded(const std::vector<const TsdfLayer*>& my_submap_layers,
                                    const std::vector<Transformation>& T_M_S, TsdfLayer* partial_layer,
@@ -468,6 +473,18 @@ struct LayerMesh {
   std::vector<Color> colors;
 };
 namespace detail {
+// cg_mesh_fetch of the nb blocks / nv vertices retained in ctx
+inline void fetchMesh(cg_context* ctx, size_t nb, size_t nv, LayerMesh* mesh) {
+  mesh->block_indices.resize(nb);
+  mesh->vertex_begin.assign(nb + 1, 0);
+  mesh->vertices.resize(nv);
+  mesh->normals.resize(nv);
+  mesh->colors.resize(nv);
+  if (nb == 0) return;
+  check(cg_mesh_fetch(ctx, nb, nv, &mesh->block_indices[0].x, mesh->vertex_begin.data(),
+                      nv ? &mesh->vertices[0].x : nullptr, nv ? &mesh->normals[0].x : nullptr,
+                      nv ? &mesh->colors[0].r : nullptr));
+}
 // cg_layer_mesh or cg_layer_mesh_sharded (same arguments), then cg_mesh_fetch
 template <class MeshEntry>
 inline void meshAndFetch(MeshEntry entry, const TsdfLayer& layer, LayerMesh* mesh,
@@ -476,15 +493,7 @@ inline void meshAndFetch(MeshEntry entry, const TsdfLayer& layer, LayerMesh* mes
   check(entry(layer.handle(), config.min_weight, config.use_color ? 1 : 0,
               only_mesh_updated_blocks ? 1 : 0, 0, 0, nullptr, nullptr, nullptr, nullptr, nullptr,
               &nb, &nv));
-  mesh->block_indices.resize(nb);
-  mesh->vertex_begin.assign(nb + 1, 0);
-  mesh->vertices.resize(nv);
-  mesh->normals.resize(nv);
-  mesh->colors.resize(nv);
-  if (nb == 0) return;
-  check(cg_mesh_fetch(layer.context(), nb, nv, &mesh->block_indices[0].x, mesh->vertex_begin.data(),
-                      nv ? &mesh->vertices[0].x : nullptr, nv ? &mesh->normals[0].x : nullptr,
-                      nv ? &mesh->colors[0].r : nullptr));
+  fetchMesh(layer.context(), nb, nv, mesh);
 }
 }  // namespace detail
 inline void generateMesh(const TsdfLayer& layer, LayerMesh* mesh,
@@ -499,6 +508,17 @@ inline void generateMeshSharded(const TsdfLayer& owned_layer, LayerMesh* mesh,
                                 const MeshIntegratorConfig& config = MeshIntegratorConfig(),
                                 bool only_mesh_updated_blocks = false) {
   detail::meshAndFetch(cg_layer_mesh_sharded, owned_layer, mesh, config, only_mesh_updated_blocks);
+}
+// Right after generateMeshSharded on every rank (collective): the ranks' block meshes go to rank
+// `root`, whose context then holds the mesh of the whole map, byte for byte what generateMesh
+// leaves for the gathered map.  On the root `mesh` (may be null) is filled with it and
+// getConnectedMesh / outputMeshAsPly of any layer of that context write the combined map's PLY;
+// elsewhere `mesh` is left alone.  Returns the global {blocks, vertices} on every rank.
+inline std::pair<size_t, size_t> gatherMeshSharded(const Context& ctx, int root, LayerMesh* mesh) {
+  size_t nb = 0, nv = 0;
+  check(cg_mesh_gather_sharded(ctx.handle(), root, &nb, &nv));
+  if (mesh && ctx.commRank() == root) detail::fetchMesh(ctx.handle(), nb, nv, mesh);
+  return {nb, nv};
 }
 
 // ---- MeshLayer::getConnectedMesh + io::outputMeshAsPly: what saveAndPubCombinedMesh does with a

@@ -164,3 +164,13 @@ def mesh_sharded(owned_layer, min_weight=1e-4, use_color=True, only_updated=Fals
     merged by block index, the ranks' results equal generateMesh of the gathered map."""
     from .api import generateMeshSharded
     return generateMeshSharded(owned_layer, min_weight, use_color, only_updated, fetch)
+
+
+def mesh_gather(ctx, root=0):
+    """The output half of saveAndPubCombinedMesh over all ranks (cg_mesh_gather_sharded), right
+    after mesh_sharded on every rank: the block meshes go to rank `root`, whose context then holds
+    the mesh of the whole map, byte for byte generateMesh of the gathered map; Layer.getConnectedMesh
+    of any layer of that context gives the PLY's connected mesh.  Returns gatherMeshSharded's result:
+    the mesh tuple on the root, the global (blocks, vertices) elsewhere."""
+    from .api import gatherMeshSharded
+    return gatherMeshSharded(ctx, root)

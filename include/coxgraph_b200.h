@@ -597,13 +597,35 @@ int32_t cg_reproject_submaps_sharded(const cg_layer* const* submaps, size_t num_
  * message names the rank or the key.  The call ends with a barrier: a rank may clear or refill its
  * owned layer as soon as it returns.  The owned layer's buffers are mapped into the peers the first
  * time it is used and stay mapped until every rank has passed another owned layer or destroyed its
- * communicator; destroy an owned layer only after that.  cg_mesh_connect stays rank-local (the
- * first-occurrence order over the global block order would need a gather). */
+ * communicator; destroy an owned layer only after that.  The combined mesh of the whole map (the
+ * published message, and cg_mesh_connect for the PLY) comes from cg_mesh_gather_sharded below. */
 int32_t cg_layer_mesh_sharded(const cg_layer* owned_layer, float min_weight, int32_t use_color,
                               int32_t only_updated, size_t capacity_blocks, size_t capacity_vertices,
                               int32_t* block_idx_xyz, uint32_t* vertex_begin, float* vertices_xyz,
                               float* normals_xyz, uint8_t* colors_rgba,
                               size_t* num_blocks_out, size_t* num_vertices_out);
+/* The output half of saveAndPubCombinedMesh on several GPUs: the block meshes every rank's latest
+ * cg_layer_mesh_sharded left in its context are gathered onto rank `root`.  Collective over the
+ * context's communicator; every rank calls it right after that cg_layer_mesh_sharded.  On return
+ * the root's context holds exactly what cg_layer_mesh leaves for ONE layer holding the union of all
+ * ranks' owned layers (voxels and `updated` flags), meshed with the same arguments: the block list
+ * in (z, y, x) order, vertex_begin, vertices, normals and colours.  cg_mesh_fetch, the NULL-array
+ * count query and cg_mesh_connect on the root therefore return that layer's bytes (the combined
+ * mesh message and the PLY's connected mesh).  The other ranks keep their own share for
+ * cg_mesh_fetch.  *num_blocks_out / *num_vertices_out (may be NULL) are the global totals on every
+ * rank.  Only the block meshes move (28 B per vertex, 16 B per block), never a TSDF block.
+ * Errors: ctx NULL, or no communicator (cg_comm_init) -> CG_ERR_INVALID_ARG on this rank alone.
+ * Every other error is returned on every rank with the same status, the message naming the rank or
+ * value; a rejected call moves nothing and leaves every rank's retained mesh as it was:
+ * CG_ERR_INVALID_ARG for a root outside [0, nranks) or ranks passing different roots; a rank whose
+ * retained mesh is not the result of its latest successful cg_layer_mesh_sharded (none retained, a
+ * plain cg_layer_mesh or a failed mesh call since, cg_esdf_free_points since — it reuses the mesh
+ * buffers —, or the mesh gathered already: a mesh is gathered once per cg_layer_mesh_sharded); a
+ * global vertex total above 2^32 - 1 (vertex_begin is uint32).  A root that cannot reserve its
+ * buffers makes every rank fail with its status.  The call ends with a barrier: a rank may re-mesh
+ * or clear its owned layer as soon as it returns. */
+int32_t cg_mesh_gather_sharded(cg_context* ctx, int32_t root, size_t* num_blocks_out,
+                               size_t* num_vertices_out);
 /* Peer mappings (cudaIpcOpenMemHandle) of the context's communicator: opened since cg_comm_init,
  * and open now.  A layer is mapped once per role (partial, owned), not once per call. */
 int32_t cg_comm_peer_mappings(const cg_context* ctx, uint64_t* opened_total, uint64_t* open_now);
